@@ -163,6 +163,24 @@ def make_inputs(wl, seed, device, host_copy, coeff_budget=None):
 
 
 COEFF_BUDGET = 40e9
+DUMP_BUDGET = 63_000_000   # bytes of array data written by --dump-outputs (the .npy headers keep the total under 64 MB)
+
+
+def dump_outputs(out_dir, arrays, budget=DUMP_BUDGET):
+    """Writes every array as `out_dir/<name>.npy` in float32.  If all of them together exceed `budget` bytes, each array is cut to
+    the same fraction of its elements, taken flat at positions drawn with a fixed seed (sorted), so that two builds of the project
+    run with the same arguments write values from the same positions and can be compared output for output."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    total = 4 * sum(a.numel() for a in arrays.values())
+    for name, a in arrays.items():
+        a = a.detach().float()
+        if total > budget:
+            keep = max(1, a.numel() * budget // total)
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            a = a.reshape(-1)[idx.to(a.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
 
 
 def tensor_peaks(dev):
@@ -228,9 +246,10 @@ def operand_flags(args):
     return flags
 
 
-def measure_fixed(D, wl_name, wl, args, steps, warmup, with_e2e, tpeaks, e2e_steps, coeff_budget=None):
+def measure_fixed(D, wl_name, wl, args, steps, warmup, with_e2e, tpeaks, e2e_steps, coeff_budget=None, dump_dir=None):
     """One fixed-step workload on this rank's GPU: device-resident value (CUDA-graph replay), the roofline of the contraction
-    launches, and (optionally) the end-to-end legs from pinned host buffers.  Returns a dict (rank-local; times are max over ranks)."""
+    launches, and (optionally) the end-to-end legs from pinned host buffers.  Returns a dict (rank-local; times are max over ranks).
+    With `dump_dir`, rank 0 writes the outputs of the last timed step there (dump_outputs)."""
     import perm_equiv_graph_neural_cdes_b200 as P
     from perm_equiv_graph_neural_cdes_b200 import _lib
     from perm_equiv_graph_neural_cdes_b200 import dist as pdist
@@ -253,15 +272,17 @@ def measure_fixed(D, wl_name, wl, args, steps, warmup, with_e2e, tpeaks, e2e_ste
     params = list(vf.parameters())
 
     def solve_step(pc_, y0_, reduce=True):
+        """Returns what a caller of the solve receives: (loss, flat parameter gradient, y(t1), dloss/dy0)."""
         vf.zero_grad(set_to_none=True)
         y = y0_.detach().requires_grad_(True)
         sol = P.diffeqsolve(term, P.Tsit5(), 0.0, t1_solve, wl["dt0"], y, [pc_, None] if e > 0 else pc_,
                             stepsize_controller=P.ConstantStepSize(), saveat=P.SaveAt(t1=True))
-        loss = (sol.ys[-1] * gy).sum()
+        yT = sol.ys[-1]
+        loss = (yT * gy).sum()
         loss.backward()
         if reduce:   # ONE all-reduce of the flat parameter-gradient buffer (dist.allreduce_gradients; a no-op at world size 1)
-            return loss, pdist.allreduce_gradients(params)
-        return loss, torch.cat([p.grad.reshape(-1) for p in params])
+            return loss, pdist.allreduce_gradients(params), yT.detach(), y.grad
+        return loss, torch.cat([p.grad.reshape(-1) for p in params]), yT.detach(), y.grad
 
     for _ in range(max(warmup, 1)):
         solve_step(pc, y0)
@@ -280,7 +301,7 @@ def measure_fixed(D, wl_name, wl, args, steps, warmup, with_e2e, tpeaks, e2e_ste
         l.pegncde_profile_enable(args.profile_stride)
         launches0 = l.pegncde_launch_count()
         with torch.cuda.graph(graph):
-            g_loss, g_flat = solve_step(pc, y0, reduce=False)
+            g_out = solve_step(pc, y0, reduce=False)
         launches_per_step = l.pegncde_launch_count() - launches0
         for _ in range(2):
             graph.replay()
@@ -290,9 +311,9 @@ def measure_fixed(D, wl_name, wl, args, steps, warmup, with_e2e, tpeaks, e2e_ste
         if graph is not None:
             graph.replay()
             if world > 1:
-                torch.distributed.all_reduce(g_flat)
-            return g_flat
-        return solve_step(pc, y0)[1]
+                torch.distributed.all_reduce(g_out[1])
+            return g_out
+        return solve_step(pc, y0)
 
     sampler = ClockSampler(D.local_rank)
     sampler.start()
@@ -300,12 +321,15 @@ def measure_fixed(D, wl_name, wl, args, steps, warmup, with_e2e, tpeaks, e2e_ste
     host_t0 = time.perf_counter()
     e0.record()
     for _ in range(steps):
-        reduced = timed_step()
+        out = timed_step()
     e1.record()
     host_ms = (time.perf_counter() - host_t0) * 1e3 / steps
     D.barrier()
     clocks = sampler.summary()
     ms = e0.elapsed_time(e1)
+    reduced = out[1]
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, dict(zip(("loss", "grad_params", "yT", "grad_y0"), out)))
     # the reduced gradient buffer must be finite and identical on every rank
     grad_check = {"finite": bool(torch.isfinite(reduced).all())}
     if world > 1:
@@ -339,7 +363,7 @@ def measure_fixed(D, wl_name, wl, args, steps, warmup, with_e2e, tpeaks, e2e_ste
             # streams them piece by piece (copy + pack of piece i+1 overlap the steps inside piece i)
             y0_d = host["y0"].to(dev, non_blocking=True)
             pc_ = P.pack_control(host["ts"], host["cadj"], host["xco"], device=dev)
-            loss, flat_g = solve_step(pc_, y0_d)
+            loss, flat_g = solve_step(pc_, y0_d)[:2]
             return float(loss.item()), flat_g.cpu()
 
         def e2e_snap_step():
@@ -349,7 +373,7 @@ def measure_fixed(D, wl_name, wl, args, steps, warmup, with_e2e, tpeaks, e2e_ste
             x_d = None if host["x_t"] is None else host["x_t"].to(dev, non_blocking=True)
             y0_d = host["y0"].to(dev, non_blocking=True)
             pc_ = P.build_control(ts_d, A_d, x_d)
-            loss, flat_g = solve_step(pc_, y0_d)
+            loss, flat_g = solve_step(pc_, y0_d)[:2]
             return float(loss.item()), flat_g.cpu()
 
         def time_leg(fn):
@@ -469,7 +493,7 @@ def run_ours(args):
         wl["t1_solve"] = args.t1
     tpeaks = None if args.no_tensor_peaks else tensor_peaks(D.dev)
     head = measure_fixed(D, args.workload, wl, args, args.steps, args.warmup, with_e2e=True, tpeaks=tpeaks,
-                         e2e_steps=max(1, min(args.steps, args.e2e_steps)))
+                         e2e_steps=max(1, min(args.steps, args.e2e_steps)), dump_dir=args.dump_outputs)
 
     # ---- the other points of BASELINE.json configs[4] (short solves: t1 = 0.5 -> 5 solver steps, T = 3 knots) and configs[0..3] ----
     sweep, configs = [], []
@@ -808,7 +832,14 @@ def main():
     ap.add_argument("--no-tensor-peaks", action="store_true", help="skip the live cuBLAS tf32 / fp16 / bf16 GEMM measurement")
     ap.add_argument("--shard", default="batch", choices=["batch", "rows"],
                     help="batch: trajectories sharded over the GPUs (default); rows: ONE graph row-sharded over the GPUs (large n)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (loss, flat parameter gradient, y(t1), dloss/dy0; "
+                         "rank 0's shard) as DIR/<name>.npy in float32, at most 64 MB in all (a fixed, seeded sample past that)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.shard != "batch"):
+        ap.error("--dump-outputs writes the outputs of the batch-sharded CUDA path (--impl ours --shard batch)")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "ours" and args.gpus > 1 and world == 1 and "RANK" not in os.environ:
         # `python bench.py --gpus N` outside torchrun: launch the ranks ourselves (one per GPU, NCCL, loopback rendezvous)

@@ -230,6 +230,32 @@ def test_bench_reference_arm_is_silent_on_nonzero_ranks():
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
+def test_bench_dump_outputs_samples_past_the_budget_at_fixed_positions(tmp_path):
+    """`bench.py --dump-outputs` writes float32 arrays; past the byte budget every array keeps the same share of its elements, at
+    positions that depend only on the array's size, so two runs (or two builds) write comparable samples."""
+    import bench
+
+    a = torch.arange(1000, dtype=torch.float32)
+    b = torch.arange(3000, dtype=torch.float64).reshape(30, 100)
+    for d in ("x", "y"):
+        bench.dump_outputs(str(tmp_path / d), {"a": a, "b": b}, budget=1600)
+    xa, xb = np.load(tmp_path / "x" / "a.npy"), np.load(tmp_path / "x" / "b.npy")
+    assert xa.dtype == xb.dtype == np.float32 and xa.shape == (100,) and xb.shape == (300,)
+    assert np.array_equal(xa, np.load(tmp_path / "y" / "a.npy")) and np.array_equal(xb, np.load(tmp_path / "y" / "b.npy"))
+    assert np.all(np.diff(xa) > 0) and xa[-1] < 1000 and np.all(xa == np.round(xa))   # a sorted subset of the elements
+    bench.dump_outputs(str(tmp_path / "z"), {"b": b}, budget=4 * 3000)                # within the budget: whole, shape kept
+    assert np.array_equal(np.load(tmp_path / "z" / "b.npy"), b.numpy().astype(np.float32))
+
+
+def test_bench_rejects_zero_timed_steps():
+    import subprocess
+    import sys
+
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"], capture_output=True, text=True,
+                         timeout=600, cwd=ROOT)
+    assert out.returncode != 0 and "--steps" in out.stderr
+
+
 def test_c_abi_dense_weights_satisfy_the_continuous_order_conditions():
     """pegncde_tsit5_dense_weights (fp32, expanded Horner form) against the order-4 conditions of the interpolant -- a check that
     does not go through the oracle's (factored) restatement of the same polynomials."""

@@ -184,7 +184,7 @@ def test_oracle_matches_reference_source_fixtures(name):
 
 
 @pytest.mark.skipif(not os.path.isdir(os.path.join(PIN.REFERENCE_SRC, "models", "vector_fields")),
-                    reason="the reference tree exists only in the build container")
+                    reason="needs the reference project's source tree (PEG_REFERENCE_SRC)")
 def test_reference_source_fixtures_are_reproducible_from_the_reference_tree():
     """Re-executes the unmodified reference files (numpy stand-ins for jax / equinox) and compares with the committed fixtures."""
     mods = PIN.load_reference_vector_fields()
@@ -255,7 +255,7 @@ def test_oracle_models_match_reference_source_fixtures(name):
 
 
 @pytest.mark.skipif(not os.path.isdir(os.path.join(PIN.REFERENCE_SRC, "models", "vector_fields")),
-                    reason="the reference tree exists only in the build container")
+                    reason="needs the reference project's source tree (PEG_REFERENCE_SRC)")
 def test_reference_model_fixture_is_reproducible_from_the_reference_tree():
     """Re-runs the unmodified reference PGTGraphNeuralCDE on the stand-ins and requires the committed fixture bit for bit."""
     import types
@@ -322,7 +322,7 @@ def test_product_hermite_builder_matches_reference_source_fixture():
 
 
 @pytest.mark.skipif(not os.path.isdir(os.path.join(PIN.REFERENCE_SRC, "models", "vector_fields")),
-                    reason="the reference tree exists only in the build container")
+                    reason="needs the reference project's source tree (PEG_REFERENCE_SRC)")
 def test_reference_dataset_fixture_is_reproducible_from_the_reference_tree():
     import types
 
