@@ -25,10 +25,10 @@
  * Conventions
  *   - every pointer except `step_ts` is a DEVICE pointer owned by the caller (XLA / torch);
  *     the library never allocates, frees or retains device memory.  Host-side state is limited to: the process-wide
- *     launch counter and the optional profiling hooks (pegncde_profile_*, off by default), and two PER-THREAD caches
- *     (TMA descriptors keyed on buffer address and shape; a snapshot of the PEG_TC_* schedule-tuning environment
- *     variables taken at the start of every API call).  Nothing a call computes depends on an earlier call; accuracy
- *     modes are selected through PegDims.flags only, never through the environment.
+ *     launch counter, the optional profiling hooks (pegncde_profile_*, off by default), a PER-THREAD cache of TMA
+ *     descriptors keyed on buffer address and shape, and per-kernel bitmasks of the devices whose kernel attributes
+ *     (opt-in shared memory, cluster size) have been set.  Nothing a call computes depends on an earlier call; every
+ *     mode is selected through PegDims.flags, the library reads no environment variables.
  *   - functions only ENQUEUE work on `stream` (no device synchronisation, no host callbacks),
  *     so they are safe inside an XLA custom call and capturable in a CUDA graph.
  *   - all floating-point data is fp32 (the reference never enables x64), row-major.

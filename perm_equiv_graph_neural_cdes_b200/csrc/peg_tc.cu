@@ -22,7 +22,6 @@
 #include <cuda.h>
 #include <atomic>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 
 #include "peg_tc.cuh"
@@ -100,18 +99,6 @@ __global__ void __launch_bounds__(256) k_block_exponent(const float* __restrict_
 // ------------------------------------------------------------------------------------------
 // the contraction kernel
 // ------------------------------------------------------------------------------------------
-#ifndef PEG_TC_EARLY_RELOAD
-#define PEG_TC_EARLY_RELOAD 0   // measured: earlier re-issue makes the forward launch slower (159 vs 137 us at n=2048, d=128, B=9)
-#endif
-#ifndef PEG_TC_BWD_HALF_EARLY
-#define PEG_TC_BWD_HALF_EARLY 0
-#endif
-// Experiment, NOT YET RUN ON A GPU (round-1 GPU budget was spent): full / empty barriers per operand VARIANT of an adjoint A slot
-// (A_s and A'_s tiles, 32 KB each) instead of per slot, so a converter group may store A_s of item j+2 while the MMAs on A'_s of
-// item j are still running and the MMA thread may start on A_s while A'_s is still being stored (DESIGN.md (f) item 1).
-#ifndef PEG_TC_VARIANT_SLOTS
-#define PEG_TC_VARIANT_SLOTS 0
-#endif
 constexpr int TC_THREADS = 576;   // 2 converter groups x 8 warps + TMA warp + MMA warp
 constexpr int TC_CONV_THREADS = 256;
 constexpr int TC_BM = 128;   // output rows per CTA (UMMA M)
@@ -126,7 +113,6 @@ struct TcParams {
   int stages_b;  // ring depth of the B-operand tiles (one slot per PAIR of items)
   int nkc;       // number of 32-wide K chunks = npad / 32
   int tmem_cols; // power of two >= 32
-  int cluster;   // CTAs per cluster sharing the B operand by TMA multicast (1 = no cluster)
   int mode;      // 0 = whole K range + epilogue; 1 = one K slice of `ksplit`, accumulators added into `partial` (no epilogue);
                  // 2 = epilogue only, accumulators read from `partial`  (split-K for grids far smaller than the GPU)
   int ksplit;    // K slices per row block in mode 1 (blockIdx.x = row block * ksplit + slice)
@@ -134,15 +120,7 @@ struct TcParams {
   const int* vexp; // fp16x2 format: [B][vexp_stride] block exponents of V^T (one per 128 nodes)
   int vexp_stride;
   float* partial; // [B][accumulators][n][d] fp32, zeroed by the host before mode 1
-  int stagger_ns; // 16-bit formats: start-up delay of converter group 1 (see the conversion loop)
-  int experiment; // timing experiments, compiled in only with -DPEG_TC_EXPERIMENTS (never in the shipped library):
-                  // 1 = B operand loaded for the first pairs only, 2 = no MMAs.  Always 0 otherwise.
 };
-#ifdef PEG_TC_EXPERIMENTS
-#define PEG_EXPERIMENT(p, k) ((p).experiment == (k))
-#else
-#define PEG_EXPERIMENT(p, k) false
-#endif
 
 // Per item type of the LIGHT adjoint: the operand pair is (combined = cA A_s + cD A'_s, 3xTF32: it carries the state cotangent)
 // and (sep = A'_s or A_s, ONE tf32 pass: it only feeds two scalar Frobenius gradients).  <sep V, M> and <combined V, M> give
@@ -158,9 +136,6 @@ __device__ __forceinline__ LightCoef light_coef(float wa, float wd) {
 // fp16x2 (block floating point): V^T holds V * 2^(e_J) per 128-node block J.  The blocks are aligned to the smallest exponent E
 // inside the A operand (its entries are multiplied by 2^(E - e_J) <= 1, exact), so every accumulator ends up scaled by 2^E times the
 // A scale.  E is cheap enough (one exponent per 128 nodes) for every thread that needs it to recompute it from global memory.
-#ifndef PEG_VEXP_LOAD
-#define PEG_VEXP_LOAD __ldcg      // (A/B builds only: -DPEG_VEXP_LOAD=__ldg measures what the coherent path costs; wrong on >1 rank)
-#endif
 __device__ __forceinline__ int bfp_min_exponent(const int* __restrict__ ve, int nblk) {
   int e = PEG_VEXP_MAX;
   for (int J = 0; J < nblk; ++J) e = min(e, __ldcg(ve + J));     // L2: in row-sharded mode peers write these entries over NVLink
@@ -187,15 +162,9 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
   constexpr int NA = BWD ? 2 : 1;  // A-operand variants per item: fwd = combined X or Y; bwd = (A_s, A'_s)
   const ContractArgs& a = p.a;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int kslice = p.mode == 1 ? (int)blockIdx.x % p.ksplit : 0;
   const int b = blockIdx.z, I = p.mode == 1 ? (int)blockIdx.x / p.ksplit : (int)blockIdx.x, ntile = blockIdx.y;
+  const int kslice = p.mode == 1 ? (int)blockIdx.x - I * p.ksplit : 0;
   const int n = a.n, d = a.d, nd = p.nd;
-  // CTAs of a cluster walk the K chunks in lockstep (schedule keyed on the cluster's first row block), so one
-  // B tile serves all of them: each CTA fetches 1/C of its rows and multicasts the slice to every peer.
-  const int C = p.cluster;
-  const int crank = C > 1 ? (int)cluster_ctarank() : 0;
-  const int Ibase = (I / C) * C;
-  const uint16_t cmask = (uint16_t)((1u << C) - 1u);
   const bool split = F16 || p.nsplit == 3;
 
   // ---- shared memory carve-up (1024-B aligned operand tiles) ----
@@ -205,14 +174,12 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
   const int b_bytes = (split ? 2 : 1) * b_tile;                 // [hi,lo]
   const int SA = p.stages_a, SB = p.stages_b;
   const uint32_t b_ring = smem_base + SA * a_bytes;
-  constexpr int NV = PEG_TC_VARIANT_SLOTS ? NA : 1;   // barrier pairs per A slot (1: the whole slot is published / released at once)
-  const int SAV = SA * NV;
-  const uint32_t bar_base = b_ring + SB * b_bytes;  // full_a[SA*NV], empty_a[SA*NV], full_b[SB], empty_b[SB], accum_full, tmem slot
-  auto full_a = [&](int s, int v) { return bar_base + 8u * (s * NV + (NV > 1 ? v : 0)); };
-  auto empty_a = [&](int s, int v) { return bar_base + 8u * (SAV + s * NV + (NV > 1 ? v : 0)); };
-  auto full_b = [&](int s) { return bar_base + 8u * (2 * SAV + s); };
-  auto empty_b = [&](int s) { return bar_base + 8u * (2 * SAV + SB + s); };
-  const uint32_t accum_bar = bar_base + 8u * (2 * SAV + 2 * SB);
+  const uint32_t bar_base = b_ring + SB * b_bytes;  // full_a[SA], empty_a[SA], full_b[SB], empty_b[SB], accum_full, tmem slot
+  auto full_a = [&](int s) { return bar_base + 8u * s; };
+  auto empty_a = [&](int s) { return bar_base + 8u * (SA + s); };
+  auto full_b = [&](int s) { return bar_base + 8u * (2 * SA + s); };
+  auto empty_b = [&](int s) { return bar_base + 8u * (2 * SA + SB + s); };
+  const uint32_t accum_bar = bar_base + 8u * (2 * SA + 2 * SB);
   const uint32_t tmem_slot = accum_bar + 8u;
   uint8_t* smem_gen = smem_raw + (smem_base - smem_u32(smem_raw));  // generic pointer to the aligned base
   // 16-bit formats: the chunk schedule of this CTA as a table (pair -> K chunk; BFP: + per A-operand variant the factor
@@ -223,14 +190,13 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
   int* emin_s = reinterpret_cast<int*>(sched_f_s + p.nkc);                                   // smallest block exponent of this graph's V^T
 
   if (tid == 0) {
-    for (int s = 0; s < SA; ++s)
-      for (int v = 0; v < NV; ++v) {
-        mbar_init(full_a(s, v), TC_CONV_THREADS);
-        mbar_init(empty_a(s, v), 1);           // A tiles are CTA-local
-      }
+    for (int s = 0; s < SA; ++s) {
+      mbar_init(full_a(s), TC_CONV_THREADS);
+      mbar_init(empty_a(s), 1);
+    }
     for (int s = 0; s < SB; ++s) {
       mbar_init(full_b(s), 1);
-      mbar_init(empty_b(s), (uint32_t)C);   // one tcgen05.commit arrival from every CTA of the cluster
+      mbar_init(empty_b(s), 1);
     }
     mbar_init(accum_bar, 1);
     fence_barrier_init();
@@ -241,7 +207,6 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
   }
   tc_fence_before();
   __syncthreads();
-  if (C > 1) cluster_sync_all();   // peers' barriers are initialised before any remote arrive / multicast lands
   tc_fence_after();
   const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(smem_gen + (tmem_slot - smem_base));
 
@@ -255,9 +220,9 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
   const int pr0 = p.mode == 1 ? kslice * p.pairs_per_slice : 0;
   const int npairs = p.mode == 2 ? 0 : (p.mode == 1 ? max(0, min(nkc, pr0 + p.pairs_per_slice) - pr0) : nkc);
   const int items = 2 * npairs;   // local item j = 2 * local pair + type (0 direct, 1 transposed); pair works on chunk kc_of(pr0 + pair)
-  // chunk order: 128-column blocks J(S) = (S - Ibase) mod nb, four 32-chunks each (the last block may hold fewer)
+  // chunk order: 128-column blocks J(S) = (S - I) mod nb, four 32-chunks each (the last block may hold fewer)
   const int nb = (nkc + 3) >> 2, r_last = nkc - 4 * (nb - 1);
-  const int Imod = (Ibase + a.row_block0) % nb, Sstar = (nb - 1 + Imod) % nb;   // keyed on the GLOBAL row block (row-sharded mode)
+  const int Imod = (I + a.row_block0) % nb, Sstar = (nb - 1 + Imod) % nb;   // keyed on the GLOBAL row block (row-sharded mode)
   auto kc_of = [&](int pr) -> int {
     int S, u;
     if (pr < 4 * Sstar) { S = pr >> 2; u = pr & 3; }
@@ -300,7 +265,7 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
     const int Emin = BFP ? bfp_min_exponent(ve, (a.ldk + 127) >> 7) : 0;
     for (int pr = tid; pr < npairs; pr += TC_THREADS) {
       const int kc = kc_of(pr0 + pr);
-      const float f = BFP ? exp2_int(max(Emin - PEG_VEXP_LOAD(ve + (kc >> 2)), -120)) : 1.f;
+      const float f = BFP ? exp2_int(max(Emin - __ldcg(ve + (kc >> 2)), -120)) : 1.f;
       sched_kc_s[pr] = kc;
       if (BFP) sched_f_s[pr] = make_float2(f * as0, f * as1);
     }
@@ -346,11 +311,7 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
     // bank-conflict-free (rows are 64 bytes), so the lanes with sw = 1 keep the rows of their micro tile in swapped order
     // (register row m holds tile row m ^ 1).  It costs nothing: only the load addresses and the store offsets change.
     const int sw = (F16 && dirlike) ? ((lane >> 3) & 1) : 0;
-    // `half`: 0 = the first PEG_TC_BWD_HALF_EARLY rows m of the micro tile, 1 = the remaining rows, 2 = all four (the adjoint can
-    // issue the two parts at different times)
-    auto load_tile = [&](int rt, int ct, int half) {
-      constexpr int ME = PEG_TC_BWD_HALF_EARLY > 0 ? PEG_TC_BWD_HALF_EARLY : 2;
-      const int m0 = half == 1 ? ME : 0, m1 = half == 0 ? ME : 4;
+    auto load_tile = [&](int rt, int ct) {
       if constexpr (F16) {
         // row tiles beyond the padded matrix (last 128-row block of a ragged n: 4 I + u >= nt, a per-warp, loop-invariant condition)
         // are read from row tile 0 and their weights are zero: no zero-fill path, the loads stay unconditional
@@ -370,14 +331,10 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
 #pragma unroll
         for (int q = 0; q < 4; ++q)
 #pragma unroll
-          for (int m = 0; m < 4; ++m)
-            if (m >= m0 && m < m1) buf[q * 4 + m] = ldg_stream(((m & 1) ? base_odd : base_even) + (q * 4 + m) * 128);
+          for (int m = 0; m < 4; ++m) buf[q * 4 + m] = ldg_stream(((m & 1) ? base_odd : base_even) + (q * 4 + m) * 128);
       } else {
 #pragma unroll
-        for (int q = 0; q < 4; ++q)
-#pragma unroll
-          for (int m = 0; m < 4; ++m)
-            if (m >= m0 && m < m1) buf[q * 4 + m] = make_float4(0.f, 0.f, 0.f, 0.f);
+        for (int q = 0; q < 16; ++q) buf[q] = make_float4(0.f, 0.f, 0.f, 0.f);
       }
     };
     // item j -> its plane tile: direct = rows of block I x chunk kc, transposed = chunk kc x columns of block I
@@ -389,15 +346,15 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
     for (int v = 0; v < NA; ++v) fitem[v] = 1.f;
     const bool tile_ok = 4 * I + cv_u < ntr;           // this warp's 32-row (direct) / 32-column (transposed) strip exists
     const int my_tile = tile_ok ? 4 * I + cv_u : 0;
-    auto load_item = [&](int j, int half) {
+    auto load_item = [&](int j) {
       const int kc = F16 ? sched_kc_s[j >> 1] : kc_of(pr0 + (j >> 1));
       if constexpr (BFP) {
         const float2 e = sched_f_s[j >> 1];
         fitem[0] = e.x;
         if (NA > 1) fitem[NA - 1] = e.y;
       }
-      if (dirlike) load_tile(F16 ? my_tile : 4 * I + cv_u, kc, half);
-      else load_tile(kc, F16 ? my_tile : 4 * I + cv_u, half);
+      if (dirlike) load_tile(F16 ? my_tile : 4 * I + cv_u, kc);
+      else load_tile(kc, F16 ? my_tile : 4 * I + cv_u);
     };
     // store 4 consecutive k (k = 4 * chunk .. 4 * chunk + 3) of operand row r as hi (+ lo) parts into the swizzled K-major tile:
     // tf32: one 16-byte chunk of a 128-byte row (SWIZZLE_128B); bf16x2: 8 bytes of a 64-byte row (SWIZZLE_64B: 16-byte chunk
@@ -442,18 +399,12 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
           }
         }
       }
-      // forward: the plane registers are dead now -> re-issue the group's next loads before the slot wait and the stores
-      // (the adjoint keeps 32 combined values live and would spill at 96 registers: it reloads after publishing)
-      if (PEG_TC_EARLY_RELOAD && !BWD && j + 2 < items) load_item(j + 2, 2);
-      // adjoint, PEG_TC_BWD_HALF_EARLY: half of the next item's loads go out here (32 registers), under the slot wait and the stores
-      constexpr bool half_early = BWD && PEG_TC_BWD_HALF_EARLY > 0;
-      if (half_early && j + 2 < items) load_item(j + 2, 0);
       const int st = j % SA;
       const uint32_t ph = (uint32_t)(j / SA) & 1u;
       const uint32_t a_base = smem_base + st * a_bytes;
+      mbar_wait(empty_a(st), ph ^ 1u);   // the MMAs that read this slot's previous contents have completed
 #pragma unroll
       for (int v = 0; v < NA; ++v) {
-        if (v == 0 || NV > 1) mbar_wait(empty_a(st, v), ph ^ 1u);   // the MMAs that read this slot's (variant's) previous contents have completed
         const uint32_t hi_base = a_base + v * (split ? 2 : 1) * ATILE;
         const bool with_lo = !(LIGHT && v == NA - 1);   // the single-pass operand needs no correction tile
         if (!transposed) {
@@ -465,12 +416,12 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
           for (int e = 0; e < 4; ++e)   // operand row = tile column 4 cq + e, chunk = rq: the four k values are the rows m = 0..3
             store_chunk(hi_base, 32 * cv_u + 4 * cv_cq + e, cv_rq, t[v][e], t[v][4 + e], t[v][8 + e], t[v][12 + e], with_lo);
         }
-        if (NV > 1 || v == NA - 1) {
-          fence_proxy_async();       // generic-proxy smem writes -> visible to the tensor core (async proxy)
-          mbar_arrive(full_a(st, v));
-        }
       }
-      if (!(PEG_TC_EARLY_RELOAD && !BWD) && j + 2 < items) load_item(j + 2, half_early ? 1 : 2);
+      fence_proxy_async();       // generic-proxy smem writes -> visible to the tensor core (async proxy)
+      mbar_arrive(full_a(st));
+      // the group's next loads go out only now: issued before the slot wait they were measured slower in the forward (159 vs
+      // 137 us at n=2048, d=128, B=9), and the adjoint keeps 32 combined values live that would spill at 96 registers
+      if (j + 2 < items) load_item(j + 2);
     };
 
     // ---- 16-bit operand formats: streaming conversion ----
@@ -507,7 +458,7 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
     // zeroes its rows of each A slot the first time its group uses the slot (a slot is only ever written by one group) and then
     // just keeps the barrier protocol going.  This keeps the plane weights of every working warp warp-uniform (uniform registers).
     auto idle16 = [&](int j) {
-      mbar_wait(empty_a(cur_st, 0), cur_ph ^ 1u);
+      mbar_wait(empty_a(cur_st), cur_ph ^ 1u);
       if (j < SA) {
         const uint32_t a_base = smem_base + cur_st * a_bytes;
 #pragma unroll
@@ -516,14 +467,14 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
           for (int t = 0; t < 2 * NA; ++t) asm volatile("st.shared.v2.b32 [%0], {%1, %1};" ::"r"(a_base + o_m[m] + t * ATILE), "r"(0u) : "memory");
       }
       fence_proxy_async();
-      mbar_arrive(full_a(cur_st, 0));
+      mbar_arrive(full_a(cur_st));
       cur_st += 2;
       if (cur_st >= SA) { cur_st -= SA; cur_ph ^= 1u; }
     };
     auto convert16 = [&](int j, bool transposed) {
 
       const uint32_t a_base = smem_base + cur_st * a_bytes;
-      mbar_wait(empty_a(cur_st, 0), cur_ph ^ 1u);   // the MMAs that read this slot's previous contents have completed
+      mbar_wait(empty_a(cur_st), cur_ph ^ 1u);   // the MMAs that read this slot's previous contents have completed
       if (!transposed) {
 #pragma unroll
         for (int m = 0; m < 4; ++m) {   // operand row = tile row, the four k values are the columns 4 cq .. 4 cq + 3
@@ -565,27 +516,27 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
         }
       }
       fence_proxy_async();       // generic-proxy smem writes -> visible to the tensor core (async proxy)
-      mbar_arrive(full_a(cur_st, 0));
+      mbar_arrive(full_a(cur_st));
       cur_st += 2;               // this group's next item is j + 2
       if (cur_st >= SA) { cur_st -= SA; cur_ph ^= 1u; }
-      if (j + 2 < items) load_item(j + 2, 2);
+      if (j + 2 < items) load_item(j + 2);
     };
 
     if constexpr (F16) {
-      static_assert(!F16 || PEG_TC_VARIANT_SLOTS == 0, "per-variant slot barriers exist for the 3xTF32 format only");
       if (!tile_ok) {
         for (int j = grp; j < items; j += 2) idle16(j);
       } else {
         // The two groups must run OUT of phase (one converts while the other's loads are in flight).  Started together they can
         // lock in phase -- both wait for loads, then both convert and share the issue slots -- which costs a conversion time per
-        // item pair (measured on the fp16x2 adjoint: 195 vs 156 us per launch).  Group 1 therefore starts half a cycle late.
-        if (grp == 1 && p.stagger_ns > 0) __nanosleep((unsigned)p.stagger_ns);
-        if (items > 0) load_item(grp, 2);   // group 0: direct items (even j); group 1: transposed items (odd j)
+        // item pair (measured on the fp16x2 adjoint: 195 vs 156 us per launch).  Group 1 therefore starts half a cycle late
+        // (1200 ns in the adjoint; the forward needs no stagger).
+        if (BWD && grp == 1) __nanosleep(1200u);
+        if (items > 0) load_item(grp);   // group 0: direct items (even j); group 1: transposed items (odd j)
         if (grp == 0) for (int j = 0; j < items; j += 2) convert16(j, false);
         else          for (int j = 1; j < items; j += 2) convert16(j, tposed);
       }
     } else {
-      if (items > 0) load_item(grp, 2);
+      if (items > 0) load_item(grp);
       if (grp == 0) for (int j = 0; j < items; j += 2) convert(j, false);
       else          for (int j = 1; j < items; j += 2) convert(j, tposed);
     }
@@ -597,19 +548,11 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
         const int st = pr % SB;
         const uint32_t ph = (uint32_t)(pr / SB) & 1u;
         const int kc = kc_of(pr0 + pr);
-        mbar_wait(empty_b(st), ph ^ 1u);   // every CTA of the cluster has finished reading this slot
+        mbar_wait(empty_b(st), ph ^ 1u);   // the MMAs have finished reading this slot
         const uint32_t b_base = b_ring + st * b_bytes;
-        if (PEG_EXPERIMENT(p, 1) && pr >= SB) { mbar_arrive(full_b(st)); continue; }   // timing experiment: stale B
         mbar_expect_tx(full_b(st), (uint32_t)b_bytes);
-        if (C == 1) {
-          tma_load_2d(b_base, &map_hi, kc * TC_BK, row0, full_b(st));
-          if (split) tma_load_2d(b_base + b_tile, &map_lo, kc * TC_BK, row0, full_b(st));
-        } else {
-          const int rows = nd / C;                       // this CTA's slice of the B tile (box = 32 x rows)
-          const uint32_t off = (uint32_t)(crank * rows) * (uint32_t)(TC_BK * ESZ);
-          tma_load_2d_mcast(b_base + off, &map_hi, kc * TC_BK, row0 + crank * rows, full_b(st), cmask);
-          if (split) tma_load_2d_mcast(b_base + b_tile + off, &map_lo, kc * TC_BK, row0 + crank * rows, full_b(st), cmask);
-        }
+        tma_load_2d(b_base, &map_hi, kc * TC_BK, row0, full_b(st));
+        if (split) tma_load_2d(b_base + b_tile, &map_lo, kc * TC_BK, row0, full_b(st));
       }
     }
   } else {
@@ -626,12 +569,10 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
         if (type == 0) mbar_wait(full_b(sb), (uint32_t)(pr / SB) & 1u);   // the pair's B tile
         const uint32_t a_base = smem_base + st * a_bytes;
         const uint32_t b_base = b_ring + sb * b_bytes;
+        mbar_wait(full_a(st), ph);
+        tc_fence_after();
 #pragma unroll
         for (int v = 0; v < NA; ++v) {
-          if (v == 0 || NV > 1) {
-            mbar_wait(full_a(st, v), ph);
-            tc_fence_after();
-          }
           // fwd: one accumulator; bwd: acc index = type*2 + v  (0: A V, 1: A'V, 2: A^T V, 3: A'^T V;
           // LIGHT: 0 / 2 = combined operand, 1 / 3 = the single-pass sep operand of the direct / transposed items)
           const int acc = BWD ? (type * 2 + v) : 0;
@@ -640,7 +581,7 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
           if constexpr (F16) {
             // one MMA consumes K = 16 bf16 = 32 bytes of every operand row: two K steps per 32-wide chunk, three products each
 #pragma unroll
-            for (int k16 = 0; k16 < TC_BK / 16 && !(PEG_EXPERIMENT(p, 2) && j >= 2); ++k16) {
+            for (int k16 = 0; k16 < TC_BK / 16; ++k16) {
               const uint64_t dah = make_desc_sw64(ahi + k16 * 32), dbh = make_desc_sw64(b_base + k16 * 32);
               const uint64_t dal = make_desc_sw64(alo + k16 * 32), dbl = make_desc_sw64(b_base + b_tile + k16 * 32);
               umma_bf16(tacc, dah, dbh, idesc, (started >> acc) & 1u);
@@ -650,7 +591,7 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
             }
           } else {
 #pragma unroll
-            for (int k8 = 0; k8 < TC_BK / 8 && !(PEG_EXPERIMENT(p, 2) && j >= 2); ++k8) {
+            for (int k8 = 0; k8 < TC_BK / 8; ++k8) {
               const uint64_t dah = make_desc_sw128(ahi + k8 * 32), dbh = make_desc_sw128(b_base + k8 * 32);
               umma_tf32(tacc, dah, dbh, idesc, (started >> acc) & 1u);
               started |= 1u << acc;
@@ -661,12 +602,9 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
               }
             }
           }
-          if (NV > 1 || v == NA - 1) umma_commit(empty_a(st, v));   // frees this A slot (variant) once the MMAs above have read it
         }
-        if (type == 1) {            // ... and the pair's B slot, in every CTA of the cluster (their producers multicast into it)
-          if (C == 1) umma_commit(empty_b(sb));
-          else umma_commit_mcast(empty_b(sb), cmask);
-        }
+        umma_commit(empty_a(st));                 // frees this A slot once the MMAs above have read it
+        if (type == 1) umma_commit(empty_b(sb));  // ... and the pair's B slot
       }
       if (items > 0) umma_commit(accum_bar);     // all accumulators final
     }
@@ -850,7 +788,6 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
     else { atomicAdd(a.g_fus + 12, t * totA * inv_n2); atomicAdd(a.g_fus + 13, t * totA * inv_n2); }   // reference quirk: both use sum(A)
   }
   __syncwarp();
-  if (C > 1) cluster_sync_all();   // no CTA exits while peers may still multicast into it or arrive on its barriers
   if (warp == 17) {
     __syncwarp();
     tc_fence_after();
@@ -878,39 +815,6 @@ static EncodeTiledFn get_encode() {
   }
   return fn;
 }
-
-// Tuning knobs from the environment (PEG_TC_*): schedule shapes only -- none of them changes what is computed or how
-// accurately (accuracy modes are PegDims.flags).  They are parsed once per API call (tc_refresh_env from make_ctx; a getenv
-// walks the whole environment and a solve enqueues thousands of launches) into a PER-THREAD snapshot: API calls on different
-// threads never share or overwrite each other's copy.
-struct TcEnv {
-  int nd_max = 0, stages_a = 0, stages_b = 0, cluster = 0, experiment = 0, split_max = 0, split_minpairs = 0, stagger_ns = -1;
-  bool no_splitk = false, no_linear = false;
-};
-static thread_local TcEnv g_env;
-static int env_int(const char* name) { const char* ev = getenv(name); return ev ? atoi(ev) : 0; }
-void tc_refresh_env() {
-  TcEnv e;
-  e.nd_max = env_int("PEG_TC_ND_MAX");
-  e.stages_a = env_int("PEG_TC_STAGES_A");
-  e.stages_b = env_int("PEG_TC_STAGES_B");
-  e.cluster = env_int("PEG_TC_CLUSTER");
-#ifdef PEG_TC_EXPERIMENTS
-  e.experiment = env_int("PEG_TC_EXPERIMENT");
-#endif
-  e.split_max = env_int("PEG_TC_SPLIT_MAX");
-  e.split_minpairs = env_int("PEG_TC_SPLIT_MINPAIRS");
-  e.stagger_ns = getenv("PEG_TC_STAGGER_NS") ? env_int("PEG_TC_STAGGER_NS") : -1;
-  e.no_splitk = getenv("PEG_TC_NO_SPLITK") != nullptr;
-  e.no_linear = getenv("PEG_TC_NO_LINEAR") != nullptr;
-  g_env = e;
-}
-
-#define PEG_TC_TRY(expr)              \
-  do {                                \
-    int _rc = (expr);                 \
-    if (_rc != PEG_OK) return _rc;    \
-  } while (0)
 
 // Tensor maps of a K-major fp32 hi / lo operand pair [rows][cols] (cols contiguous), box = 32 cols x box_rows rows,
 // SWIZZLE_128B.  They depend only on (buffers, shape, box): a small per-thread cache keeps the driver call off the
@@ -950,26 +854,6 @@ static int get_maps(const float* hi, const float* lo, uint64_t cols, uint64_t ro
   }
   *mhi = &ent->mhi;
   *mlo = &ent->mlo;
-  return PEG_OK;
-}
-
-// raises the dynamic-smem limit of a kernel once per device (the attribute is per function and device, NOT per thread)
-template <typename K>
-static int optin_smem(K kernel, std::atomic<unsigned>& done) {
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess) { set_last_cuda((int)cudaGetLastError()); return PEG_ERR_CUDA; }
-  const unsigned bit = 1u << (dev & 31);
-  if ((done.load(std::memory_order_acquire) & bit) != 0u) return PEG_OK;
-  int lim = 0;
-  cudaDeviceGetAttribute(&lim, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-  cudaFuncAttributes fa;
-  if (cudaFuncGetAttributes(&fa, kernel) == cudaSuccess) lim -= (int)fa.sharedSizeBytes;   // static smem counts against the limit
-  const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, lim);
-  if (e != cudaSuccess) {
-    fprintf(stderr, "pegncde: cudaFuncSetAttribute(smem %d) failed: %s\n", lim, cudaGetErrorString(e));
-    set_last_cuda((int)e); (void)cudaGetLastError(); return PEG_ERR_CUDA;
-  }
-  done.fetch_or(bit, std::memory_order_release);
   return PEG_OK;
 }
 
@@ -1016,8 +900,6 @@ bool tc_supported(const PegDims& d, int dcols) {
   return get_encode() != nullptr;
 }
 
-int tc_launches_per_contract(bool) { return 2; }
-
 static int tmem_cols_pow2(int cols) {
   int c = 32;
   while (c < cols) c <<= 1;
@@ -1048,12 +930,10 @@ int tc_contract(cudaStream_t st, const PegDims& dm, const TcWs& w, const Contrac
   if (!w.Vt_hi || !w.Vt_lo) return PEG_ERR_WORKSPACE;
   if (!get_encode()) return PEG_ERR_UNSUPPORTED;
   const int fmt = w.fmt, f16 = fmt != PEG_FMT_TF32X3 ? 1 : 0;
-  if (!a.vt_ready) PEG_TC_TRY(tc_convert_v(st, dm, w, a));
+  if (!a.vt_ready) PEG_TRY(tc_convert_v(st, dm, w, a));
   TcParams p;
   p.a = a;
-  int nd_max = bwd ? 128 : 256;
-  { const int v = g_env.nd_max; if (v >= 32 && v <= nd_max) nd_max = v; }
-  p.nd = pick_nd(d, nd_max);
+  p.nd = pick_nd(d, bwd ? 128 : 256);
   p.nsplit = (dm.flags & PEG_FLAG_TF32_FAST) ? 1 : 3;
   p.nkc = ldk / 32;
   const int na = bwd ? 2 : 1, sp = (f16 || p.nsplit == 3) ? 2 : 1;
@@ -1067,28 +947,19 @@ int tc_contract(cudaStream_t st, const PegDims& dm, const TcWs& w, const Contrac
     sb = (208 * 1024 - sa * a_bytes) / b_bytes;
     sb = sb > 4 ? 4 : sb;
   }
-  { const int v = g_env.stages_a; if (v >= 2 && v <= sa && (v & 1) == 0) sa = v; }
-  { const int v = g_env.stages_b; if (v >= 1 && (size_t)sa * a_bytes + (size_t)v * b_bytes <= 224 * 1024) sb = v; }
   if (sa < 2) return PEG_ERR_UNSUPPORTED;
   p.stages_a = sa;
   p.stages_b = sb;
   p.tmem_cols = tmem_cols_pow2((bwd ? 4 : 1) * p.nd);
   const int nblk = (n + TC_BM - 1) / TC_BM;
-  int cluster = 1;   // measured on B200: multicast does not pay (the SM ingress port, not L2, is the limit); PEG_TC_CLUSTER=2|4 enables it
-  { const int v = g_env.cluster; if (v == 1 || v == 2 || v == 4 || v == 8) cluster = v; }
-  while (cluster > 1 && (nblk < cluster || (p.nd / cluster) % 8 != 0)) cluster >>= 1;
-  p.cluster = cluster;
-  p.experiment = g_env.experiment;
-  p.stagger_ns = g_env.stagger_ns >= 0 ? g_env.stagger_ns : (bwd ? 1200 : 0);
   p.vexp = w.vexp;
   p.vexp_stride = w.vexp_stride;
-  const int nv = PEG_TC_VARIANT_SLOTS ? na : 1;   // barrier pairs per A slot (see the kernel)
   const size_t sched_bytes = f16 ? (size_t)12 * p.nkc + 32 : 0;   // chunk-schedule table of the 16-bit formats (at most nkc pairs per CTA)
-  const size_t smem = (size_t)sa * a_bytes + (size_t)sb * b_bytes + 1024 + 8 * (2 * sa * nv + 2 * sb + 2) + 64 + sched_bytes;
+  const size_t smem = (size_t)sa * a_bytes + (size_t)sb * b_bytes + 1024 + 8 * (2 * sa + 2 * sb + 2) + 64 + sched_bytes;
 
   const CUtensorMap* mhi_p = nullptr;
   const CUtensorMap* mlo_p = nullptr;
-  PEG_TC_TRY(get_maps(w.Vt_hi, w.Vt_lo, (uint64_t)ldk, (uint64_t)dm.B * d, p.nd / cluster, &mhi_p, &mlo_p, fmt));
+  PEG_TRY(get_maps(w.Vt_hi, w.Vt_lo, (uint64_t)ldk, (uint64_t)dm.B * d, p.nd, &mhi_p, &mlo_p, fmt));
   const CUtensorMap& mhi = *mhi_p;
   const CUtensorMap& mlo = *mlo_p;
 
@@ -1099,21 +970,18 @@ int tc_contract(cudaStream_t st, const PegDims& dm, const TcWs& w, const Contrac
   {
     const int total = nblk * (d / p.nd) * dm.B;
     int S = 148 / (total > 0 ? total : 1);
-    int smax = 16, minpairs = 2;   // measured on the Twitter shape: 8/4 -> 288, 16/2 -> 298 solver steps/s
-    { const int v = g_env.split_max; if (v >= 2 && v <= 32) smax = v; }
-    { const int v = g_env.split_minpairs; if (v >= 1 && v <= 16) minpairs = v; }
+    const int smax = 16, minpairs = 2;   // measured on the Twitter shape: 8/4 -> 288, 16/2 -> 298 solver steps/s
     S = S > smax ? smax : S;
     S = S > p.nkc / minpairs ? p.nkc / minpairs : S;
-    if (S >= 2 && p.nkc >= 16 && cluster == 1 && w.partial != nullptr && !g_env.no_splitk) {
+    if (S >= 2 && p.nkc >= 16 && w.partial != nullptr) {
       p.pairs_per_slice = (p.nkc + S - 1) / S;
       p.ksplit = (p.nkc + p.pairs_per_slice - 1) / p.pairs_per_slice;   // every slice non-empty
       p.partial = w.partial;
       p.mode = 1;
     }
   }
-  dim3 grid((nblk + cluster - 1) / cluster * cluster, d / p.nd, dm.B);   // padded row blocks only keep the cluster in lockstep
+  dim3 grid(nblk * p.ksplit, d / p.nd, dm.B);
   if (p.mode == 1) {
-    grid.x = (unsigned)(nblk * p.ksplit);
     if (cudaMemsetAsync(w.partial, 0, (size_t)dm.B * (bwd ? 4 : 1) * n * d * sizeof(float), st) != cudaSuccess) {
       set_last_cuda((int)cudaGetLastError());
       return PEG_ERR_CUDA;
@@ -1128,13 +996,13 @@ int tc_contract(cudaStream_t st, const PegDims& dm, const TcWs& w, const Contrac
   {
     static std::atomic<unsigned> done[7] = {{0u}, {0u}, {0u}, {0u}, {0u}, {0u}, {0u}};
     switch (inst) {
-      case 0: PEG_TC_TRY(optin_smem(k_tc_contract<0, 0>, done[0])); break;
-      case 1: PEG_TC_TRY(optin_smem(k_tc_contract<1, 0>, done[1])); break;
-      case 2: PEG_TC_TRY(optin_smem(k_tc_contract<2, 0>, done[2])); break;
-      case 3: PEG_TC_TRY(optin_smem(k_tc_contract<0, 1>, done[3])); break;
-      case 4: PEG_TC_TRY(optin_smem(k_tc_contract<1, 1>, done[4])); break;
-      case 5: PEG_TC_TRY(optin_smem(k_tc_contract<0, 2>, done[5])); break;
-      default: PEG_TC_TRY(optin_smem(k_tc_contract<1, 2>, done[6])); break;
+      case 0: PEG_TRY(optin_smem(k_tc_contract<0, 0>, done[0])); break;
+      case 1: PEG_TRY(optin_smem(k_tc_contract<1, 0>, done[1])); break;
+      case 2: PEG_TRY(optin_smem(k_tc_contract<2, 0>, done[2])); break;
+      case 3: PEG_TRY(optin_smem(k_tc_contract<0, 1>, done[3])); break;
+      case 4: PEG_TRY(optin_smem(k_tc_contract<1, 1>, done[4])); break;
+      case 5: PEG_TRY(optin_smem(k_tc_contract<0, 2>, done[5])); break;
+      default: PEG_TRY(optin_smem(k_tc_contract<1, 2>, done[6])); break;
     }
   }
   cudaLaunchConfig_t cfg;
@@ -1143,13 +1011,6 @@ int tc_contract(cudaStream_t st, const PegDims& dm, const TcWs& w, const Contrac
   cfg.blockDim = dim3(TC_THREADS);
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = cluster;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
   auto launch = [&]() -> cudaError_t {
     switch (inst) {
       case 0: return cudaLaunchKernelEx(&cfg, k_tc_contract<0, 0>, mhi, mlo, p);
@@ -1514,7 +1375,6 @@ static int nl_pick_nd(int dout) {
 bool tc_norm_linear_full_columns(int dout) { return nl_pick_nd(dout) == dout; }
 
 bool tc_linear_supported(int din, int dout) {
-  if (g_env.no_linear) return false;
   return din % 32 == 0 && din >= 32 && nl_pick_nd(dout) != 0 && get_encode() != nullptr;
 }
 
@@ -1551,9 +1411,9 @@ int tc_norm_linear(cudaStream_t st, const PegDims& dm, const TcLinear& w, int la
   const size_t smem = (size_t)stages * stage_bytes + 1024 + 8 * (3 * stages + 2) + 64;
   const CUtensorMap* mhi = nullptr;
   const CUtensorMap* mlo = nullptr;
-  PEG_TC_TRY(get_maps(w.Wn_hi[layer], w.Wn_lo[layer], (uint64_t)din, (uint64_t)dout, p.nd, &mhi, &mlo));
+  PEG_TRY(get_maps(w.Wn_hi[layer], w.Wn_lo[layer], (uint64_t)din, (uint64_t)dout, p.nd, &mhi, &mlo));
   static std::atomic<unsigned> done{0u};
-  PEG_TC_TRY(optin_smem(k_tc_norm_linear, done));
+  PEG_TRY(optin_smem(k_tc_norm_linear, done));
   dim3 grid((dm.n + 127) / 128, dout / p.nd, dm.B);
   k_tc_norm_linear<<<grid, NL_THREADS, smem, st>>>(*mhi, *mlo, p);
   if (cudaPeekAtLastError() != cudaSuccess) {
@@ -1854,7 +1714,6 @@ k_tc_linear_bwd(const __grid_constant__ CUtensorMap map_hi, const __grid_constan
 }
 
 bool tc_linear_bwd_supported(int din, int dout) {
-  if (g_env.no_linear) return false;
   return din % 32 == 0 && din >= 32 && din <= 256 && dout % 32 == 0 && dout >= 32 && get_encode() != nullptr;
 }
 
@@ -1878,9 +1737,9 @@ int tc_linear_bwd(cudaStream_t st, const PegDims& dm, const TcLinear& w, int lay
   const size_t smem = (size_t)stages * stage_bytes + 1024 + 8 * (3 * stages + 2) + 64;
   const CUtensorMap* mhi = nullptr;
   const CUtensorMap* mlo = nullptr;
-  PEG_TC_TRY(get_maps(w.Wt_hi[layer], w.Wt_lo[layer], (uint64_t)dout, (uint64_t)din, din, &mhi, &mlo));
+  PEG_TRY(get_maps(w.Wt_hi[layer], w.Wt_lo[layer], (uint64_t)dout, (uint64_t)din, din, &mhi, &mlo));
   static std::atomic<unsigned> done{0u};
-  PEG_TC_TRY(optin_smem(k_tc_linear_bwd, done));
+  PEG_TRY(optin_smem(k_tc_linear_bwd, done));
   dim3 grid((dm.n + 127) / 128, 1, dm.B);
   k_tc_linear_bwd<<<grid, NL_THREADS, smem, st>>>(*mhi, *mlo, p);
   if (cudaPeekAtLastError() != cudaSuccess) {
@@ -2064,7 +1923,6 @@ __global__ void __launch_bounds__(WG_THREADS, 1) k_tc_weight_grad(const WgParams
 }
 
 bool tc_weight_grad_supported(int din, int dout) {
-  if (g_env.no_linear) return false;
   return dout % 4 == 0 && dout >= 32 && din % 32 == 0 && din >= 32 && din <= 256;
 }
 
@@ -2092,7 +1950,7 @@ int tc_weight_grad(cudaStream_t st, const PegDims& dm, const float* Mbar, const 
   const unsigned nsl = (unsigned)((rows + rps - 1) / rps);
   const size_t smem = (size_t)stages * stage_bytes + 1024 + 8 * (2 * stages + 2) + 64;
   static std::atomic<unsigned> done{0u};
-  PEG_TC_TRY(optin_smem(k_tc_weight_grad, done));
+  PEG_TRY(optin_smem(k_tc_weight_grad, done));
   k_tc_weight_grad<<<dim3(nsl, otiles), WG_THREADS, smem, st>>>(p);
   if (cudaPeekAtLastError() != cudaSuccess) {
     const cudaError_t e = cudaGetLastError();

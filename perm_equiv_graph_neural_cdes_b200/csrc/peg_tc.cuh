@@ -1,7 +1,16 @@
 // tcgen05 (5th-gen tensor core) implementation of the matrix-free equivariant contraction.
 // Declarations only; the kernels live in peg_tc.cu.
 #pragma once
+#include <atomic>
+#include <cstdio>
+
 #include "peg_common.cuh"
+
+#define PEG_TRY(expr)            \
+  do {                           \
+    int _rc = (expr);            \
+    if (_rc != PEG_OK) return _rc; \
+  } while (0)
 
 namespace peg {
 
@@ -31,7 +40,6 @@ struct TcLinear {
   bool ready;   // carved (tensor-core flag set)
 };
 
-void tc_refresh_env();   // re-reads the PEG_TC_* environment knobs (once per API call)
 void tc_carve(Bump& bp, const PegDims& d, int dmax, TcWs& w);
 void tc_carve_linear(Bump& bp, const PegDims& d, const Model& m, TcLinear& w);
 bool tc_linear_supported(int din, int dout);
@@ -53,7 +61,40 @@ bool tc_supported(const PegDims& d, int dcols);
 int tc_fmt(const PegDims& d, bool have_absmax);   // operand format of the contraction (PEG_FMT_*)
 int tc_convert_v(cudaStream_t st, const PegDims& d, const TcWs& w, const ContractArgs& a);
 int tc_contract(cudaStream_t st, const PegDims& d, const TcWs& w, const ContractArgs& a, bool bwd);
-int tc_launches_per_contract(bool bwd);
 void set_last_cuda(int err);   // records a cudaError_t for pegncde_last_cuda_error() (defined in pegncde.cu)
+
+// Kernel attributes are per function AND device: `done` holds one bit per device on which `set(dev)` has succeeded, so each device
+// is configured once per process, also when one process drives several GPUs or calls in from several threads.
+template <typename F>
+int once_per_device(std::atomic<unsigned>& done, F set) {
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess) { set_last_cuda((int)cudaGetLastError()); return PEG_ERR_CUDA; }
+  const unsigned bit = 1u << (dev & 31);
+  if ((done.load(std::memory_order_acquire) & bit) != 0u) return PEG_OK;
+  const cudaError_t e = set(dev);
+  if (e != cudaSuccess) { set_last_cuda((int)e); (void)cudaGetLastError(); return PEG_ERR_CUDA; }
+  done.fetch_or(bit, std::memory_order_release);
+  return PEG_OK;
+}
+
+// raises the dynamic-smem limit of a kernel to the device's opt-in maximum
+template <typename K>
+int optin_smem(K kernel, std::atomic<unsigned>& done) {
+  return once_per_device(done, [kernel](int dev) {
+    int lim = 0;
+    cudaDeviceGetAttribute(&lim, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+    cudaFuncAttributes fa;
+    if (cudaFuncGetAttributes(&fa, kernel) == cudaSuccess) lim -= (int)fa.sharedSizeBytes;   // static smem counts against the limit
+    const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, lim);
+    if (e != cudaSuccess) fprintf(stderr, "pegncde: cudaFuncSetAttribute(smem %d) failed: %s\n", lim, cudaGetErrorString(e));
+    return e;
+  });
+}
+
+// allows a kernel cluster sizes beyond the portable 8 CTAs
+template <typename K>
+int optin_nonportable_cluster(K kernel, std::atomic<unsigned>& done) {
+  return once_per_device(done, [kernel](int) { return cudaFuncSetAttribute(kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1); });
+}
 
 }  // namespace peg

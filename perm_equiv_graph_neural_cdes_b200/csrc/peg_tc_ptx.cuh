@@ -45,22 +45,6 @@ __device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map
       : "memory");
 }
 
-__device__ __forceinline__ void tma_load_2d_mcast(uint32_t dst, const CUtensorMap* map, int c0, int c1, uint32_t bar, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%2, %3}], [%4], %5;" ::"r"(dst),
-      "l"(map), "r"(c0), "r"(c1), "r"(bar), "h"(mask)
-      : "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-
 __device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accum) {
   asm volatile(
       "{\n\t"
@@ -74,10 +58,6 @@ __device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t adesc, uint6
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
-__device__ __forceinline__ void umma_commit_mcast(uint32_t bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar), "h"(mask)
-               : "memory");
-}
 __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t* r) {
   asm volatile(
       "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
@@ -90,22 +70,9 @@ __device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.
 
 // streaming 128-bit plane loads.  Measured on B200 (n=2048, d=128, B=9, forward launch): ld.global.cg 137.6 us, ld.global.nc 139.6,
 // ld.global.nc.L1::no_allocate 156.1, ld.global.cs 159.8, ...no_allocate.L2::256B 156.7 -- the adjoint is insensitive (217 us)
-#ifndef PEG_LDG_VARIANT
-#define PEG_LDG_VARIANT 2
-#endif
 __device__ __forceinline__ float4 ldg_stream(const float* p) {
   float4 r;
-#if PEG_LDG_VARIANT == 0
-  asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
-#elif PEG_LDG_VARIANT == 1
-  asm volatile("ld.global.nc.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
-#elif PEG_LDG_VARIANT == 2
   asm volatile("ld.global.cg.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
-#elif PEG_LDG_VARIANT == 3
-  asm volatile("ld.global.cs.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
-#elif PEG_LDG_VARIANT == 4
-  asm volatile("ld.global.nc.L1::no_allocate.L2::256B.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
-#endif
   return r;
 }
 

@@ -35,12 +35,6 @@ void set_last_cuda(int err) { g_last_cuda = err; }
     }                                              \
   } while (0)
 
-#define PEG_TRY(expr)            \
-  do {                           \
-    int _rc = (expr);            \
-    if (_rc != PEG_OK) return _rc; \
-  } while (0)
-
 // ---- optional per-launch timing of the contraction kernel (bench.py roofline) ----
 struct Prof {
   int stride = 0;
@@ -380,47 +374,29 @@ static int contract(Ctx& c, int l, bool bwd, const float* V, const float* Mref, 
 // ------------------------------------------------------------------------------------------
 // small graphs: one cluster kernel per evaluation / per VJP (peg_small.cuh)
 // ------------------------------------------------------------------------------------------
-struct SmallEnv { int max_n = 0, cluster = 0; bool off = false; };
-static thread_local SmallEnv g_small_env;
-static void small_refresh_env() {
-  SmallEnv e;
-  if (const char* v = getenv("PEG_SMALL_MAX_N")) e.max_n = atoi(v);
-  if (const char* v = getenv("PEG_SMALL_CLUSTER")) e.cluster = atoi(v);
-  e.off = getenv("PEG_SMALL_OFF") != nullptr;
-  g_small_env = e;
-}
-
 // decides whether this call runs on the small-graph kernels and with how many CTAs per graph
 static void small_plan(Ctx& c) {
   c.small_C = 0;
   c.small_smem = 0;
   const PegDims& d = c.d;
-  if (g_small_env.off || (d.flags & PEG_FLAG_NO_FUSED_SMALL)) return;
-  // default: below the smallest tcgen05 shape; PEG_FLAG_FUSED_SMALL widens it (PEG_SMALL_MAX_N: experiments)
-  const int max_n = g_small_env.max_n > 0 ? g_small_env.max_n : ((d.flags & PEG_FLAG_FUSED_SMALL) ? 256 : 127);
+  if (d.flags & PEG_FLAG_NO_FUSED_SMALL) return;
+  // default: below the smallest tcgen05 shape; PEG_FLAG_FUSED_SMALL widens it
+  const int max_n = (d.flags & PEG_FLAG_FUSED_SMALL) ? 256 : 127;
   if (c.sh || c.m.directed || d.n > max_n || d.n > SG_MAX_N || d.h > SG_MAX_DIN) return;
   const size_t smem = small_smem_floats(d.n, d.L) * sizeof(float);
   if (smem > 220 * 1024) return;
-  static int sm_count = 0;
-  static bool attr_done = false, nonportable = false;
-  if (!attr_done) {
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) { (void)cudaGetLastError(); return; }
-    bool ok = cudaFuncSetAttribute(k_small_fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024) == cudaSuccess &&
-              cudaFuncSetAttribute(k_small_vjp, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024) == cudaSuccess;
-    if (!ok) { (void)cudaGetLastError(); return; }
-    nonportable = cudaFuncSetAttribute(k_small_fwd, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess &&
-                  cudaFuncSetAttribute(k_small_vjp, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess;
-    if (!nonportable) (void)cudaGetLastError();
-    attr_done = true;
-  }
+  int dev = 0, sm_count = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) { (void)cudaGetLastError(); return; }
+  static std::atomic<unsigned> smem_done[2] = {{0u}, {0u}}, cluster_done[2] = {{0u}, {0u}};
+  if (optin_smem(k_small_fwd, smem_done[0]) != PEG_OK || optin_smem(k_small_vjp, smem_done[1]) != PEG_OK) return;
+  const bool nonportable = optin_nonportable_cluster(k_small_fwd, cluster_done[0]) == PEG_OK &&
+                           optin_nonportable_cluster(k_small_vjp, cluster_done[1]) == PEG_OK;
   // CTAs per graph: as many as keep the batch within one wave of SMs, no more than the widest phase has work items
   const int dL = c.m.layer[d.L - 1].dout;
   const int items = ((d.n + SG_RB - 1) / SG_RB) * ((dL + SG_WB - 1) / SG_WB);
   int C = 1;
   for (int cand = nonportable ? 16 : 8; cand >= 1; cand >>= 1)
     if ((long long)d.B * cand <= sm_count && cand <= items) { C = cand; break; }
-  if (g_small_env.cluster > 0) C = g_small_env.cluster;
   c.small_C = C;
   c.small_smem = smem;
 }
@@ -520,11 +496,8 @@ static int feval_vjp(Ctx& c, float t, float* const* zin, const float* kbar, floa
   // column sums, block exponents and V^T (otherwise: k_wrapper_bwd here, k_colsums / tc_convert_v further down)
   const bool top_fused = d.e == 0 && contract_on_tc(c, d.L - 1) && dL <= 256 && (dL % 4) == 0;
   if (top_fused) {
-    static bool attr_done = false;
-    if (!attr_done) {
-      PEG_CUDA(cudaFuncSetAttribute(k_top_producer, cudaFuncAttributeMaxDynamicSharedMemorySize, 128 * 257 * (int)sizeof(float)));
-      attr_done = true;
-    }
+    static std::atomic<unsigned> smem_done{0u};
+    PEG_TRY(optin_smem(k_top_producer, smem_done));
     const ProducerOut po = producer_out(c, dL, true, c.w.colG, true, svec_r(d.n, d.L - 1), true);
     if (po.Thi == nullptr) return PEG_ERR_WORKSPACE;
     dim3 grid((unsigned)((po.rows_pad + 127) / 128), d.B);
@@ -634,12 +607,10 @@ static int make_ctx(Ctx& c, peg_stream_t stream, const PegDims* dims, const PegC
   c.m = make_model(*dims);
   c.sv_stride = svec_stride(dims->n, dims->L, dims->e);
   c.use_tc = (dims->flags & PEG_FLAG_TENSOR_CORES) != 0;
-  if (c.use_tc) tc_refresh_env();
   c.fmt = tc_fmt(*dims, ctl->adj_absmax != nullptr);
   c.t_dev = c.dt_dev = nullptr;
   c.tcoef = 0.f;
   c.sh = ctl->shard;
-  small_refresh_env();
   small_plan(c);
   if (c.sh) {
     const PegShard& sh = *c.sh;

@@ -645,26 +645,26 @@ def test_directed_vector_field_against_oracle(cuda, flags):
         assert rel_err(mine.conv_layer.norm.weight.grad, lp.norm_weight.grad) < TOL_G
 
 
-def test_split_k_matches_the_single_pass_contraction(cuda, monkeypatch):
+def test_split_k_matches_the_single_pass_contraction(cuda):
     """Launches far smaller than the GPU (one graph, n = 1000: 8 row blocks) run the contraction split-K (K slices on their
     own SMs, vector-atomic accumulation, epilogue-only second launch).  Same result as the single-pass kernel up to the
-    fp32 summation order of the slices."""
+    fp32 summation order of the slices.  The graph alone (8 row-block tiles on 148 SMs) takes split-K; as one of 10 identical
+    copies (80 tiles) it takes the single-pass kernel, and its dy, d loss / dy and a tenth of the batch's parameter gradients
+    must agree."""
     # seed 21: no hidden unit within fp32 rounding of its ReLU kink at t = 1.3 (seed 8 has one at |z| = 3.5e-7, where the
-    # two summation orders legitimately pick different masks and d loss / d y differs by 7 % -- tools/probes/split_probe2.py)
-    p = R.make_problem(n=1000, h=64, e=0, L=2, T=3, t1=2, dt0=0.5, seed=21)
+    # two summation orders legitimately pick different masks and d loss / d y differs by 7 %)
     outs = []
-    for no_split in ("1", None):
-        if no_split:
-            monkeypatch.setenv("PEG_TC_NO_SPLITK", no_split)
-        else:
-            monkeypatch.delenv("PEG_TC_NO_SPLITK", raising=False)
-        vf, term, args = device_model(p, cuda, flags=TC)
-        y = p.y0.to(cuda).requires_grad_(True)
+    for B in (1, 10):
+        ps = _batched_problems(1000, 64, 0, 2, 3, 2, 0.5, seeds=[21] * B)
+        vf, term, _ = device_model(ps[0], cuda, flags=TC)
+        args = _batched_device_args(ps, cuda)
+        y = torch.stack([p.y0 for p in ps]).to(cuda).requires_grad_(True)
         dy = term(1.3, y, args)
-        (dy * p.gyT.to(cuda)).sum().backward()
-        outs.append((dy.detach().clone(), y.grad.clone(), torch.cat([t.reshape(-1) for layer in product_grads_as_oracle(vf) for t in layer])))
+        (dy * torch.stack([p.gyT for p in ps]).to(cuda)).sum().backward()
+        grads = torch.cat([t.reshape(-1) for layer in product_grads_as_oracle(vf) for t in layer]) / B
+        outs.append((dy[0].detach().clone(), y.grad[0].clone(), grads))
     for a, b in zip(*outs):
-        assert rel_err(a, b) < 5e-6
+        assert rel_err(b, a) < 5e-6
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -1159,3 +1159,28 @@ def test_nccl_reduced_sharded_gradients_equal_the_full_batch_gradients(cuda):
     assert torch.equal(out[0][0], out[1][0])                                   # every rank holds the same reduced buffer
     assert rel_err(out[0][0], full_g) < 1e-5
     assert rel_err(torch.cat([out[0][1], out[1][1]]), full_y) < 1e-6          # the shards are the rows of the full batch
+
+
+@pytest.mark.parametrize("kw,flags", [(dict(n=100, h=32, e=0, L=3, T=4, t1=2, dt0=0.5, seed=4), None),
+                                      (dict(n=256, h=128, e=0, L=2, T=4, t1=2, dt0=0.5, seed=6), TC)],
+                         ids=["small-graph", "tcgen05-top-producer"])
+def test_one_process_drives_two_gpus(cuda, kw, flags):
+    """Kernel attributes (the dynamic shared memory of k_small_fwd / k_small_vjp / k_top_producer, the non-portable cluster size
+    of the small-graph kernels) are per device: after an evaluation and its VJP on cuda:0, the same on cuda:1 runs and gives the
+    same dy and d loss / dy (1e-6, not bit equality: the small-graph path sums some terms with atomics).  n = 100 takes the
+    default small-graph path; the e = 0 tcgen05 case starts its VJP with k_top_producer (128 x 129 floats of shared memory)."""
+    if torch.cuda.device_count() < 2:
+        pytest.skip("needs two GPUs")
+    p = R.make_problem(**kw)
+    outs = []
+    for dev in (torch.device("cuda", 0), torch.device("cuda", 1)):
+        with torch.cuda.device(dev):
+            vf, term, args = device_model(p, dev, flags=flags)
+            y = p.y0.to(dev).requires_grad_(True)
+            dy = term(1.3, y, args)
+            (dy * p.gyT.to(dev)).sum().backward()
+            torch.cuda.synchronize(dev)
+            outs.append((dy.detach().cpu(), y.grad.cpu()))
+    (dy0, g0), (dy1, g1) = outs
+    assert rel_err(dy1, dy0) < 1e-6
+    assert rel_err(g1, g0) < 1e-6
