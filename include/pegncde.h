@@ -125,6 +125,26 @@ typedef struct PegShard {
   uint32_t* epoch_dev;       /* nullable DEVICE word (this rank's own memory, zero-initialised): epoch base for graph replay  */
 } PegShard;
 
+/* Sparse (CSR) adjacency path of one batch, built by pegncde_build_adj_sparse / pegncde_pack_adj_sparse.  The batch shares
+ * one entry axis: graph b's row i holds the entries [row_ptr[b, i], row_ptr[b, i + 1]) (ABSOLUTE offsets into col and into the
+ * entry axis of coef), so a view of one graph needs no copy.  The transposed pattern is stored the same way with its own copy of
+ * the coefficients (row i of the transpose = the entries (k, i) of the path), so that both orientations walk contiguous memory.
+ *
+ * A sparse control runs the n x n x d contraction as an fp32 FMA gather (k_sparse_contract): the operand-format flags
+ * PEG_FLAG_TF32X3, PEG_FLAG_BF16X2, PEG_FLAG_TF32_FAST and PEG_FLAG_ADJ_LIGHT mean nothing for it, and the small-graph cluster
+ * kernels are not used.  PEG_FLAG_TENSOR_CORES still selects the tcgen05 RMSNorm -> Linear kernels.  Not combinable with
+ * PegControl.shard (PEG_ERR_UNSUPPORTED). */
+typedef struct PegSparse {
+  int64_t nnz;              /* entries of the whole batch (both orientations hold the same count)                            */
+  int64_t nnz_stride;       /* entries per coefficient slab, >= nnz                                                          */
+  const int32_t* row_ptr;   /* [B, n+1]  absolute offsets of every row                                                       */
+  const int32_t* col;       /* [nnz]     column of each entry, ascending inside a row                                        */
+  const float* coef;        /* [T-1, nnz_stride, 4]  (a, b, c, d) of each entry for each cubic piece (one 16-byte load)      */
+  const int32_t* row_ptr_t; /* the same three arrays for the transposed pattern                                              */
+  const int32_t* col_t;
+  const float* coef_t;
+} PegSparse;
+
 /* Planar control path, built once per batch by pegncde_pack_adj / pegncde_pack_x.
  * Coefficient order everywhere is (a, b, c, d):  X(t) = a + s(b + s(c + s d)), s = t - ts[i]. */
 typedef struct PegControl {
@@ -146,6 +166,9 @@ typedef struct PegControl {
   const PegShard* shard;   /* NULL = the whole graph lives on this GPU; otherwise row-sharded mode (see PegShard): every array
                               above holds this rank's rows only (adj_coef: [B, T-1, 4 * ldn * n_glob]), adj_total / adj_absmax are
                               already reduced over the ranks, adj_diag[i] = entry (row0 + i) of local row i                  */
+  const PegSparse* sparse; /* NULL = dense planes (adj_coef).  Otherwise the adjacency path is the CSR path of PegSparse: adj_coef may be
+                              NULL, adj_absmax is unused, adj_rowsum / adj_diag / adj_total / adj_colsum / tch_coef keep their meaning
+                              (the sparse builders fill all of them, adj_colsum included)                                    */
 } PegControl;
 
 /* ---- parameter packing ---------------------------------------------------------------
@@ -197,6 +220,20 @@ int pegncde_adj_colsums(peg_stream_t stream, const PegDims* dims, const float* a
  * independent, hence reproducible) */
 int pegncde_adj_absmax(peg_stream_t stream, const PegDims* dims, int32_t piece_begin, int32_t piece_count, const float* adj_coef,
                        float* adj_absmax);
+/* Sparse control-path builders (see PegSparse).  `sp` describes the pattern (row_ptr, col, row_ptr_t, col_t, nnz, nnz_stride);
+ * its coef / coef_t are the OUTPUTS (cast away const).  perm_t [nnz] scatters entry e of the pattern to position perm_t[e] of the
+ * transposed pattern.  Both write coef, coef_t, adj_rowsum, adj_diag, adj_total, adj_colsum ([B, T-1, 4, n] each, totals [B, T-1, 4])
+ * and tch_coef = (1, 0, 0) (the time channel is implied).  Every reduction runs in a fixed order: the control is reproducible.
+ *   pegncde_build_adj_sparse: knot times ts [B, T] and the values of the path on the pattern, values [T, nnz] (0 where an edge is
+ *     absent at a knot); backward_hermite_coefficients is fused in with the per-element arithmetic of pegncde_build_adj, so the
+ *     coefficients are bit-identical to the dense builder's at every pattern position.
+ *   pegncde_pack_adj_sparse: coefficients given, d, c, b, a each [T-1, nnz] (adjacency channel only; the sparse form of the
+ *     reference's coeffs_adj -- linear interpolation is c = d = 0). */
+int pegncde_build_adj_sparse(peg_stream_t stream, const PegDims* dims, const PegSparse* sp, const int32_t* perm_t, const float* ts,
+                             const float* values, float* adj_rowsum, float* adj_diag, float* adj_total, float* adj_colsum, float* tch_coef);
+int pegncde_pack_adj_sparse(peg_stream_t stream, const PegDims* dims, const PegSparse* sp, const int32_t* perm_t, const float* d,
+                            const float* c, const float* b, const float* a, float* adj_rowsum, float* adj_diag, float* adj_total,
+                            float* adj_colsum, float* tch_coef);
 /* d,c,b,a each [B, T-1, n, e, 2] -> x_coef [B, T-1, 3, n, 2e] */
 int pegncde_pack_x(peg_stream_t stream, const PegDims* dims, const float* d, const float* c, const float* b,
                    const float* a, float* x_coef);
@@ -302,7 +339,9 @@ uint64_t pegncde_launch_count(void);
  * When enabled, every `stride`-th launch of the dominant kernel (the n x n x d contraction) is
  * bracketed by CUDA events on the launching stream.  pegncde_profile_read synchronises those events
  * and returns, per direction (0 = forward contraction, 1 = backward/adjoint contraction): launches seen,
- * launches timed, summed milliseconds of the timed ones and the algorithmic bytes / flops of one launch.
+ * launches timed, summed milliseconds of the timed ones and the algorithmic bytes / flops of one launch.  For a sparse control
+ * the bytes are its HBM traffic (both orientations' coefficients and columns, row pointers, V, OUT, M in the adjoint); the
+ * gathers of V rows (2 nnz d 4 bytes, mostly served from L2) are not included.
  * stride <= 0 disables and frees the events. */
 int pegncde_profile_enable(int32_t stride);
 int pegncde_profile_read(int32_t direction, uint64_t* launches, uint64_t* timed, double* ms_total,

@@ -9,6 +9,7 @@ from ._lib import LIB_PATH, PegControl, PegDims, PegError, lib  # noqa: F401
 lib()  # raise ImportError right here if libpegncde.so is missing
 
 from .control import CubicInterpolation, LinearInterpolation, PackedControl, backward_hermite_coefficients, build_control, pack_control  # noqa: E402,F401
+from .control import SparseControl, SparsePattern, build_sparse_control, pack_sparse_control, sparse_pattern  # noqa: E402,F401
 from .models import MLP, GraphNeuralCDE, PGTGraphNeuralCDE, TGBGraphNeuralCDE  # noqa: E402,F401
 from .solve import (ConstantStepSize, ODETerm, PIDController, SaveAt, Solution, Tsit5, clip_to_end, constant_step_table,  # noqa: E402,F401
                     dense_weights, diffeqsolve, tsit5_step)  # noqa: E402,F401

@@ -41,8 +41,13 @@ class PegAdaptState(Structure):
                 ("mi", c_int32), ("mi0", c_int32), ("mi1", c_int32), ("keep", c_int32), ("h", c_float), ("overflow", c_int32)]
 
 
+class PegSparse(Structure):
+    """Sparse (CSR) adjacency path of one batch (include/pegncde.h): absolute row offsets, both orientations."""
+    _fields_ = [("nnz", c_int64), ("nnz_stride", c_int64)] + [(k, c_void_p) for k in ("row_ptr", "col", "coef", "row_ptr_t", "col_t", "coef_t")]
+
+
 class PegControl(Structure):
-    _fields_ = [(k, c_void_p) for k in ("ts", "adj_coef", "adj_rowsum", "adj_diag", "adj_total", "tch_coef", "x_coef", "adj_colsum", "adj_absmax")] + [("shard", POINTER(PegShard))]
+    _fields_ = [(k, c_void_p) for k in ("ts", "adj_coef", "adj_rowsum", "adj_diag", "adj_total", "tch_coef", "x_coef", "adj_colsum", "adj_absmax")] + [("shard", POINTER(PegShard)), ("sparse", POINTER(PegSparse))]
 
 
 class PegError(RuntimeError):
@@ -72,6 +77,8 @@ SIGNATURES = {
     "pegncde_build_adj_rect": (c_int, [_P, _DIMS, c_int32, c_int32, _P, _P, _P, _P, _P, _P, _P, _P]),
     "pegncde_shard_buffer_bytes": (c_int, [_DIMS, c_int32, POINTER(c_size_t)]),
     "pegncde_adj_absmax": (c_int, [_P, _DIMS, c_int32, c_int32, _P, _P]),
+    "pegncde_build_adj_sparse": (c_int, [_P, _DIMS, POINTER(PegSparse), _P, _P, _P, _P, _P, _P, _P, _P]),
+    "pegncde_pack_adj_sparse": (c_int, [_P, _DIMS, POINTER(PegSparse), _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "pegncde_pack_x": (c_int, [_P, _DIMS, _P, _P, _P, _P, _P]),
     "pegncde_workspace_bytes": (c_size_t, [_DIMS, c_int32, c_int32]),
     "pegncde_vf_fwd": (c_int, [_P, _DIMS, _CTL, _P, c_float, _P, _P, _P, c_size_t]),

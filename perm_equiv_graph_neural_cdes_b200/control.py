@@ -335,3 +335,272 @@ def build_control(ts: torch.Tensor, snapshots: torch.Tensor, x_t: Optional[torch
     _attach_x(pc, cx, device)
     pc._keepalive = A
     return pc
+
+
+# ------------------------------------------------------------------------------------------------------------------------
+# sparse (CSR) controls: PegSparse in pegncde.h
+# ------------------------------------------------------------------------------------------------------------------------
+class SparsePattern:
+    """Coalesced CSR pattern of a batch of B graphs (:func:`sparse_pattern`).  Every index array is absolute: graph b's rows point
+    into one shared entry axis of ``nnz`` entries.
+
+    ``row_ptr``/``row_ptr_t`` ``[B, n+1]``, ``col``/``col_t`` ``[nnz]`` (int32): the pattern and its transpose, columns ascending
+    inside a row.  ``perm_t`` ``[nnz]`` (int32): entry e sits at position ``perm_t[e]`` of the transposed pattern.  ``edge_map[b]``
+    ``[E_b]`` (int64): the entry every input edge of graph b was coalesced into."""
+
+    def __init__(self, n, row_ptr, col, row_ptr_t, col_t, perm_t, edge_map):
+        self.n, self.B, self.nnz = n, row_ptr.shape[0], int(col.numel())
+        self.row_ptr, self.col, self.row_ptr_t, self.col_t, self.perm_t, self.edge_map = row_ptr, col, row_ptr_t, col_t, perm_t, edge_map
+
+
+def _edge_list(edge_index) -> list:
+    if isinstance(edge_index, torch.Tensor):
+        return [edge_index]
+    if isinstance(edge_index, (list, tuple)) and len(edge_index) > 0 and all(isinstance(e, torch.Tensor) for e in edge_index):
+        return list(edge_index)
+    raise ValueError("edge_index must be a [2, E] integer tensor or a non-empty list of them (one per graph)")
+
+
+def sparse_pattern(edge_index, num_nodes: int) -> SparsePattern:
+    """Edge list(s) -> the coalesced CSR pattern and its transpose (torch ops on the device of ``edge_index``).
+
+    ``edge_index``: ``[2, E]`` (rows, columns) or a list of B of them with any E per graph.  Duplicate edges become one entry (their
+    values are summed, as ``index_put_(accumulate=True)`` into a dense matrix would).  Malformed input raises ``ValueError``."""
+    n = int(num_nodes)
+    if n < 1:
+        raise ValueError(f"num_nodes must be >= 1, got {num_nodes}")
+    graphs = _edge_list(edge_index)
+    rp, cols, rpt, colts, perms, maps = [], [], [], [], [], []
+    base = 0
+    for g, ei in enumerate(graphs):
+        if ei.dim() != 2 or ei.shape[0] != 2:
+            raise ValueError(f"edge_index of graph {g} must have shape [2, E], got {tuple(ei.shape)}")
+        if ei.dtype.is_floating_point or ei.dtype.is_complex or ei.dtype == torch.bool:
+            raise ValueError(f"edge_index of graph {g} must hold integers, got {ei.dtype}")
+        ei = ei.to(torch.int64)
+        if ei.numel() > 0 and (int(ei.min()) < 0 or int(ei.max()) >= n):
+            raise ValueError(f"edge_index of graph {g} has a node index outside [0, {n})")
+        key = ei[0] * n + ei[1]
+        uniq, inv = torch.unique(key, sorted=True, return_inverse=True)
+        rows, cs = uniq // n, uniq % n
+        m = int(uniq.numel())
+        if base + m > 2**31 - 1:
+            raise ValueError("the batch has more than 2^31 - 1 entries")
+        dev = ei.device
+        counts = torch.bincount(rows, minlength=n)
+        rp.append(torch.cat([torch.zeros(1, dtype=torch.int64, device=dev), counts.cumsum(0)]) + base)
+        cols.append(cs)
+        order = torch.argsort(cs * n + rows)                     # transposed order: by column, then row
+        pos = torch.empty_like(order)
+        pos[order] = torch.arange(m, device=dev)
+        counts_t = torch.bincount(cs, minlength=n)
+        rpt.append(torch.cat([torch.zeros(1, dtype=torch.int64, device=dev), counts_t.cumsum(0)]) + base)
+        colts.append(rows[order])
+        perms.append(pos + base)
+        maps.append(inv.reshape(-1) + base)
+        base += m
+    i32 = lambda xs: torch.cat(xs).to(torch.int32).contiguous()
+    return SparsePattern(n, torch.stack(rp).to(torch.int32).contiguous(), i32(cols), torch.stack(rpt).to(torch.int32).contiguous(),
+                         i32(colts), i32(perms), maps)
+
+
+class SparseControl(PackedControl):
+    """A control path on a sparse (CSR) adjacency pattern: ``PegControl.sparse`` is set and ``adj_coef`` is NULL.  Used wherever a
+    :class:`PackedControl` is (vector fields, ``diffeqsolve``, ``tsit5_step``, the models); built by :func:`build_sparse_control` or
+    :func:`pack_sparse_control`.  ``coef``/``coef_t`` are ``[T-1, nnz, 4]`` (a,b,c,d per entry) in pattern and transposed order."""
+
+    def __init__(self, pattern: SparsePattern, T: int, device):
+        B, n = pattern.B, pattern.n
+        self.B, self.n, self.T, self.e, self.ldn = B, n, T, 0, _pad32(n)
+        self.pattern = pattern
+        f = dict(dtype=torch.float32, device=device)
+        self.ts = torch.empty((B, T), **f)
+        self.adj_coef = None
+        self.adj_absmax = None
+        self.adj_rowsum = torch.empty((B, T - 1, 4, n), **f)
+        self.adj_diag = torch.empty((B, T - 1, 4, n), **f)
+        self.adj_total = torch.empty((B, T - 1, 4), **f)
+        self.tch_coef = torch.empty((B, T - 1, 3, n), **f)
+        nnz = max(pattern.nnz, 1)
+        self.coef = torch.empty((T - 1, nnz, 4), **f)
+        self.coef_t = torch.empty((T - 1, nnz, 4), **f)
+        self.row_ptr, self.row_ptr_t = pattern.row_ptr, pattern.row_ptr_t
+        self.col, self.col_t = pattern.col, pattern.col_t
+        self.x_coef, self.x_packed = None, None
+        self._adj = {"colsum": torch.empty((B, T - 1, 4, n), **f), "pending": None, "host_ts": None}
+
+    @property
+    def nnz(self) -> int:
+        return self.pattern.nnz
+
+    def sparse_struct(self):
+        from ._lib import PegSparse
+        return PegSparse(self.pattern.nnz, self.coef.shape[1], self.row_ptr.data_ptr(), self.col.data_ptr(), self.coef.data_ptr(),
+                         self.row_ptr_t.data_ptr(), self.col_t.data_ptr(), self.coef_t.data_ptr())
+
+    def struct(self) -> PegControl:
+        import ctypes
+        self._sp = self.sparse_struct()      # the PegControl below points at it: kept alive with the control
+        return PegControl(self.ts.data_ptr(), None, self.adj_rowsum.data_ptr(), self.adj_diag.data_ptr(), self.adj_total.data_ptr(),
+                          self.tch_coef.data_ptr(), self.x_coef.data_ptr() if self.x_coef is not None else None,
+                          self.adj_colsum.data_ptr(), None, None, ctypes.pointer(self._sp))
+
+    def _view(self) -> "SparseControl":
+        v = SparseControl.__new__(SparseControl)
+        v.B, v.n, v.T, v.e, v.ldn = self.B, self.n, self.T, self.e, self.ldn
+        for name in ("pattern", "ts", "adj_coef", "adj_absmax", "adj_rowsum", "adj_diag", "adj_total", "tch_coef", "coef", "coef_t",
+                     "row_ptr", "row_ptr_t", "col", "col_t", "x_coef", "x_packed"):
+            setattr(v, name, getattr(self, name))
+        v._adj = self._adj
+        v._keepalive = self
+        return v
+
+    def with_x(self, x_coeffs) -> "SparseControl":
+        """The same pattern and coefficients (shared, no copy) paired with the node-signal coefficients ``x_coeffs``."""
+        v = self._view()
+        _attach_x(v, x_coeffs, self.device)
+        return v
+
+    def select(self, b: int) -> "SparseControl":
+        """View of graph ``b`` as a batch of one (no copy: the row offsets are absolute into the shared entry axis)."""
+        v = self._view()
+        v.B = 1
+        for name in ("ts", "adj_rowsum", "adj_diag", "adj_total", "tch_coef", "row_ptr", "row_ptr_t"):
+            setattr(v, name, getattr(self, name)[b:b + 1])
+        v.x_coef = self.x_coef[b:b + 1] if self.x_coef is not None else None
+        v.x_packed = None
+        v._adj = {"colsum": self.adj_colsum[b:b + 1], "pending": None, "host_ts": None}
+        return v
+
+    def materialize(self) -> "SparseControl":
+        return self
+
+    def ensure_colsums(self) -> "SparseControl":
+        return self            # the sparse builders always write the column sums
+
+    def pack_pieces(self, *args, **kwargs):
+        raise TypeError("sparse controls are built in one go; they have no streamed pieces")
+
+    def plane_maxima(self, *args, **kwargs):
+        raise TypeError("sparse controls have no tiled planes (adj_absmax is unused)")
+
+    def dense_planes(self) -> torch.Tensor:
+        """The path densified to [B, T-1, 4(a,b,c,d), n, n] (inspection / tests: O(n^2) memory)."""
+        out = torch.zeros((self.B, self.T - 1, 4, self.n, self.n), dtype=torch.float32, device=self.device)
+        rp = self.row_ptr.to(torch.int64)
+        for b in range(self.B):
+            e0, e1 = int(rp[b, 0]), int(rp[b, -1])
+            rows = torch.repeat_interleave(torch.arange(self.n, device=self.device), rp[b, 1:] - rp[b, :-1])
+            cols = self.col[e0:e1].to(torch.int64)
+            out[b][:, :, rows, cols] = self.coef[:, e0:e1].permute(0, 2, 1)
+        return out
+
+
+def _sparse_dims(pat: SparsePattern, T: int, e: int = 0) -> PegDims:
+    return PegDims(pat.B, pat.n, _pad32(pat.n), 4, e, 1, T, 0)
+
+
+def _per_graph(x, B: int, what: str) -> list:
+    xs = list(x) if isinstance(x, (list, tuple)) else [x]
+    if len(xs) != B:
+        raise ValueError(f"{what}: expected {B} graphs, got {len(xs)}")
+    return xs
+
+
+def _node_signal_coeffs(ts_b: torch.Tensor, x_t: torch.Tensor, B: int, T: int, n: int, device):
+    xb = _as_batched(x_t, 3).to(device=device, dtype=torch.float32)
+    if tuple(xb.shape[:3]) != (B, T, n):
+        raise ValueError(f"x_t must be [T={T}, n={n}, e] or [B={B}, T, n, e], got {tuple(x_t.shape)}")
+    e = xb.shape[-1]
+    per = []
+    for b in range(B):
+        X = torch.stack([ts_b[b][:, None, None].expand(T, n, e), xb[b]], dim=-1)
+        per.append(backward_hermite_coefficients(ts_b[b], X))
+    return [torch.stack([per[b][i] for b in range(B)]).contiguous() for i in range(4)]
+
+
+def _new_sparse_control(ts, pattern: SparsePattern, T: int, device) -> SparseControl:
+    if T < 2:
+        raise ValueError("a control path needs at least two knots")
+    sc = SparseControl(pattern, T, device)
+    tsb = _as_batched(torch.as_tensor(ts), 1).to(device=device, dtype=torch.float32)
+    if tsb.shape[-1] != T or tsb.shape[0] not in (1, pattern.B):
+        raise ValueError(f"ts must be [T={T}] or [B={pattern.B}, T], got {tuple(tsb.shape)}")
+    sc.ts.copy_(tsb.expand(pattern.B, T))
+    return sc
+
+
+def build_sparse_control(ts: torch.Tensor, edge_index, edge_weight, num_nodes: int, x_t: Optional[torch.Tensor] = None,
+                         device=None) -> SparseControl:
+    """Edge list(s) + per-knot edge weights -> :class:`SparseControl` (``pegncde_build_adj_sparse``: the sparse form of
+    :func:`build_control`, with the same Hermite arithmetic, so the coefficients equal the dense builder's bit for bit).
+
+    ``edge_index``: ``[2, E]`` or a list of B; ``edge_weight``: ``[T, E]`` (or a list of B, matching), the value of every edge at
+    every knot (0 where it is absent); ``ts``: ``[T]`` or ``[B, T]``; ``x_t``: optional node signals ``[T, n, e]`` / ``[B, T, n, e]``."""
+    graphs = _edge_list(edge_index)
+    device = torch.device(device if device is not None else graphs[0].device)
+    if device.type != "cuda":
+        raise RuntimeError("build_sparse_control needs a CUDA device: the fused path has no CPU fallback")
+    pat = sparse_pattern([g.to(device) for g in graphs], num_nodes)
+    ws = [w.to(device=device, dtype=torch.float32) for w in _per_graph(edge_weight, pat.B, "edge_weight")]
+    T = ws[0].shape[0]
+    for b, (w, g) in enumerate(zip(ws, graphs)):
+        if w.dim() != 2 or w.shape != (T, g.shape[1]):
+            raise ValueError(f"edge_weight of graph {b} must be [T={T}, E={g.shape[1]}], got {tuple(w.shape)}")
+    values = torch.zeros((T, max(pat.nnz, 1)), dtype=torch.float32, device=device)
+    for w, m in zip(ws, pat.edge_map):
+        values.index_add_(1, m, w)
+    sc = _new_sparse_control(ts, pat, T, device)
+    sp = sc.sparse_struct()
+    check(lib().pegncde_build_adj_sparse(_stream_ptr(device), _sparse_dims(pat, T), sp, pat.perm_t.data_ptr(), sc.ts.data_ptr(),
+                                         values.data_ptr(), sc.adj_rowsum.data_ptr(), sc.adj_diag.data_ptr(), sc.adj_total.data_ptr(),
+                                         sc.adj_colsum.data_ptr(), sc.tch_coef.data_ptr()), "pegncde_build_adj_sparse")
+    if x_t is not None:
+        _attach_x(sc, _node_signal_coeffs(sc.ts, x_t, pat.B, T, pat.n, device), device)
+    sc._keepalive = values      # the source lives until the builder has run (stream-ordered)
+    return sc
+
+
+def pack_sparse_control(ts: torch.Tensor, edge_index, coeffs_adj, x_coeffs=None, num_nodes: Optional[int] = None,
+                        device=None) -> SparseControl:
+    """Coefficients on an edge list -> :class:`SparseControl` (``pegncde_pack_adj_sparse``): the sparse form of
+    :func:`pack_control`'s ``coeffs_adj``.
+
+    ``coeffs_adj``: ``(d, c, b, a)`` each ``[T-1, E]`` -- the adjacency channel only (the time channel is t itself) -- or a list of B
+    such tuples, one per pattern of ``edge_index``.  Linear interpolation is ``c = d = 0``.  ``x_coeffs`` as in :func:`pack_control`.
+    ``num_nodes`` defaults to the node count of ``x_coeffs`` (required without it)."""
+    graphs = _edge_list(edge_index)
+    device = torch.device(device if device is not None else graphs[0].device)
+    if device.type != "cuda":
+        raise RuntimeError("pack_sparse_control needs a CUDA device: the fused path has no CPU fallback")
+    if num_nodes is None:
+        if x_coeffs is None:
+            raise ValueError("num_nodes is required without x_coeffs")
+        num_nodes = int((x_coeffs[0] if not isinstance(x_coeffs, torch.Tensor) else x_coeffs[0]).shape[-3])
+    pat = sparse_pattern([g.to(device) for g in graphs], num_nodes)
+    one_graph = isinstance(coeffs_adj, torch.Tensor) or (len(coeffs_adj) == 4 and all(isinstance(c, torch.Tensor) for c in coeffs_adj))
+    per = _per_graph([coeffs_adj] if one_graph else list(coeffs_adj), pat.B, "coeffs_adj")
+    Tm1 = None
+    for b, (co, g) in enumerate(zip(per, graphs)):
+        if len(co) != 4:
+            raise ValueError("coeffs_adj must be (d, c, b, a)")
+        co = [c.to(device=device, dtype=torch.float32) for c in co]
+        Tm1 = co[0].shape[0] if Tm1 is None else Tm1
+        for c in co:
+            if c.dim() != 2 or c.shape != (Tm1, g.shape[1]):
+                raise ValueError(f"coefficients of graph {b} must be [T-1={Tm1}, E={g.shape[1]}], got {tuple(c.shape)}")
+        per[b] = co
+    cf = [torch.zeros((Tm1, max(pat.nnz, 1)), dtype=torch.float32, device=device) for _ in range(4)]
+    for co, m in zip(per, pat.edge_map):
+        for q in range(4):
+            cf[q].index_add_(1, m, co[q])
+    sc = _new_sparse_control(ts, pat, Tm1 + 1, device)
+    sp = sc.sparse_struct()
+    check(lib().pegncde_pack_adj_sparse(_stream_ptr(device), _sparse_dims(pat, Tm1 + 1), sp, pat.perm_t.data_ptr(), cf[0].data_ptr(),
+                                        cf[1].data_ptr(), cf[2].data_ptr(), cf[3].data_ptr(), sc.adj_rowsum.data_ptr(),
+                                        sc.adj_diag.data_ptr(), sc.adj_total.data_ptr(), sc.adj_colsum.data_ptr(),
+                                        sc.tch_coef.data_ptr()), "pegncde_pack_adj_sparse")
+    if x_coeffs is not None:
+        _attach_x(sc, x_coeffs, device)
+    sc._keepalive = cf
+    return sc

@@ -14,6 +14,17 @@ namespace peg {
 // reference layout: d,c,b,a each [B, T-1, n, n, 2], last axis (time, adjacency)
 // =====================================================================================
 
+// diffrax.backward_hermite_coefficients of one element on one cubic piece (the dense and the sparse builders share it, so both give
+// the same bits): a = y0, b = previous secant (first piece: own secant), c = 2 (m - b) / dt, d = -(m - b) / dt^2
+__device__ __forceinline__ void hermite_piece(float y0, float y1, float yprev, bool first, float dt, float dtp, float (&hv)[4]) {
+  const float m = (y1 - y0) / dt;
+  const float bb = first ? m : (y0 - yprev) / dtp;
+  hv[0] = y0;
+  hv[1] = bb;
+  hv[2] = 2.0f * (m - bb) / dt;
+  hv[3] = -(m - bb) / (dt * dt);
+}
+
 // grid (nt column tiles, T-1, B), block 256: one block per COLUMN of 32x32 tiles, walked top to bottom.  Source is the
 // reference layout (d,c,b,a each [B,T-1,n,n,2]), or the already tiled planes (tiled_in, pegncde_adj_stats), or the raw graph
 // snapshots A_k [B,T,n,n] + knot times (snap / ts, pegncde_build_adj: backward_hermite_coefficients fused in,
@@ -61,17 +72,11 @@ __global__ void __launch_bounds__(256) k_pack_adj(const float* __restrict__ cd, 
       const int i = rt * 32 + r, k = ct * 32 + c;
       float hv[4] = {0.f, 0.f, 0.f, 0.f};
       if (snap && i < n && k < ncols) {
-        // diffrax.backward_hermite_coefficients per element: a = y_i, b = previous secant (first piece: own secant),
-        // c = 2 (m - b) / dt, d = -(m - b) / dt^2
         const float* Ab = snap + ((size_t)b * (Tm1 + 1) * n + i) * (size_t)ncols + k;
         const size_t knot = (size_t)n * ncols;
         const float y0 = __ldg(Ab + (size_t)iv * knot), y1 = __ldg(Ab + (size_t)(iv + 1) * knot);
-        const float m = (y1 - y0) / dt;
-        const float bb = iv > 0 ? (y0 - __ldg(Ab + (size_t)(iv - 1) * knot)) / dtp : m;
-        hv[0] = y0;
-        hv[1] = bb;
-        hv[2] = 2.0f * (m - bb) / dt;
-        hv[3] = -(m - bb) / (dt * dt);
+        const float yp = iv > 0 ? __ldg(Ab + (size_t)(iv - 1) * knot) : 0.f;
+        hermite_piece(y0, y1, yp, iv == 0, dt, dtp, hv);
       }
 #pragma unroll
       for (int p = 0; p < 4; ++p) {
@@ -861,6 +866,45 @@ __global__ void __launch_bounds__(256) k_colsums(const float* __restrict__ V, in
 
 constexpr int CT_TI = 64, CT_TC = 64, CT_KC = 16, CT_LD = CT_TI + 4;
 
+// Epilogue of the contraction for row gi, columns gc..gc+3 (shared by k_dual_contract and k_sparse_contract in peg_sparse.cuh).
+// acc[.][i] = the products of this row (forward: [0] = X V + Y^T V; backward: A V, A'V, A^T V, A'^T V), ss / tt = the column sums
+// 1^T V / vec^T V of these columns, Vb = V of graph b, alpha..delta = 1 + p1_0, 1 + p1_1, p2_0, p2_1.  Writes OUT; backward: adds the param1 / param2
+// Frobenius-product terms of this row to g4.
+template <int NACC, int R>
+__device__ __forceinline__ void contract_epilogue4(const ContractArgs& a, int b, int gi, int gc, const float* __restrict__ sv, const float* Vb,
+                                                   const float (&acc)[NACC][R][4], int i, const float (&ss)[4], const float (&tt)[4],
+                                                   float kappa, float alpha, float beta, float gamma, float delta, float (&g4)[4]) {
+  const int n = a.n, d = a.d;
+  const float vi = 1.f + sv[a.v_off + gi];
+  const float rc = sv[a.rowc_off + gi];
+  const float tg = a.scale_tg ? sv[a.tg_off + gi] : 1.f;
+  const float4 vin = *reinterpret_cast<const float4*>(Vb + (size_t)gi * d + gc);
+  const float vv[4] = {vin.x, vin.y, vin.z, vin.w};
+  float o[4];
+  if (NACC == 1) {
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      float val = vv[j] * vi + acc[0][i][j] + rc * ss[j] + tt[j] + kappa * ss[j];
+      if (a.relu) val = fmaxf(val, 0.f);
+      o[j] = val * tg;
+    }
+  } else {
+    const float4 m4 = *reinterpret_cast<const float4*>(a.Mref + ((size_t)b * n + gi) * d + gc);
+    const float mm[4] = {m4.x, m4.y, m4.z, m4.w};
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      // acc[0]=A V, acc[1]=A'V, acc[2]=A^T V, acc[3]=A'^T V   (V = cotangent of the layer output)
+      o[j] = vv[j] * vi + alpha * acc[2][i][j] + beta * acc[3][i][j] + gamma * acc[0][i][j] +
+             delta * acc[1][i][j] + rc * ss[j] + tt[j] + kappa * ss[j];
+      g4[0] = fmaf(acc[2][i][j], mm[j], g4[0]);  // d/d param1[0] = <A^T g, M>
+      g4[1] = fmaf(acc[3][i][j], mm[j], g4[1]);  // d/d param1[1] = <A'^T g, M>
+      g4[2] = fmaf(acc[0][i][j], mm[j], g4[2]);  // d/d param2[0] = <A g, M>
+      g4[3] = fmaf(acc[1][i][j], mm[j], g4[3]);  // d/d param2[1] = <A' g, M>
+    }
+  }
+  *reinterpret_cast<float4*>(a.out + ((size_t)b * n + gi) * d + gc) = make_float4(o[0], o[1], o[2], o[3]);
+}
+
 template <int NACC>
 __global__ void __launch_bounds__(256) k_dual_contract(ContractArgs a) {
   constexpr int NS = (NACC == 1) ? 2 : 4;
@@ -1000,34 +1044,7 @@ __global__ void __launch_bounds__(256) k_dual_contract(ContractArgs a) {
     for (int i = 0; i < 4; ++i) {
       const int gi = i0 + 4 * ty + i;
       if (gi >= n) continue;
-      const float vi = 1.f + sv[a.v_off + gi];
-      const float rc = sv[a.rowc_off + gi];
-      const float tg = a.scale_tg ? sv[a.tg_off + gi] : 1.f;
-      const float4 vin = *reinterpret_cast<const float4*>(Vb + (size_t)gi * d + gc);
-      const float vv[4] = {vin.x, vin.y, vin.z, vin.w};
-      float o[4];
-      if (NACC == 1) {
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          float val = vv[j] * vi + acc[0][i][j] + rc * ss[j] + tt[j] + kappa * ss[j];
-          if (a.relu) val = fmaxf(val, 0.f);
-          o[j] = val * tg;
-        }
-      } else {
-        const float4 m4 = *reinterpret_cast<const float4*>(a.Mref + ((size_t)b * n + gi) * d + gc);
-        const float mm[4] = {m4.x, m4.y, m4.z, m4.w};
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          // acc[0]=A V, acc[1]=A'V, acc[2]=A^T V, acc[3]=A'^T V   (V = cotangent of the layer output)
-          o[j] = vv[j] * vi + alpha * acc[2][i][j] + beta * acc[3][i][j] + gamma * acc[0][i][j] +
-                 delta * acc[1][i][j] + rc * ss[j] + tt[j] + kappa * ss[j];
-          g4[0] = fmaf(acc[2][i][j], mm[j], g4[0]);  // d/d param1[0] = <A^T g, M>
-          g4[1] = fmaf(acc[3][i][j], mm[j], g4[1]);  // d/d param1[1] = <A'^T g, M>
-          g4[2] = fmaf(acc[0][i][j], mm[j], g4[2]);  // d/d param2[0] = <A g, M>
-          g4[3] = fmaf(acc[1][i][j], mm[j], g4[3]);  // d/d param2[1] = <A' g, M>
-        }
-      }
-      *reinterpret_cast<float4*>(a.out + ((size_t)b * n + gi) * d + gc) = make_float4(o[0], o[1], o[2], o[3]);
+      contract_epilogue4<NACC, 4>(a, b, gi, gc, sv, Vb, acc, i, ss, tt, kappa, alpha, beta, gamma, delta, g4);
     }
   }
   if (NACC == 4) {

@@ -7,6 +7,7 @@
 
 #include "peg_kernels.cuh"
 #include "peg_small.cuh"
+#include "peg_sparse.cuh"
 #include "peg_tc.cuh"
 
 namespace peg {
@@ -206,7 +207,7 @@ static int stage_prep(Ctx& c, float t) {
 static ProducerOut producer_out(Ctx& c, int dcols, bool want_vt, float* cb, bool with_vec, size_t vec_off, bool bfp_capable) {
   ProducerOut po;
   memset(&po, 0, sizeof(po));
-  if (want_vt && c.use_tc && tc_supported(c.d, dcols) && (c.w.tc.fmt != PEG_FMT_FP16X2 || bfp_capable)) {
+  if (want_vt && c.use_tc && !c.ctl.sparse && tc_supported(c.d, dcols) && (c.w.tc.fmt != PEG_FMT_FP16X2 || bfp_capable)) {
     po.Thi = c.w.tc.Vt_hi;
     po.Tlo = c.w.tc.Vt_lo;
     po.npad = c.w.tc.npad;
@@ -306,7 +307,7 @@ static void shard_select_half(Ctx& c) {
   c.w.tc.vexp = sh.vexp[sh.rank] + (size_t)(next & 1u) * c.d.B * c.w.tc.vexp_stride;
 }
 
-static bool contract_on_tc(const Ctx& c, int l) { return c.use_tc && tc_supported(c.d, c.m.layer[l].dout); }
+static bool contract_on_tc(const Ctx& c, int l) { return c.use_tc && !c.ctl.sparse && tc_supported(c.d, c.m.layer[l].dout); }
 
 static int contract(Ctx& c, int l, bool bwd, const float* V, const float* Mref, const float* colbuf, float* out,
                     bool relu, bool scale_tg, float* g_fus, bool vt_ready, const float* cbM = nullptr) {
@@ -340,12 +341,29 @@ static int contract(Ctx& c, int l, bool bwd, const float* V, const float* Mref, 
   // algorithmic work of one launch: the four coefficient planes are traversed once (16 n^2 B per graph),
   // V is read and OUT written once; 2 (fwd) or 4 (bwd) n x n x d products.
   const double nn = (double)c.d.n * c.d.n, nd = (double)c.d.n * ld.dout;
-  const double bytes = c.d.B * (16.0 * nn + 4.0 * nd * (bwd ? 3.0 : 2.0));
-  const double flops = c.d.B * (bwd ? 8.0 : 4.0) * nn * ld.dout;
+  double bytes = c.d.B * (16.0 * nn + 4.0 * nd * (bwd ? 3.0 : 2.0));
+  double flops = c.d.B * (bwd ? 8.0 : 4.0) * nn * ld.dout;
+  if (c.ctl.sparse) {
+    // sparse path: both orientations' coefficients (one piece) and columns, both row-pointer arrays, V and OUT once (+ M in the
+    // adjoint).  The gathers of V rows (2 nnz d 4 bytes, mostly served from L2) are not HBM traffic and are not counted here.
+    const double nnz = (double)c.ctl.sparse->nnz;
+    bytes = 2.0 * nnz * (16.0 + 4.0) + 2.0 * c.d.B * (c.d.n + 1.0) * 4.0 + c.d.B * 4.0 * nd * (bwd ? 3.0 : 2.0);
+    flops = (bwd ? 8.0 : 4.0) * nnz * ld.dout;
+  }
   const int dir = bwd ? 1 : 0;
   const bool timed = prof_begin(dir, c.st, bytes, flops);
   int rc = PEG_OK;
-  if (c.sh) {
+  if (c.ctl.sparse) {
+    const int glog = sparse_glog(ld.dout), G = 1 << glog;
+    dim3 grid((unsigned)((c.d.n + 8 * (32 / G) - 1) / (8 * (32 / G))), (unsigned)((ld.dout + 4 * G - 1) / (4 * G)), c.d.B);
+    if (!bwd)
+      k_sparse_contract<1><<<grid, 256, 0, c.st>>>(a, *c.ctl.sparse, glog);
+    else
+      k_sparse_contract<4><<<grid, 256, 0, c.st>>>(a, *c.ctl.sparse, glog);
+    g_launches.fetch_add(1);
+    cudaError_t e = cudaPeekAtLastError();
+    if (e != cudaSuccess) { g_last_cuda = (int)e; (void)cudaGetLastError(); rc = PEG_ERR_CUDA; }
+  } else if (c.sh) {
     // row-sharded: every rank needs ALL rows of V^T and the column sums over ALL nodes -> convert V if no producer did, then the
     // exchange over peer memory (push + flags, wait + rank-ordered column sums), then the local row blocks of the contraction
     if (!vt_ready) { rc = tc_convert_v(c.st, c.d, c.w.tc, a); g_launches.fetch_add(c.w.tc.fmt == PEG_FMT_FP16X2 ? 2 : 1); }
@@ -382,7 +400,7 @@ static void small_plan(Ctx& c) {
   if (d.flags & PEG_FLAG_NO_FUSED_SMALL) return;
   // default: below the smallest tcgen05 shape; PEG_FLAG_FUSED_SMALL widens it
   const int max_n = (d.flags & PEG_FLAG_FUSED_SMALL) ? 256 : 127;
-  if (c.sh || c.m.directed || d.n > max_n || d.n > SG_MAX_N || d.h > SG_MAX_DIN) return;
+  if (c.sh || c.ctl.sparse || c.m.directed || d.n > max_n || d.n > SG_MAX_N || d.h > SG_MAX_DIN) return;
   const size_t smem = small_smem_floats(d.n, d.L) * sizeof(float);
   if (smem > 220 * 1024) return;
   int dev = 0, sm_count = 0;
@@ -592,14 +610,27 @@ static int combine(Ctx& c, float* out, int cnt, const float* const* xs, const do
   return PEG_OK;
 }
 
+// a PegSparse the kernels can walk: every array present, coefficient slabs 16-byte aligned (one float4 per entry)
+static int check_sparse(const PegSparse* sp) {
+  if (!sp->row_ptr || !sp->col || !sp->coef || !sp->row_ptr_t || !sp->col_t || !sp->coef_t) return PEG_ERR_NULL_POINTER;
+  if (sp->nnz < 0 || sp->nnz > INT32_MAX || sp->nnz_stride < sp->nnz) return PEG_ERR_BAD_DIMS;
+  if ((((uintptr_t)sp->coef | (uintptr_t)sp->coef_t) & 15) != 0) return PEG_ERR_ALIGNMENT;
+  return PEG_OK;
+}
+
 static int make_ctx(Ctx& c, peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params) {
   PEG_TRY(check_dims(dims));
   if (!ctl || !params) return PEG_ERR_NULL_POINTER;
-  if (!ctl->ts || !ctl->adj_coef || !ctl->adj_rowsum || !ctl->adj_diag || !ctl->adj_total || !ctl->tch_coef)
+  if (!ctl->ts || (!ctl->adj_coef && !ctl->sparse) || !ctl->adj_rowsum || !ctl->adj_diag || !ctl->adj_total || !ctl->tch_coef)
     return PEG_ERR_NULL_POINTER;
   if (dims->e > 0 && !ctl->x_coef) return PEG_ERR_NULL_POINTER;
   if ((dims->flags & PEG_FLAG_DIRECTED) && !ctl->adj_colsum) return PEG_ERR_NULL_POINTER;
-  if (((uintptr_t)ctl->adj_coef & 15) != 0) return PEG_ERR_ALIGNMENT;
+  if (ctl->sparse) {
+    if (ctl->shard) return PEG_ERR_UNSUPPORTED;     // row-sharded sparse controls are not implemented
+    PEG_TRY(check_sparse(ctl->sparse));
+  } else if (((uintptr_t)ctl->adj_coef & 15) != 0) {
+    return PEG_ERR_ALIGNMENT;
+  }
   c.st = (cudaStream_t)stream;
   c.d = *dims;
   c.ctl = *ctl;
@@ -843,6 +874,41 @@ int pegncde_build_adj_rect(peg_stream_t stream, const PegDims* dims, int32_t n_c
     PEG_LAUNCH_CHECK();
   }
   return PEG_OK;
+}
+
+static int sparse_common(peg_stream_t stream, const PegDims* dims, const PegSparse* sp, const int32_t* perm_t, const float* ts,
+                         const float* values, const float* d, const float* c, const float* b, const float* a, float* adj_rowsum,
+                         float* adj_diag, float* adj_total, float* adj_colsum, float* tch_coef) {
+  PEG_TRY(check_dims(dims));
+  if (!sp || !perm_t || !adj_rowsum || !adj_diag || !adj_total || !adj_colsum || !tch_coef) return PEG_ERR_NULL_POINTER;
+  PEG_TRY(check_sparse(sp));
+  cudaStream_t st = (cudaStream_t)stream;
+  const int Tm1 = dims->T - 1, n = dims->n;
+  const dim3 grid((unsigned)((n + 7) / 8), Tm1, dims->B);
+  k_sparse_build<<<grid, 256, 0, st>>>(*sp, perm_t, ts, values, d, c, b, a, n, Tm1, adj_rowsum, adj_diag);
+  PEG_LAUNCH_CHECK();
+  k_sparse_colsums<<<grid, 256, 0, st>>>(*sp, n, Tm1, adj_colsum);
+  PEG_LAUNCH_CHECK();
+  k_adj_totals<<<dim3(4 * Tm1, dims->B), 256, 0, st>>>(adj_rowsum, n, Tm1, 0, adj_total);
+  PEG_LAUNCH_CHECK();
+  const size_t slabs = (size_t)dims->B * Tm1;
+  k_fill_tch_unit<<<(unsigned)((slabs * 3 * n + 255) / 256), 256, 0, st>>>(tch_coef, n, slabs);
+  PEG_LAUNCH_CHECK();
+  return PEG_OK;
+}
+
+int pegncde_build_adj_sparse(peg_stream_t stream, const PegDims* dims, const PegSparse* sp, const int32_t* perm_t, const float* ts,
+                             const float* values, float* adj_rowsum, float* adj_diag, float* adj_total, float* adj_colsum, float* tch_coef) {
+  if (!ts || !values) return PEG_ERR_NULL_POINTER;
+  return sparse_common(stream, dims, sp, perm_t, ts, values, nullptr, nullptr, nullptr, nullptr, adj_rowsum, adj_diag, adj_total,
+                       adj_colsum, tch_coef);
+}
+
+int pegncde_pack_adj_sparse(peg_stream_t stream, const PegDims* dims, const PegSparse* sp, const int32_t* perm_t, const float* d,
+                            const float* c, const float* b, const float* a, float* adj_rowsum, float* adj_diag, float* adj_total,
+                            float* adj_colsum, float* tch_coef) {
+  if (!d || !c || !b || !a) return PEG_ERR_NULL_POINTER;
+  return sparse_common(stream, dims, sp, perm_t, nullptr, nullptr, d, c, b, a, adj_rowsum, adj_diag, adj_total, adj_colsum, tch_coef);
 }
 
 int pegncde_pack_x(peg_stream_t stream, const PegDims* dims, const float* d, const float* c, const float* b,

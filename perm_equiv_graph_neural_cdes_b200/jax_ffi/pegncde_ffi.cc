@@ -31,7 +31,8 @@ template <typename Buf>
 static int32_t batch_of(const Buf& y, int32_t n, int32_t h) { return (int32_t)(y.element_count() / ((size_t)n * h)); }
 static PegControl control_of(const float* ts, const float* adj_coef, const float* adj_rowsum, const float* adj_diag, const float* adj_total,
                              const float* tch_coef, const float* x_coef, const float* adj_absmax) {
-  PegControl c{ts, adj_coef, adj_rowsum, adj_diag, adj_total, tch_coef, x_coef, /*adj_colsum=*/nullptr, adj_absmax, /*shard=*/nullptr};
+  PegControl c{ts, adj_coef, adj_rowsum, adj_diag, adj_total, tch_coef, x_coef, /*adj_colsum=*/nullptr, adj_absmax, /*shard=*/nullptr,
+               /*sparse=*/nullptr};   // the handlers take dense planes only
   return c;
 }
 

@@ -52,6 +52,8 @@ class RowShardedControl:
 
     def __init__(self, ts: torch.Tensor, snapshots_rows: torch.Tensor, snapshots_cols_t: torch.Tensor, hidden_dim: int, num_layers: int,
                  group=None, flags: int = 1):
+        if isinstance(snapshots_rows, PackedControl) or isinstance(snapshots_cols_t, PackedControl):
+            raise TypeError("RowShardedControl takes dense snapshot strips; sparse (CSR) controls cannot be row-sharded")
         dev = snapshots_rows.device
         self.group = group
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
