@@ -312,7 +312,14 @@ int pegncde_solve_fwd(peg_stream_t stream, const PegDims* dims, const PegControl
                       float* stage_store, void* workspace, size_t workspace_bytes);
 /* stage_store (nullable, pegncde_stage_store_bytes() bytes): when given, solve_fwd keeps the input of every layer
  * of every stage there and solve_bwd, handed the same buffer, skips its forward recompute (36 instead of 54 passes
- * over the coefficient planes per step).  NULL = checkpoint-per-step mode: solve_bwd recomputes each step. */
+ * over the coefficient planes per step).  NULL = checkpoint-per-step mode: solve_bwd recomputes each step.
+ * Layout, per step and stage 0..5 (steps x 6 blocks of equal size):
+ *   L slots [B,n,h]: the input of every layer (layer 0 of stage 0 is y_ckpt[step] itself, that slot stays unused);
+ *   K slots [B,n,h]: M_l = Linear(RMSNorm(input)) of the layers whose output is h wide, K = L (e == 0) or L - 1 (e > 0: the
+ *                    last layer is 2he wide and is recomputed);
+ *   K slots [B][2][h]: the column sums of those M_l (plain and weighted by the layer's contraction vector).
+ * The tensor-core adjoint reads M_l back instead of recomputing it.  A caller streaming the solve in segments offsets the
+ * buffer by pegncde_stage_store_bytes(dims, 1) per step. */
 size_t pegncde_stage_store_bytes(const PegDims* dims, int32_t steps);
 /* g_ckpt (nullable) [steps+1, B, n, h]: cotangents injected at step boundaries (SaveAt(steps) losses);
  * g_yT [B,n,h] cotangent of y(T) (either of the two may be NULL, not both).

@@ -1045,7 +1045,7 @@ int tc_contract(cudaStream_t st, const PegDims& dm, const TcWs& w, const Contrac
 // One CTA per 128 nodes x ND outputs: M = 128 (nodes), N = ND, K = din in chunks of 32.
 //   warps 0-7 : load Z rows (coalesced LDG.128, all K chunks of a 128-wide super chunk in flight at once), accumulate
 //               sum z^2, 3xTF32-split into the swizzled K-major A tiles; afterwards the epilogue (tcgen05.ld):
-//               norm scale + bias, M, V^T hi/lo (coalesced: lane = node), deterministic column sums, optional N
+//               norm scale + bias, M, V^T hi/lo (coalesced: lane = node), deterministic column sums
 //   warp 8    : TMA producer of the weight tiles (hi / lo, SWIZZLE_128B);  warp 9: TMEM allocator + MMA issuer
 // grid (ceil(n/128), dout/ND, B), block 320
 // ==========================================================================================
@@ -1085,10 +1085,7 @@ constexpr int NL_THREADS = 320;
 struct NlParams {
   const float* Z;      // [B,n,din]
   const float* cvec;   // [dout]
-  const float* nw;     // norm weight / bias (only for Nout)
-  const float* nb;
   float* M;            // [B,n,dout]
-  float* Nout;         // nullable [B,n,din]
   ProducerOut po;
   int n, din, dout, nd, stages, tmem_cols, nsplit;
 };
@@ -1293,21 +1290,6 @@ k_tc_norm_linear(const __grid_constant__ CUtensorMap map_hi, const __grid_consta
       }
     }
     tc_fence_before();
-    if (p.Nout != nullptr && ntile == 0) {   // normalised input, needed by the weight gradient
-      float* Nb = p.Nout + (size_t)b * n * din;
-      const int lr = tid >> 3, lc = tid & 7;
-      for (int i = 0; i < 4; ++i) {
-        const int rr = 32 * i + lr, rowg = row0 + rr;
-        if (rowg >= n) continue;
-        const float rv = rinv_s[rr];
-        for (int k = lc * 4; k < din; k += 32) {
-          const float4 z4 = __ldg(reinterpret_cast<const float4*>(Zb + (size_t)rowg * din + k));
-          const float4 s4 = __ldg(reinterpret_cast<const float4*>(p.nw + k)), t4 = __ldg(reinterpret_cast<const float4*>(p.nb + k));
-          *reinterpret_cast<float4*>(Nb + (size_t)rowg * din + k) =
-              make_float4(z4.x * rv * s4.x + t4.x, z4.y * rv * s4.y + t4.y, z4.z * rv * s4.z + t4.z, z4.w * rv * s4.w + t4.w);
-        }
-      }
-    }
   }
   __syncthreads();
   if (p.po.cb != nullptr) {
@@ -1390,12 +1372,12 @@ int tc_prep_weights(cudaStream_t st, const Model& m, const float* params, const 
   return PEG_OK;
 }
 
-int tc_norm_linear(cudaStream_t st, const PegDims& dm, const TcLinear& w, int layer, const float* Z, int din, int dout,
-                   const float* nw, const float* nb, float* M, float* Nout, const ProducerOut& po) {
+int tc_norm_linear(cudaStream_t st, const PegDims& dm, const TcLinear& w, int layer, const float* Z, int din, int dout, float* M,
+                   const ProducerOut& po) {
   if (!w.ready) return PEG_ERR_WORKSPACE;
   NlParams p;
   memset(&p, 0, sizeof(p));
-  p.Z = Z; p.cvec = w.cvec[layer]; p.nw = nw; p.nb = nb; p.M = M; p.Nout = Nout; p.po = po;
+  p.Z = Z; p.cvec = w.cvec[layer]; p.M = M; p.po = po;
   p.n = dm.n; p.din = din; p.dout = dout;
   p.nd = nl_pick_nd(dout);
   p.nsplit = (dm.flags & PEG_FLAG_TF32_FAST) ? 1 : 3;
@@ -1433,17 +1415,27 @@ int tc_norm_linear(cudaStream_t st, const PegDims& dm, const TcLinear& w, int la
 //   Zbar = rinv w Nbar - z rinv^3 <w Nbar, z> / din ; optional ReLU mask (z > 0) ; g_nw += sum Nbar zhat ; g_nb += sum Nbar
 // plus the producer outputs of Zbar (V^T hi/lo, deterministic column sums) for the next adjoint contraction.
 // A thread of the epilogue owns one node: the per-node reductions are thread-local apart from one exchange between the
-// two column halves; per-column reductions use the butterfly above.  grid (ceil(n/128), 1, B), block 320
+// two column halves; per-column reductions use the butterfly above.
+// The Linear's own gradient needs the normalised input N = z rinv nw + nb, which this kernel has at hand:
+//   dout == 128 (gW set): Wbar += Mbar^T N and bbar += 1^T Mbar of the CTA's 128 nodes on tcgen05 as well.  The epilogue stores
+//     both operands transposed (node = K) into the idle operand ring, one 32-node K step per warp quarter, and a second TMEM
+//     accumulator takes the 128 x din partial, which is added with vector atomics.
+//   otherwise (Nout set): N is written out for k_tc_weight_grad.
+// grid (ceil(n/128), 1, B), block 320
 // ==========================================================================================
 struct LbParams {
   const float* Mbar;   // [B,n,dout]
   const float* Z;      // [B,n,din]
   const float* nw;     // [din]
+  const float* nb;     // [din]
   float* Zbar;         // [B,n,din]
   float* g_nw;
   float* g_nb;
+  float* gW;           // nullable [dout][din]: fused weight gradient (dout == 128)
+  float* gb;           // [dout] (with gW)
+  float* Nout;         // nullable [B,n,din]
   ProducerOut po;
-  int n, din, dout, stages, tmem_cols, nsplit, relu_mask;
+  int n, din, dout, stages, tmem_cols, nsplit, relu_mask, wg_col;
 };
 
 __global__ void __launch_bounds__(NL_THREADS, 1)
@@ -1464,22 +1456,30 @@ k_tc_linear_bwd(const __grid_constant__ CUtensorMap map_hi, const __grid_constan
   const int b_tile = nd * TC_BK * 4;
   const int b_bytes = (split ? 2 : 1) * b_tile;
   const int stage_bytes = a_bytes + b_bytes;
-  const uint32_t bar_base = smem_base + S * stage_bytes;
+  const bool wg = p.gW != nullptr;
+  uint8_t* smem_gen = smem_raw + (smem_base - smem_u32(smem_raw));
+  float* csum = reinterpret_cast<float*>(smem_gen + S * stage_bytes);   // [4 row quarters][4 sums][din]
+  float* bsum = csum + 16 * din;                                        // [4 row quarters][dout] (wg)
+  const uint32_t bar_base = smem_base + S * stage_bytes + (16 * din + (wg ? 4 * dout : 0)) * 4;
   auto full_a = [&](int s) { return bar_base + 8u * s; };
   auto full_b = [&](int s) { return bar_base + 8u * (S + s); };
   auto empty = [&](int s) { return bar_base + 8u * (2 * S + s); };
-  const uint32_t accum_bar = bar_base + 8u * (3 * S);
-  const uint32_t tmem_slot = accum_bar + 8u;
-  uint8_t* smem_gen = smem_raw + (smem_base - smem_u32(smem_raw));
-  float* csum = reinterpret_cast<float*>(smem_gen);   // [4 row quarters][4 sums][din]: reuses stage 0 after the MMAs
+  auto wg_full = [&](int s) { return bar_base + 8u * (3 * S + s); };
+  auto wg_free = [&](int s) { return bar_base + 8u * (4 * S + s); };
+  const uint32_t accum_bar = bar_base + 8u * (5 * S);
+  const uint32_t wg_bar = accum_bar + 8u;
+  const uint32_t tmem_slot = wg_bar + 8u;
 
   if (tid == 0) {
     for (int s = 0; s < S; ++s) {
       mbar_init(full_a(s), 256);
       mbar_init(full_b(s), 1);
       mbar_init(empty(s), 1);
+      mbar_init(wg_full(s), 64);
+      mbar_init(wg_free(s), 1);
     }
     mbar_init(accum_bar, 1);
+    mbar_init(wg_bar, 1);
     fence_barrier_init();
   }
   if (warp == 9) {
@@ -1561,6 +1561,26 @@ k_tc_linear_bwd(const __grid_constant__ CUtensorMap map_hi, const __grid_constan
         umma_commit(empty(st));
       }
       umma_commit(accum_bar);
+      if (wg) {   // Wbar partial: K = the 128 nodes, one 32-node step per warp quarter of the epilogue, step c in ring slot c % S
+        for (int c = 0; c < 4; ++c) {
+          const int st = c % S;
+          mbar_wait(wg_full(st), (uint32_t)(c / S) & 1u);
+          tc_fence_after();
+          const uint32_t ahi = smem_base + st * stage_bytes, alo = ahi + TC_ATILE;
+          const uint32_t bhi = ahi + a_bytes, blo = bhi + b_tile;
+#pragma unroll
+          for (int k8 = 0; k8 < TC_BK / 8; ++k8) {
+            const uint64_t dah = make_desc_sw128(ahi + k8 * 32), dbh = make_desc_sw128(bhi + k8 * 32);
+            umma_tf32(tmem_base + (uint32_t)p.wg_col, dah, dbh, idesc, (c > 0 || k8 > 0) ? 1u : 0u);
+            if (split) {
+              umma_tf32(tmem_base + (uint32_t)p.wg_col, make_desc_sw128(alo + k8 * 32), dbh, idesc, 1u);
+              umma_tf32(tmem_base + (uint32_t)p.wg_col, dah, make_desc_sw128(blo + k8 * 32), idesc, 1u);
+            }
+          }
+          umma_commit(wg_free(st));
+        }
+        umma_commit(wg_bar);
+      }
     }
   }
 
@@ -1601,6 +1621,43 @@ k_tc_linear_bwd(const __grid_constant__ CUtensorMap map_hi, const __grid_constan
     dot = red_s[0][1][row] + red_s[1][1][row];
     const float rinv = rsqrtf(ss / (float)din + 1e-5f);
     const float coef = rinv * rinv * rinv * dot / (float)din;
+    if (wg) {
+      // K step q of the weight gradient: this quarter's 32 nodes (lane = K index) into ring slot q % S, which the main MMAs have
+      // released (accum_bar) or the weight-gradient MMA of step q - S frees.  A' = Mbar^T (row = output), B' = N^T (row = input).
+      const int st = q % S;
+      if (q >= S) mbar_wait(wg_free(st), 0u);
+      const uint32_t a_base = smem_base + st * stage_bytes, b_base = a_base + a_bytes;
+      auto put = [&](uint32_t tile, uint32_t lo_off, int r, float x) {
+        const uint32_t off = (uint32_t)(r >> 3) * 1024u + (uint32_t)(r & 7) * 128u + ((uint32_t)((lane >> 2) ^ (r & 7)) << 4) + (uint32_t)(lane & 3) * 4u;
+        const float h = tf32_rna(x);
+        asm volatile("st.shared.f32 [%0], %1;" ::"r"(tile + off), "f"(h) : "memory");
+        if (split) asm volatile("st.shared.f32 [%0], %1;" ::"r"(tile + lo_off + off), "f"(x - h) : "memory");
+      };
+      const float* Mrow = Mb + (size_t)(rowok ? gi : 0) * dout;
+      for (int oc = half * (dout / 2); oc < (half + 1) * (dout / 2); oc += 16) {
+        float m[16];
+#pragma unroll
+        for (int v4 = 0; v4 < 4; ++v4) {
+          const float4 m4 = rowok ? __ldg(reinterpret_cast<const float4*>(Mrow + oc + 4 * v4)) : make_float4(0.f, 0.f, 0.f, 0.f);
+          m[4 * v4] = m4.x; m[4 * v4 + 1] = m4.y; m[4 * v4 + 2] = m4.z; m[4 * v4 + 3] = m4.w;
+        }
+#pragma unroll
+        for (int u = 0; u < 16; ++u) put(a_base, TC_ATILE, oc + u, m[u]);
+        warp_colsum16(m, lane);
+        if ((lane & 1) == 0) bsum[q * dout + oc + warp_col16(lane)] = m[0];
+      }
+      for (int kc = half * (din / 2); kc < (half + 1) * (din / 2); kc += 4) {
+        float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (rowok) z4 = *reinterpret_cast<const float4*>(Zrow + kc);
+        const float4 s4 = __ldg(reinterpret_cast<const float4*>(p.nw + kc)), t4 = __ldg(reinterpret_cast<const float4*>(p.nb + kc));
+        put(b_base, b_tile, kc + 0, rowok ? z4.x * rinv * s4.x + t4.x : 0.f);
+        put(b_base, b_tile, kc + 1, rowok ? z4.y * rinv * s4.y + t4.y : 0.f);
+        put(b_base, b_tile, kc + 2, rowok ? z4.z * rinv * s4.z + t4.z : 0.f);
+        put(b_base, b_tile, kc + 3, rowok ? z4.w * rinv * s4.w + t4.w : 0.f);
+      }
+      fence_proxy_async();
+      mbar_arrive(wg_full(st));
+    }
     const float vv = (p.po.vec && rowok) ? p.po.vec[(size_t)b * p.po.vec_stride + gi] : 0.f;
     float* Zbrow = p.Zbar + ((size_t)b * n + (rowok ? gi : 0)) * din;
     // pass 2: Zbar, its producer outputs, and the per-column sums (g_nw, g_nb, column sums of Zbar)
@@ -1633,6 +1690,16 @@ k_tc_linear_bwd(const __grid_constant__ CUtensorMap map_hi, const __grid_constan
 #pragma unroll
         for (int v4 = 0; v4 < 4; ++v4)
           *reinterpret_cast<float4*>(Zbrow + col + 4 * v4) = make_float4(zb[4 * v4], zb[4 * v4 + 1], zb[4 * v4 + 2], zb[4 * v4 + 3]);
+      }
+      if (p.Nout != nullptr && rowok) {
+        float* Nrow = p.Nout + ((size_t)b * n + gi) * din;
+#pragma unroll
+        for (int v4 = 0; v4 < 4; ++v4) {
+          const float4 z4 = *reinterpret_cast<const float4*>(Zrow + col + 4 * v4);
+          const float4 s4 = __ldg(reinterpret_cast<const float4*>(p.nw + col + 4 * v4)), t4 = __ldg(reinterpret_cast<const float4*>(p.nb + col + 4 * v4));
+          *reinterpret_cast<float4*>(Nrow + col + 4 * v4) =
+              make_float4(z4.x * rinv * s4.x + t4.x, z4.y * rinv * s4.y + t4.y, z4.z * rinv * s4.z + t4.z, z4.w * rinv * s4.w + t4.w);
+        }
       }
       if (p.po.Thi != nullptr && gi < p.po.rows_pad && p.po.t16 != PEG_FMT_FP16X2) {
 #pragma unroll
@@ -1687,9 +1754,25 @@ k_tc_linear_bwd(const __grid_constant__ CUtensorMap map_hi, const __grid_constan
         }
       }
     }
+    if (wg) {   // TMEM lane = output o (dout == 128), columns = inputs: add the CTA's Wbar partial
+      mbar_wait(wg_bar, 0u);
+      tc_fence_after();
+      float* grow = p.gW + (size_t)row * din;
+      for (int cc = 0; cc < cols_per_half; cc += 16) {
+        const int col = half * cols_per_half + cc;
+        uint32_t r[16];
+        tmem_ld16(trow + (uint32_t)(p.wg_col + col), r);
+        tmem_wait_ld();
+#pragma unroll
+        for (int v4 = 0; v4 < 4; ++v4)
+          atomicAdd(reinterpret_cast<float4*>(grow + col + 4 * v4),
+                    make_float4(__uint_as_float(r[4 * v4]), __uint_as_float(r[4 * v4 + 1]), __uint_as_float(r[4 * v4 + 2]), __uint_as_float(r[4 * v4 + 3])));
+      }
+    }
     tc_fence_before();
   }
   __syncthreads();
+  if (wg && tid < dout) atomicAdd(p.gb + tid, bsum[tid] + bsum[dout + tid] + bsum[2 * dout + tid] + bsum[3 * dout + tid]);
   if (tid < nd) {
     float t[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
@@ -1717,24 +1800,41 @@ bool tc_linear_bwd_supported(int din, int dout) {
   return din % 32 == 0 && din >= 32 && din <= 256 && dout % 32 == 0 && dout >= 32 && get_encode() != nullptr;
 }
 
-int tc_linear_bwd(cudaStream_t st, const PegDims& dm, const TcLinear& w, int layer, const float* Mbar, const float* Z,
-                  const float* nw, int din, int dout, int relu_mask, float* Zbar, float* g_nw, float* g_nb, const ProducerOut& po) {
-  if (!w.ready) return PEG_ERR_WORKSPACE;
-  LbParams p;
-  memset(&p, 0, sizeof(p));
-  p.Mbar = Mbar; p.Z = Z; p.nw = nw; p.Zbar = Zbar; p.g_nw = g_nw; p.g_nb = g_nb; p.po = po;
-  p.n = dm.n; p.din = din; p.dout = dout; p.relu_mask = relu_mask;
-  p.nsplit = (dm.flags & PEG_FLAG_TF32_FAST) ? 1 : 3;
-  const int sp = p.nsplit == 3 ? 2 : 1;
+static int lb_stages(int din, int dout, int nsplit) {
+  const int sp = nsplit == 3 ? 2 : 1;
   const int stage_bytes = sp * TC_ATILE + sp * din * TC_BK * 4;
   int stages = (200 * 1024) / stage_bytes;
   const int nchunks = dout / 32;
   stages = stages > nchunks ? nchunks : stages;
-  stages = stages > 4 ? 4 : stages;
-  if (stages < 1 || (size_t)16 * din * 4 > (size_t)stage_bytes) return PEG_ERR_UNSUPPORTED;
+  return stages > 4 ? 4 : stages;
+}
+
+// the weight-gradient MMA takes all dout outputs as its 128 rows, and its second accumulator (din columns) must fit next to the first
+bool tc_linear_bwd_fuses_weight_grad(const PegDims& dm, int din, int dout) {
+  return tc_linear_bwd_supported(din, dout) && dout == TC_BM && 2 * tmem_cols_pow2(din) <= 512 &&
+         lb_stages(din, dout, (dm.flags & PEG_FLAG_TF32_FAST) ? 1 : 3) >= 2;
+}
+
+int tc_linear_bwd(cudaStream_t st, const PegDims& dm, const TcLinear& w, int layer, const float* Mbar, const float* Z,
+                  const float* nw, const float* nb, int din, int dout, int relu_mask, float* Zbar, float* g_nw, float* g_nb,
+                  float* gW, float* gb, float* Nout, const ProducerOut& po) {
+  if (!w.ready) return PEG_ERR_WORKSPACE;
+  if (gW != nullptr && !tc_linear_bwd_fuses_weight_grad(dm, din, dout)) return PEG_ERR_UNSUPPORTED;
+  LbParams p;
+  memset(&p, 0, sizeof(p));
+  p.Mbar = Mbar; p.Z = Z; p.nw = nw; p.nb = nb; p.Zbar = Zbar; p.g_nw = g_nw; p.g_nb = g_nb; p.po = po;
+  p.gW = gW; p.gb = gb; p.Nout = gW != nullptr ? nullptr : Nout;
+  p.n = dm.n; p.din = din; p.dout = dout; p.relu_mask = relu_mask;
+  p.nsplit = (dm.flags & PEG_FLAG_TF32_FAST) ? 1 : 3;
+  const int sp = p.nsplit == 3 ? 2 : 1;
+  const int stage_bytes = sp * TC_ATILE + sp * din * TC_BK * 4;
+  const int stages = lb_stages(din, dout, p.nsplit);
+  if (stages < 1) return PEG_ERR_UNSUPPORTED;
   p.stages = stages;
-  p.tmem_cols = tmem_cols_pow2(din);
-  const size_t smem = (size_t)stages * stage_bytes + 1024 + 8 * (3 * stages + 2) + 64;
+  p.wg_col = tmem_cols_pow2(din);
+  p.tmem_cols = gW != nullptr ? 2 * p.wg_col : p.wg_col;
+  const size_t sums = (size_t)(16 * din + (gW != nullptr ? 4 * dout : 0)) * 4;
+  const size_t smem = (size_t)stages * stage_bytes + sums + 1024 + 8 * (5 * stages + 3) + 64;
   const CUtensorMap* mhi = nullptr;
   const CUtensorMap* mlo = nullptr;
   PEG_TRY(get_maps(w.Wt_hi[layer], w.Wt_lo[layer], (uint64_t)dout, (uint64_t)din, din, &mhi, &mlo));
@@ -1920,10 +2020,6 @@ __global__ void __launch_bounds__(WG_THREADS, 1) k_tc_weight_grad(const WgParams
     tc_fence_after();
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(p.tmem_cols));
   }
-}
-
-bool tc_weight_grad_supported(int din, int dout) {
-  return dout % 4 == 0 && dout >= 32 && din % 32 == 0 && din >= 32 && din <= 256;
 }
 
 int tc_weight_grad(cudaStream_t st, const PegDims& dm, const float* Mbar, const float* N, size_t rows, int din, int dout,

@@ -47,16 +47,20 @@ bool tc_linear_supported(int din, int dout);
 int tc_prep_weights(cudaStream_t st, const Model& m, const float* params, const TcLinear& w);
 // M = rmsnorm(Z) W^T + b on tcgen05 (3xTF32), fused producer outputs as k_norm_linear (peg_kernels.cuh)
 bool tc_norm_linear_full_columns(int dout);   // one CTA holds every output column of its 128 nodes (it can emit fp16x2 V^T)
-// backward of Linear + RMSNorm wrt the layer input on tcgen05, epilogue as k_linear_bwd (peg_kernels.cuh)
+// backward of Linear + RMSNorm wrt the layer input on tcgen05, epilogue as k_linear_bwd (peg_kernels.cuh).  With gW (only where
+// tc_linear_bwd_fuses_weight_grad) it also accumulates gW += Mbar^T N and gb += 1^T Mbar; otherwise Nout (nullable) receives the
+// normalised input N for tc_weight_grad.
 int tc_linear_bwd(cudaStream_t st, const PegDims& d, const TcLinear& w, int layer, const float* Mbar, const float* Z,
-                  const float* nw, int din, int dout, int relu_mask, float* Zbar, float* g_nw, float* g_nb, const ProducerOut& po);
+                  const float* nw, const float* nb, int din, int dout, int relu_mask, float* Zbar, float* g_nw, float* g_nb,
+                  float* gW, float* gb, float* Nout, const ProducerOut& po);
 bool tc_linear_bwd_supported(int din, int dout);
-// Wbar += Mbar^T N, bbar += 1^T Mbar over all rows, on tcgen05 (both operands transposed in the loaders)
-bool tc_weight_grad_supported(int din, int dout);
+bool tc_linear_bwd_fuses_weight_grad(const PegDims& d, int din, int dout);
+// Wbar += Mbar^T N, bbar += 1^T Mbar over all rows, on tcgen05 (both operands transposed in the loaders); the shapes of
+// tc_linear_bwd_supported
 int tc_weight_grad(cudaStream_t st, const PegDims& d, const float* Mbar, const float* N, size_t rows, int din, int dout, float* gW,
                    float* gb);
-int tc_norm_linear(cudaStream_t st, const PegDims& d, const TcLinear& w, int layer, const float* Z, int din, int dout,
-                   const float* nw, const float* nb, float* M, float* Nout, const ProducerOut& po);
+int tc_norm_linear(cudaStream_t st, const PegDims& d, const TcLinear& w, int layer, const float* Z, int din, int dout, float* M,
+                   const ProducerOut& po);
 bool tc_supported(const PegDims& d, int dcols);
 int tc_fmt(const PegDims& d, bool have_absmax);   // operand format of the contraction (PEG_FMT_*)
 int tc_convert_v(cudaStream_t st, const PegDims& d, const TcWs& w, const ContractArgs& a);

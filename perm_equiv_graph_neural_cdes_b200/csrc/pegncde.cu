@@ -179,6 +179,8 @@ struct Ctx {
 // one vector-field evaluation: dy = f(t, yin)
 //   save[l] (nullable array of L pointers): where to keep the input of layer l (l = 0: yin itself is
 //   the input, nothing is copied; save[l>=1] receives relu(O_l)).
+//   msave[l] / csave[l] (nullable arrays, nullable entries): where to keep M_l [B,n,dout] and its column sums [B][2][dout]
+//   (written in place of the scratch copies, the contraction reads them from there).  The small-graph kernels keep neither.
 // ------------------------------------------------------------------------------------------
 static int stage_prep(Ctx& c, float t) {
   PrepArgs a;
@@ -230,10 +232,12 @@ static bool norm_linear_on_tc(const Ctx& c, int l) {
   return c.use_tc && c.w.lin.ready && tc_linear_supported(c.m.layer[l].din, c.m.layer[l].dout);
 }
 
+// Nout (nullable): the normalised input, for k_weight_grad; the tensor-core path never needs it (k_tc_linear_bwd forms N itself)
 static int norm_linear(Ctx& c, int l, const float* Zin, float* M, float* Nout, const ProducerOut& po) {
   const LayerDesc& ld = c.m.layer[l];
   if (norm_linear_on_tc(c, l)) {
-    const int rc = tc_norm_linear(c.st, c.d, c.w.lin, l, Zin, ld.din, ld.dout, c.params + ld.nw_off, c.params + ld.nb_off, M, Nout, po);
+    if (Nout != nullptr) return PEG_ERR_UNSUPPORTED;
+    const int rc = tc_norm_linear(c.st, c.d, c.w.lin, l, Zin, ld.din, ld.dout, M, po);
     if (rc == PEG_OK) g_launches.fetch_add(1);
     return rc;
   }
@@ -309,8 +313,9 @@ static void shard_select_half(Ctx& c) {
 
 static bool contract_on_tc(const Ctx& c, int l) { return c.use_tc && !c.ctl.sparse && tc_supported(c.d, c.m.layer[l].dout); }
 
+// cbM_global: cbM is already summed over all ranks (solve_fwd kept it after its own exchange), so the exchange leaves it alone
 static int contract(Ctx& c, int l, bool bwd, const float* V, const float* Mref, const float* colbuf, float* out,
-                    bool relu, bool scale_tg, float* g_fus, bool vt_ready, const float* cbM = nullptr) {
+                    bool relu, bool scale_tg, float* g_fus, bool vt_ready, const float* cbM = nullptr, bool cbM_global = false) {
   const LayerDesc& ld = c.m.layer[l];
   ContractArgs a;
   a.planes = c.ctl.adj_coef;
@@ -367,7 +372,7 @@ static int contract(Ctx& c, int l, bool bwd, const float* V, const float* Mref, 
     // row-sharded: every rank needs ALL rows of V^T and the column sums over ALL nodes -> convert V if no producer did, then the
     // exchange over peer memory (push + flags, wait + rank-ordered column sums), then the local row blocks of the contraction
     if (!vt_ready) { rc = tc_convert_v(c.st, c.d, c.w.tc, a); g_launches.fetch_add(c.w.tc.fmt == PEG_FMT_FP16X2 ? 2 : 1); }
-    if (rc == PEG_OK) rc = shard_exchange(c, true, ld.dout, const_cast<float*>(colbuf), const_cast<float*>(cbM));
+    if (rc == PEG_OK) rc = shard_exchange(c, true, ld.dout, const_cast<float*>(colbuf), cbM_global ? nullptr : const_cast<float*>(cbM));
     a.vt_ready = 1;
     if (rc == PEG_OK) rc = tc_contract(c.st, c.d, c.w.tc, a, bwd);
     if (rc == PEG_OK) g_launches.fetch_add(1);
@@ -446,7 +451,8 @@ static int small_launch(Ctx& c, const SmallArgs& a, bool vjp) {
   return PEG_OK;
 }
 
-static int feval_fwd(Ctx& c, float t, const float* yin, float* dy, float* const* save, int nlayers = -1) {
+static int feval_fwd(Ctx& c, float t, const float* yin, float* dy, float* const* save, int nlayers = -1, float* const* msave = nullptr,
+                     float* const* csave = nullptr) {
   const PegDims& d = c.d;
   if (nlayers < 0) nlayers = d.L;
   if (c.small_C > 0 && !c.t_dev) {
@@ -461,15 +467,17 @@ static int feval_fwd(Ctx& c, float t, const float* yin, float* dy, float* const*
   for (int l = 0; l < nlayers; ++l) {
     const LayerDesc& ld = c.m.layer[l];
     const bool last = (l == d.L - 1);
-    const ProducerOut po = producer_out(c, ld.dout, true, c.w.colM, true, svec_c(d.n, l), norm_linear_on_tc(c, l) && tc_norm_linear_full_columns(ld.dout));
-    PEG_TRY(norm_linear(c, l, Zin, c.w.M, nullptr, po));
+    float* M = (msave && msave[l]) ? msave[l] : c.w.M;
+    float* colM = (csave && csave[l]) ? csave[l] : c.w.colM;
+    const ProducerOut po = producer_out(c, ld.dout, true, colM, true, svec_c(d.n, l), norm_linear_on_tc(c, l) && tc_norm_linear_full_columns(ld.dout));
+    PEG_TRY(norm_linear(c, l, Zin, M, nullptr, po));
     float* out;
     if (!last) {
       out = (save && save[l + 1]) ? save[l + 1] : ((l & 1) ? c.w.Zb : c.w.Za);
     } else {
       out = d.e > 0 ? c.w.OL : dy;
     }
-    PEG_TRY(contract(c, l, false, c.w.M, nullptr, c.w.colM, out, !last, last, nullptr, po.Thi != nullptr));
+    PEG_TRY(contract(c, l, false, M, nullptr, colM, out, !last, last, nullptr, po.Thi != nullptr));
     Zin = out;
   }
   if (d.e > 0 && nlayers == d.L) {
@@ -484,8 +492,10 @@ static int feval_fwd(Ctx& c, float t, const float* yin, float* dy, float* const*
 // VJP of one evaluation.  zin[l] = input of layer l (l = 0..L-1) as saved by feval_fwd.
 // kbar: cotangent of dy.  Writes ybar (cotangent of the stage input), accumulates g_params.
 // If g_xd != null (control models) also writes the cotangent of control_data.derivative(t).
+// mkept / ckept (nullable arrays, nullable entries): M_l and its column sums as feval_fwd kept them (msave / csave); the
+// tensor-core path then skips the RMSNorm -> Linear recompute of that layer.
 static int feval_vjp(Ctx& c, float t, float* const* zin, const float* kbar, float* ybar, float* g_params,
-                     float* g_xd) {
+                     float* g_xd, float* const* mkept = nullptr, float* const* ckept = nullptr) {
   const PegDims& d = c.d;
   const int dL = last_width(d);
   if (g_xd != nullptr && d.e == 0) return PEG_ERR_BAD_DIMS;
@@ -533,15 +543,21 @@ static int feval_vjp(Ctx& c, float t, float* const* zin, const float* kbar, floa
   for (int l = d.L - 1; l >= 0; --l) {
     const LayerDesc& ld = c.m.layer[l];
     float* g_fus = g_params + ld.fus_off;
-    // recompute M_l (and the normalised input N_l) from the saved layer input; 1^T M comes out of the same kernel
-    PEG_TRY(norm_linear(c, l, zin[l], c.w.M, c.w.N, producer_out(c, ld.dout, false, c.w.colM, false, 0, false)));
+    const bool lb_tc = c.use_tc && c.w.lin.ready && tc_linear_bwd_supported(ld.din, ld.dout);
+    const bool wg_fused = lb_tc && tc_linear_bwd_fuses_weight_grad(d, ld.din, ld.dout);
+    // M_l and 1^T M_l: as the forward kept them, or recomputed from the saved layer input.  Without tensor cores the recompute
+    // also writes the normalised input N_l for k_weight_grad (k_tc_linear_bwd forms N_l itself).
+    const bool kept = lb_tc && mkept && mkept[l] && ckept && ckept[l];
+    const float* M = kept ? mkept[l] : c.w.M;
+    const float* colM = kept ? ckept[l] : c.w.colM;
+    if (!kept) PEG_TRY(norm_linear(c, l, zin[l], c.w.M, lb_tc ? nullptr : c.w.N, producer_out(c, ld.dout, false, c.w.colM, false, 0, false)));
     if (!obar_ready) PEG_TRY(colsums(c, c.w.Obar, ld.dout, svec_r(d.n, l), true, c.w.colG));
     // the tcgen05 adjoint epilogue also emits the param3..8 gradients (undirected layer; the directed one keeps the separate kernel)
     const bool fused_vec_grads = contract_on_tc(c, l) && !c.m.directed;
-    PEG_TRY(contract(c, l, true, c.w.Obar, c.w.M, c.w.colG, c.w.Mbar, false, false, g_fus, obar_vt, fused_vec_grads ? c.w.colM : nullptr));
+    PEG_TRY(contract(c, l, true, c.w.Obar, M, c.w.colG, c.w.Mbar, false, false, g_fus, obar_vt, fused_vec_grads ? colM : nullptr, kept));
     if (!fused_vec_grads) {
       FusGradArgs a;
-      a.G = c.w.Obar; a.M = c.w.M; a.cbM = c.w.colM; a.cbG = c.w.colG;
+      a.G = c.w.Obar; a.M = M; a.cbM = colM; a.cbG = c.w.colG;
       a.sc = c.w.sc; a.svec = c.w.svec; a.sv_stride = c.sv_stride;
       a.n = d.n; a.d = ld.dout; a.L = d.L; a.g_fus = g_fus; a.directed = c.m.directed;
       dim3 grid((d.n + 7) / 8, d.B);
@@ -549,32 +565,16 @@ static int feval_vjp(Ctx& c, float t, float* const* zin, const float* kbar, floa
       PEG_LAUNCH_CHECK();
     }
     {
-      const size_t rows = (size_t)d.B * d.n;
-      if (c.use_tc && tc_weight_grad_supported(ld.din, ld.dout)) {
-        PEG_TRY(tc_weight_grad(c.st, c.d, c.w.Mbar, c.w.N, rows, ld.din, ld.dout, g_params + ld.w_off, g_params + ld.b_off));
-        g_launches.fetch_add(1);
-      } else {
-      // slices of the node dimension: enough blocks to fill the GPU even for small d_out x d_in
-      const int tiles = ((ld.dout + 63) / 64) * ((ld.din + 63) / 64);
-      int rps = 512;
-      while (rps > 64 && tiles * ((rows + rps - 1) / rps) < 296) rps >>= 1;
-      dim3 grid((ld.dout + 63) / 64, (ld.din + 63) / 64, (unsigned)((rows + rps - 1) / rps));
-      k_weight_grad<<<grid, 256, 0, c.st>>>(c.w.Mbar, c.w.N, rows, ld.din, ld.dout, rps, g_params + ld.w_off,
-                                            g_params + ld.b_off);
-      PEG_LAUNCH_CHECK();
-      }
-    }
-    {
       dim3 grid((d.n + 31) / 32, d.B);
       float* zb = (l == 0) ? ybar : c.w.Obar;
       // for l > 0 the output is the cotangent Obar of layer l-1: emit its column sums (vec = r_{l-1}) and V^T here
       ProducerOut po;
       memset(&po, 0, sizeof(po));
-      const bool lb_tc = c.use_tc && c.w.lin.ready && tc_linear_bwd_supported(ld.din, ld.dout);
       if (l > 0) po = producer_out(c, ld.din, true, c.w.colG, true, svec_r(d.n, l - 1), lb_tc);
       if (lb_tc) {
-        PEG_TRY(tc_linear_bwd(c.st, c.d, c.w.lin, l, c.w.Mbar, zin[l], c.params + ld.nw_off, ld.din, ld.dout, l > 0 ? 1 : 0, zb,
-                              g_params + ld.nw_off, g_params + ld.nb_off, po));
+        PEG_TRY(tc_linear_bwd(c.st, c.d, c.w.lin, l, c.w.Mbar, zin[l], c.params + ld.nw_off, c.params + ld.nb_off, ld.din, ld.dout, l > 0 ? 1 : 0,
+                              zb, g_params + ld.nw_off, g_params + ld.nb_off, wg_fused ? g_params + ld.w_off : nullptr,
+                              wg_fused ? g_params + ld.b_off : nullptr, wg_fused ? nullptr : c.w.N, po));
         g_launches.fetch_add(1);
       } else {
         k_linear_bwd<<<grid, 256, 0, c.st>>>(c.w.Mbar, c.params + ld.w_off, zin[l], c.params + ld.nw_off, d.n,
@@ -584,6 +584,23 @@ static int feval_vjp(Ctx& c, float t, float* const* zin, const float* kbar, floa
       }
       obar_ready = l > 0;
       obar_vt = po.Thi != nullptr;
+    }
+    // Linear weight / bias gradient from Mbar and N (unless k_tc_linear_bwd already added it)
+    if (!wg_fused) {
+      const size_t rows = (size_t)d.B * d.n;
+      if (lb_tc) {
+        PEG_TRY(tc_weight_grad(c.st, c.d, c.w.Mbar, c.w.N, rows, ld.din, ld.dout, g_params + ld.w_off, g_params + ld.b_off));
+        g_launches.fetch_add(1);
+      } else {
+        // slices of the node dimension: enough blocks to fill the GPU even for small d_out x d_in
+        const int tiles = ((ld.dout + 63) / 64) * ((ld.din + 63) / 64);
+        int rps = 512;
+        while (rps > 64 && tiles * ((rows + rps - 1) / rps) < 296) rps >>= 1;
+        dim3 grid((ld.dout + 63) / 64, (ld.din + 63) / 64, (unsigned)((rows + rps - 1) / rps));
+        k_weight_grad<<<grid, 256, 0, c.st>>>(c.w.Mbar, c.w.N, rows, ld.din, ld.dout, rps, g_params + ld.w_off,
+                                              g_params + ld.b_off);
+        PEG_LAUNCH_CHECK();
+      }
     }
   }
   return PEG_OK;
@@ -675,6 +692,35 @@ static int reset_tickets(Ctx& c) {
   return PEG_OK;
 }
 
+// stage_store[step][stage 0..5], one block per stage:
+//   Z: the input of every layer, L slots of [B,n,h] (layer 0 of stage 0 is y_ckpt[step] itself and stays unused);
+//   M: the output M_l = RMSNorm -> Linear of every layer whose output is h wide (all but the 2he-wide last layer of a control
+//      model), one slot of [B,n,h] each;
+//   C: the column sums of those M_l, [B][2][h] each (row 0 = 1^T M, row 1 = 1^T diag(c_l) M).
+// With it solve_bwd needs no forward recompute, and its tensor-core path no RMSNorm -> Linear recompute for the kept layers.
+static int kept_m_layers(const PegDims& d) { return d.e > 0 ? d.L - 1 : d.L; }
+static size_t store_stage_elems(const PegDims& d) {
+  const size_t st = (size_t)d.B * d.n * d.h;
+  return (size_t)(d.L + kept_m_layers(d)) * st + (size_t)kept_m_layers(d) * d.B * 2 * d.h;
+}
+struct StoreSlots {
+  float* z[PEG_MAX_LAYERS];
+  float* m[PEG_MAX_LAYERS];
+  float* cm[PEG_MAX_LAYERS];
+};
+static StoreSlots store_slots(const PegDims& d, float* store, int step, int stage) {
+  StoreSlots s;
+  memset(&s, 0, sizeof(s));
+  const size_t st = (size_t)d.B * d.n * d.h;
+  float* base = store + ((size_t)step * 6 + stage) * store_stage_elems(d);
+  for (int l = 0; l < d.L; ++l) s.z[l] = base + (size_t)l * st;
+  for (int l = 0; l < kept_m_layers(d); ++l) {
+    s.m[l] = base + (size_t)(d.L + l) * st;
+    s.cm[l] = base + (size_t)(d.L + kept_m_layers(d)) * st + (size_t)l * d.B * 2 * d.h;
+  }
+  return s;
+}
+
 struct SolveWs {
   float* k[7];
   float* Z0;         // stage input
@@ -759,7 +805,7 @@ int pegncde_shard_buffer_bytes(const PegDims* dims, int32_t world, size_t* out) 
 
 size_t pegncde_stage_store_bytes(const PegDims* dims, int32_t steps) {
   if (check_dims(dims) != PEG_OK || steps < 1) return 0;
-  return (size_t)steps * 6 * dims->L * dims->B * dims->n * dims->h * sizeof(float);
+  return (size_t)steps * 6 * store_stage_elems(*dims) * sizeof(float);
 }
 
 size_t pegncde_workspace_bytes(const PegDims* dims, int32_t which, int32_t steps) {
@@ -1127,34 +1173,31 @@ int pegncde_solve_fwd(peg_stream_t stream, const PegDims* dims, const PegControl
   PEG_CUDA(cudaMemcpyAsync(y_ckpt, y0, st * sizeof(float), cudaMemcpyDeviceToDevice, c.st));
   float* k[7];
   for (int i = 0; i < 7; ++i) k[i] = s.k[i];
-  const int L = dims->L;
-  // stage_store[step][stage 0..5][layer 0..L-1][B,n,h]: the input of every layer of every stage (layer 0 of stage 0 is
-  // y_ckpt[step] itself and stays unused), so that solve_bwd needs no forward recompute.
-  auto store_slot = [&](int step, int stage, int l) { return stage_store + (((size_t)step * 6 + stage) * L + l) * st; };
-  float* save_arr[PEG_MAX_LAYERS];
-  auto saves = [&](int step, int stage) -> float* const* {
-    if (!stage_store) return nullptr;
-    save_arr[0] = nullptr;
-    for (int l = 1; l < L; ++l) save_arr[l] = store_slot(step, stage, l);
-    return save_arr;
+  // the layout of stage_store: store_slots
+  StoreSlots slots;
+  auto fwd_stage = [&](float ti, const float* zin, float* dy, int step, int stage) -> int {
+    if (!stage_store) return feval_fwd(c, ti, zin, dy, nullptr);
+    slots = store_slots(*dims, stage_store, step, stage);
+    slots.z[0] = nullptr;   // the stage input itself
+    return feval_fwd(c, ti, zin, dy, slots.z, -1, slots.m, slots.cm);
   };
   for (int sidx = 0; sidx < steps; ++sidx) {
     const float t = step_ts[sidx];
     const float dt = step_ts[sidx + 1] - step_ts[sidx];
     const float* y = y_ckpt + (size_t)sidx * st;
     float* ynext = y_ckpt + (size_t)(sidx + 1) * st;
-    if (sidx == 0) PEG_TRY(feval_fwd(c, t, y, k[0], saves(0, 0)));
+    if (sidx == 0) PEG_TRY(fwd_stage(t, y, k[0], 0, 0));
     for (int i = 1; i < 7; ++i) {
       const float* xs[8];
       double cs[8];
       xs[0] = y; cs[0] = 1.0;
       for (int j = 0; j < i; ++j) { xs[j + 1] = k[j]; cs[j + 1] = (double)dt * tb.a[i][j]; }
-      float* zin = (i == 6) ? ynext : (stage_store ? store_slot(sidx, i, 0) : s.Z0);
+      float* zin = (i == 6) ? ynext : (stage_store ? store_slots(*dims, stage_store, sidx, i).z[0] : s.Z0);
       PEG_TRY(combine(c, zin, i + 1, xs, cs));
       if (i == 6 && sidx == steps - 1) break;  // the 7th stage only feeds FSAL: unused after the last step
       const float ti = (i == 6) ? step_ts[sidx + 1] : (t + (float)tb.c[i] * dt);
-      // the 7th stage IS stage 0 of the next step (FSAL): its layer inputs are stored there
-      PEG_TRY(feval_fwd(c, ti, zin, k[i], i == 6 ? saves(sidx + 1, 0) : saves(sidx, i)));
+      // the 7th stage IS stage 0 of the next step (FSAL): its layer data are stored there
+      PEG_TRY(i == 6 ? fwd_stage(ti, zin, k[i], sidx + 1, 0) : fwd_stage(ti, zin, k[i], sidx, i));
     }
     float* tmp = k[0]; k[0] = k[6]; k[6] = tmp;  // FSAL
   }
@@ -1179,8 +1222,9 @@ int pegncde_solve_bwd(peg_stream_t stream, const PegDims* dims, const PegControl
   const size_t st = (size_t)dims->B * dims->n * dims->h;
   const int L = dims->L;
   // one evaluation's VJP; with g_xcoef also the cotangent of the node-signal coefficients of the stage's cubic piece
-  auto stage_vjp = [&](float t, float* const* save, const float* kbar, float* ybar) -> int {
-    PEG_TRY(feval_vjp(c, t, save, kbar, ybar, g_params, g_xcoef ? c.w.gxd : nullptr));
+  auto stage_vjp = [&](float t, float* const* save, const float* kbar, float* ybar, float* const* mkept = nullptr,
+                       float* const* ckept = nullptr) -> int {
+    PEG_TRY(feval_vjp(c, t, save, kbar, ybar, g_params, g_xcoef ? c.w.gxd : nullptr, mkept, ckept));
     if (g_xcoef) {
       const size_t cnt = (size_t)dims->B * dims->n * 2 * dims->e;
       k_xcoef_accum<<<(unsigned)((cnt + 255) / 256), 256, 0, c.st>>>(c.w.gxd, c.w.sc, dims->n, 2 * dims->e, dims->T - 1, dims->B, g_xcoef);
@@ -1244,16 +1288,16 @@ int pegncde_solve_bwd(peg_stream_t stream, const PegDims* dims, const PegControl
         if (i == 0 && sidx > 0) { xs[cnt] = stage_cot(sidx - 1, 6); cs[cnt] = 1.0; ++cnt; }
       }
       PEG_TRY(combine(c, s.kbar, cnt, xs, cs));
-      float* save[PEG_MAX_LAYERS];
       if (stage_store) {
-        float* base = const_cast<float*>(stage_store) + ((size_t)sidx * 6 + i) * L * st;
-        save[0] = (i == 0) ? const_cast<float*>(y) : base;
-        for (int l = 1; l < L; ++l) save[l] = base + (size_t)l * st;
+        StoreSlots kept = store_slots(*dims, const_cast<float*>(stage_store), sidx, i);
+        if (i == 0) kept.z[0] = const_cast<float*>(y);
+        PEG_TRY(stage_vjp(tis[i], kept.z, s.kbar, s.Ybar[i], kept.m, kept.cm));
       } else {
+        float* save[PEG_MAX_LAYERS];
         save[0] = (i == 0) ? const_cast<float*>(y) : s.save[i][0];
         for (int l = 1; l < L; ++l) save[l] = s.save[i][l];
+        PEG_TRY(stage_vjp(tis[i], save, s.kbar, s.Ybar[i]));
       }
-      PEG_TRY(stage_vjp(tis[i], save, s.kbar, s.Ybar[i]));
     }
     // ---- ybar_s = g + sum_i Ybar_i (+ injected cotangent at this boundary) ----
     {

@@ -154,8 +154,7 @@ class _SolveFunction(torch.autograd.Function):
         def run_steps(s0, s1):   # solver steps [s0, s1) -- the whole table in one call unless the control is streamed
             start = y0 if s0 == 0 else y_ckpt[s0].clone()
             seg_ts = np.ascontiguousarray(host_ts[s0:s1 + 1])
-            st_elems = y0.numel()
-            store_ptr = None if store is None else store.data_ptr() + 4 * s0 * 6 * dims.L * st_elems
+            store_ptr = None if store is None else store.data_ptr() + s0 * l.pegncde_stage_store_bytes(dims, 1)
             check(l.pegncde_solve_fwd(_stream_ptr(dev), dims, ctl, flat.data_ptr(),
                                       seg_ts.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), s1 - s0, start.data_ptr(), None,
                                       y_ckpt[s0].data_ptr(), store_ptr, ws.data_ptr(), ws.numel()), "pegncde_solve_fwd")
