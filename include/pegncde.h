@@ -252,6 +252,15 @@ int pegncde_vf_fwd(peg_stream_t stream, const PegDims* dims, const PegControl* c
 int pegncde_vf_vjp(peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params, float t,
                    const float* y, const float* g_dy, float* g_y, float* g_params, float* g_xdot, void* workspace,
                    size_t workspace_bytes);
+/* pegncde_vf_vjp plus the cotangent of a sparse control's coefficients: g_adj_coef [T-1, nnz_stride, 4] (a,b,c,d per entry, in
+ * pattern order, like PegSparse.coef) ACCUMULATES d loss / d coef (caller zeroes it).  The control's statistics (row / column sums,
+ * diagonal, totals) are functions of the coefficients and are differentiated through; the knot times are not.  Every entry has one
+ * owner per layer, so the result is reproducible bit for bit.  Same workspace as pegncde_vf_vjp.  A dense control with a non-NULL
+ * g_adj_coef returns PEG_ERR_UNSUPPORTED, a pointer that is not 16-byte aligned PEG_ERR_ALIGNMENT; with g_adj_coef == NULL the
+ * call is pegncde_vf_vjp. */
+int pegncde_vf_vjp_adj(peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params, float t,
+                       const float* y, const float* g_dy, float* g_y, float* g_params, float* g_xdot, float* g_adj_coef,
+                       void* workspace, size_t workspace_bytes);
 
 /* ---- one Tsit5 step (adaptive controllers stay on the host) ----------------------------- */
 /* k1 = f(t, y) when k1_valid == 0 (first step) else taken from k1 (FSAL).  Writes y1, y_err
@@ -334,6 +343,14 @@ int pegncde_solve_bwd(peg_stream_t stream, const PegDims* dims, const PegControl
                       const float* step_ts, int32_t steps, const float* y_ckpt, const float* stage_store,
                       const float* g_yT, const float* g_ckpt, const float* g_stage, float* g_y0, float* g_params,
                       float* g_xcoef, void* workspace, size_t workspace_bytes);
+/* pegncde_solve_bwd plus g_adj_coef (nullable, sparse controls only) [T-1, nnz_stride, 4]: ACCUMULATES the cotangent of
+ * PegSparse.coef over every stage of every step, as pegncde_vf_vjp_adj does for one evaluation.  Entries are absolute, so the
+ * per-graph views of one batch (B = 1 controls whose row_ptr points into the batch's entry axis) all write the one shared buffer.
+ * Outputs other than g_adj_coef equal pegncde_solve_bwd's bit for bit. */
+int pegncde_solve_bwd_adj(peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params,
+                          const float* step_ts, int32_t steps, const float* y_ckpt, const float* stage_store,
+                          const float* g_yT, const float* g_ckpt, const float* g_stage, float* g_y0, float* g_params,
+                          float* g_xcoef, float* g_adj_coef, void* workspace, size_t workspace_bytes);
 
 /* ---- introspection ------------------------------------------------------------------------ */
 const char* pegncde_strerror(int code);

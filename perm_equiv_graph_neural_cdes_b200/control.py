@@ -107,6 +107,8 @@ class PackedControl:
 
     Built once per batch; owns the device tensors and hands raw pointers to the C-ABI."""
 
+    adj_packed = None   # differentiable source of the adjacency coefficients: sparse controls only (SparseControl)
+
     def __init__(self, B: int, n: int, T: int, e: int, device):
         self.B, self.n, self.T, self.e = B, n, T, e
         self.ldn = _pad32(n)  # planes are stored as 32x32 tiles, zero padded
@@ -407,7 +409,10 @@ def sparse_pattern(edge_index, num_nodes: int) -> SparsePattern:
 class SparseControl(PackedControl):
     """A control path on a sparse (CSR) adjacency pattern: ``PegControl.sparse`` is set and ``adj_coef`` is NULL.  Used wherever a
     :class:`PackedControl` is (vector fields, ``diffeqsolve``, ``tsit5_step``, the models); built by :func:`build_sparse_control` or
-    :func:`pack_sparse_control`.  ``coef``/``coef_t`` are ``[T-1, nnz, 4]`` (a,b,c,d per entry) in pattern and transposed order."""
+    :func:`pack_sparse_control`.  ``coef``/``coef_t`` are ``[T-1, nnz, 4]`` (a,b,c,d per entry) in pattern and transposed order.
+
+    When the builder's edge weights or coefficients require grad, ``adj_packed`` is ``coef`` on the autograd tape: the solves and
+    vector fields then return the cotangent of the coefficients (``pegncde_solve_bwd_adj``) and it flows back to the caller's tensors."""
 
     def __init__(self, pattern: SparsePattern, T: int, device):
         B, n = pattern.B, pattern.n
@@ -427,6 +432,7 @@ class SparseControl(PackedControl):
         self.row_ptr, self.row_ptr_t = pattern.row_ptr, pattern.row_ptr_t
         self.col, self.col_t = pattern.col, pattern.col_t
         self.x_coef, self.x_packed = None, None
+        self.adj_packed = None
         self._adj = {"colsum": torch.empty((B, T - 1, 4, n), **f), "pending": None, "host_ts": None}
 
     @property
@@ -449,7 +455,7 @@ class SparseControl(PackedControl):
         v = SparseControl.__new__(SparseControl)
         v.B, v.n, v.T, v.e, v.ldn = self.B, self.n, self.T, self.e, self.ldn
         for name in ("pattern", "ts", "adj_coef", "adj_absmax", "adj_rowsum", "adj_diag", "adj_total", "tch_coef", "coef", "coef_t",
-                     "row_ptr", "row_ptr_t", "col", "col_t", "x_coef", "x_packed"):
+                     "row_ptr", "row_ptr_t", "col", "col_t", "x_coef", "x_packed", "adj_packed"):
             setattr(v, name, getattr(self, name))
         v._adj = self._adj
         v._keepalive = self
@@ -462,7 +468,8 @@ class SparseControl(PackedControl):
         return v
 
     def select(self, b: int) -> "SparseControl":
-        """View of graph ``b`` as a batch of one (no copy: the row offsets are absolute into the shared entry axis)."""
+        """View of graph ``b`` as a batch of one (no copy: the row offsets are absolute into the shared entry axis, so ``coef`` and
+        ``adj_packed`` stay the whole batch's)."""
         v = self._view()
         v.B = 1
         for name in ("ts", "adj_rowsum", "adj_diag", "adj_total", "tch_coef", "row_ptr", "row_ptr_t"):
@@ -530,13 +537,41 @@ def _new_sparse_control(ts, pattern: SparsePattern, T: int, device) -> SparseCon
     return sc
 
 
+class _HermiteOnPattern(torch.autograd.Function):
+    """``values`` [T, nnz] (knot values of every entry) -> the coefficients ``[T-1, nnz, 4]`` (a,b,c,d) the CUDA builder wrote
+    (``coef``, returned as is, so they stay bit-identical to the dense builder's).  Backward: the transpose of
+    :func:`backward_hermite_coefficients` per graph (it is linear in the values), with that graph's knot times."""
+
+    @staticmethod
+    def forward(ctx, values, sc):
+        ctx.ts = sc.ts
+        ctx.bounds = sc.row_ptr[:, [0, -1]].cpu().tolist()    # each graph's entry range (on the host: no sync in backward)
+        return sc.coef.detach()
+
+    @staticmethod
+    def backward(ctx, g):
+        g = g.to(torch.float32)
+        out = torch.zeros((ctx.ts.shape[1], g.shape[1]), dtype=torch.float32, device=g.device)
+        for b, (e0, e1) in enumerate(ctx.bounds):
+            if e1 == e0:
+                continue
+            with torch.enable_grad():
+                v = torch.zeros((ctx.ts.shape[1], e1 - e0), dtype=torch.float32, device=g.device, requires_grad=True)
+                d, c, bb, a = backward_hermite_coefficients(ctx.ts[b], v)
+                out[:, e0:e1] = torch.autograd.grad((a, bb, c, d), v, tuple(g[:, e0:e1, q] for q in range(4)))[0]
+        return out, None
+
+
 def build_sparse_control(ts: torch.Tensor, edge_index, edge_weight, num_nodes: int, x_t: Optional[torch.Tensor] = None,
                          device=None) -> SparseControl:
     """Edge list(s) + per-knot edge weights -> :class:`SparseControl` (``pegncde_build_adj_sparse``: the sparse form of
     :func:`build_control`, with the same Hermite arithmetic, so the coefficients equal the dense builder's bit for bit).
 
     ``edge_index``: ``[2, E]`` or a list of B; ``edge_weight``: ``[T, E]`` (or a list of B, matching), the value of every edge at
-    every knot (0 where it is absent); ``ts``: ``[T]`` or ``[B, T]``; ``x_t``: optional node signals ``[T, n, e]`` / ``[B, T, n, e]``."""
+    every knot (0 where it is absent); ``ts``: ``[T]`` or ``[B, T]``; ``x_t``: optional node signals ``[T, n, e]`` / ``[B, T, n, e]``.
+
+    Edge weights that require grad receive their gradient through every solve and vector field run on this control (duplicate edges
+    each get the gradient of the entry they were summed into); ``edge_index`` and ``ts`` get none."""
     graphs = _edge_list(edge_index)
     device = torch.device(device if device is not None else graphs[0].device)
     if device.type != "cuda":
@@ -555,6 +590,8 @@ def build_sparse_control(ts: torch.Tensor, edge_index, edge_weight, num_nodes: i
     check(lib().pegncde_build_adj_sparse(_stream_ptr(device), _sparse_dims(pat, T), sp, pat.perm_t.data_ptr(), sc.ts.data_ptr(),
                                          values.data_ptr(), sc.adj_rowsum.data_ptr(), sc.adj_diag.data_ptr(), sc.adj_total.data_ptr(),
                                          sc.adj_colsum.data_ptr(), sc.tch_coef.data_ptr()), "pegncde_build_adj_sparse")
+    if values.requires_grad:
+        sc.adj_packed = _HermiteOnPattern.apply(values, sc)
     if x_t is not None:
         _attach_x(sc, _node_signal_coeffs(sc.ts, x_t, pat.B, T, pat.n, device), device)
     sc._keepalive = values      # the source lives until the builder has run (stream-ordered)
@@ -568,7 +605,8 @@ def pack_sparse_control(ts: torch.Tensor, edge_index, coeffs_adj, x_coeffs=None,
 
     ``coeffs_adj``: ``(d, c, b, a)`` each ``[T-1, E]`` -- the adjacency channel only (the time channel is t itself) -- or a list of B
     such tuples, one per pattern of ``edge_index``.  Linear interpolation is ``c = d = 0``.  ``x_coeffs`` as in :func:`pack_control`.
-    ``num_nodes`` defaults to the node count of ``x_coeffs`` (required without it)."""
+    ``num_nodes`` defaults to the node count of ``x_coeffs`` (required without it).  Coefficients that require grad receive their
+    gradient as in :func:`build_sparse_control`."""
     graphs = _edge_list(edge_index)
     device = torch.device(device if device is not None else graphs[0].device)
     if device.type != "cuda":
@@ -600,6 +638,8 @@ def pack_sparse_control(ts: torch.Tensor, edge_index, coeffs_adj, x_coeffs=None,
                                         cf[1].data_ptr(), cf[2].data_ptr(), cf[3].data_ptr(), sc.adj_rowsum.data_ptr(),
                                         sc.adj_diag.data_ptr(), sc.adj_total.data_ptr(), sc.adj_colsum.data_ptr(),
                                         sc.tch_coef.data_ptr()), "pegncde_pack_adj_sparse")
+    if any(c.requires_grad for c in cf):
+        sc.adj_packed = torch.stack([cf[3], cf[2], cf[1], cf[0]], dim=-1)     # [T-1, nnz, 4] (a,b,c,d): coef, on the tape
     if x_coeffs is not None:
         _attach_x(sc, x_coeffs, device)
     sc._keepalive = cf

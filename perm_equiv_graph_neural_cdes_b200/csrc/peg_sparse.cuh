@@ -187,6 +187,177 @@ __global__ void __launch_bounds__(256) k_sparse_contract(const ContractArgs a, c
   }
 }
 
+// =====================================================================================
+// Cotangent of the coefficients (pegncde_vf_vjp_adj / pegncde_solve_bwd_adj).  One layer computes O = M + F M, F = fusion(A, A').
+// With Obar = dL/dO, Gbar_ij = <Obar_i, M_j>, q_i = <Obar_i, M_i>, u_i = <Obar_i, 1^T M>, w_i = <M_i, 1^T Obar>, every pattern entry
+// (i, j) gets
+//   gA = (1 + p1) Gbar_ij + p2 Gbar_ji + [i == j] p3 q_i + rowA_i + colA_j + totA     (gD likewise with the A' coefficients)
+// where row* / col* / tot* gather the row-sum, column-sum, diag(sum) and total terms of the fusion (DESIGN.md, "Edge gradients"), and
+// adds wA[k] gA + wD[k] gD to coefficient k of the entry on the stage's cubic piece.
+// =====================================================================================
+struct AdjGradArgs {
+  const float* G;          // Obar [B,n,d]
+  const float* M;          // [B,n,d]
+  const float* cbM;        // [B][2][d]: [0] = 1^T M
+  const float* cbG;        // [B][2][d]: [0] = 1^T Obar
+  const float* fus;        // the layer's fusion scalars (16, or 22 + 2 for the directed layer)
+  const StageScalars* sc;
+  float* node;             // [B][4][n]: rowA, rowD, colA, colD
+  float* q;                // [B][n]
+  float* tot;              // [B][2]: totA, totD
+  float* g_coef;           // [T-1, nnz_stride, 4]
+  int n, d, directed;
+};
+
+// per-node tables: one warp per (node, graph), grid (ceil(n/8), B), block 256
+__global__ void __launch_bounds__(256) k_sparse_adj_node(const AdjGradArgs a) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int i = blockIdx.x * 8 + warp, b = blockIdx.y;
+  const int n = a.n, d = a.d;
+  if (i >= n) return;
+  const float* g = a.G + ((size_t)b * n + i) * d;
+  const float* m = a.M + ((size_t)b * n + i) * d;
+  const float* sM = a.cbM + (size_t)b * 2 * d;
+  const float* sG = a.cbG + (size_t)b * 2 * d;
+  float q = 0.f, u = 0.f, w = 0.f;
+  for (int c = lane; c < d; c += 32) {
+    const float gv = g[c], mv = m[c];
+    q = fmaf(gv, mv, q);
+    u = fmaf(gv, sM[c], u);
+    w = fmaf(mv, sG[c], w);
+  }
+  q = warp_sum(q); u = warp_sum(u); w = warp_sum(w);
+  if (lane != 0) return;
+  const float* f = a.fus;
+  const float inv_n = 1.f / (float)n;
+  float rA, rD, cA = 0.f, cD = 0.f;
+  if (!a.directed) {        // term 4: rowsum_i on row i (u_i), term 5: rowsum_j on column j (w_i), term 6: diag(rowsum) (q_i)
+    rA = (f[6] * u + f[8] * w + f[10] * q) * inv_n;
+    rD = (f[7] * u + f[9] * w + f[11] * q) * inv_n;
+  } else {                  // column sums feed terms 4, 5, 6 (and 4' for A'); row sums feed 4' (A), 5', 6'
+    rA = ((f[16] + f[18]) * w + f[20] * q) * inv_n;
+    rD = (f[19] * w + f[21] * q) * inv_n;
+    cA = (f[6] * u + f[8] * w + f[10] * q) * inv_n;
+    cD = (f[7] * u + (f[9] + f[17]) * w + f[11] * q) * inv_n;
+  }
+  float* nv = a.node + (size_t)b * 4 * n;
+  nv[i] = rA; nv[n + i] = rD; nv[2 * n + i] = cA; nv[3 * n + i] = cD;
+  a.q[(size_t)b * n + i] = q;
+}
+
+// per-graph totals, reduced in a fixed order: grid B, block 1024.  Term 7 multiplies sum(A) for both of its coefficients (the
+// reference's quirk), so only term 8 puts a total on A'.
+__global__ void __launch_bounds__(1024) k_sparse_adj_tot(const AdjGradArgs a) {
+  __shared__ float red[40];
+  const int b = blockIdx.x, n = a.n, d = a.d;
+  const float* q = a.q + (size_t)b * n;
+  const float* sM = a.cbM + (size_t)b * 2 * d;
+  const float* sG = a.cbG + (size_t)b * 2 * d;
+  float sq = 0.f, s = 0.f;
+  for (int i = threadIdx.x; i < n; i += blockDim.x) sq += q[i];
+  for (int c = threadIdx.x; c < d; c += blockDim.x) s = fmaf(sG[c], sM[c], s);
+  sq = block_sum(sq, red);
+  s = block_sum(s, red);
+  if (threadIdx.x == 0) {
+    const float* f = a.fus;
+    const float inv_n2 = 1.f / ((float)n * (float)n);
+    a.tot[2 * b] = ((f[12] + f[13]) * s + f[14] * sq) * inv_n2;
+    a.tot[2 * b + 1] = f[15] * sq * inv_n2;
+  }
+}
+
+// the entries: k_sparse_contract's layout with at most 8 lanes per (row i, graph) (sparse_adj_glog), grid (ceil(n / (8 * 32/G)), B),
+// block 256.  The group keeps the first ADJ_RESIDENT slabs (4G columns each) of Obar_i and M_i in registers; for each entry (i, j) of
+// row i every lane gathers its float4s of M_j and Obar_j, the two dot products are reduced over the group by a butterfly, and the
+// lane that loaded the entry read-modify-writes its four coefficients.  Narrow groups keep the butterfly short (3 shuffles per
+// product, shared by the 4 rows a warp walks at once).  One owner per entry and stream-ordered launches: no atomics, and the result
+// is reproducible bit for bit.
+constexpr int ADJ_RESIDENT = 4;
+
+__device__ __forceinline__ void adj_dot4(const float4 o, const float4 m, const float4 mj, const float4 oj, float& sij, float& sji) {
+  sij = fmaf(o.x, mj.x, fmaf(o.y, mj.y, fmaf(o.z, mj.z, fmaf(o.w, mj.w, sij))));
+  sji = fmaf(oj.x, m.x, fmaf(oj.y, m.y, fmaf(oj.z, m.z, fmaf(oj.w, m.w, sji))));
+}
+
+__global__ void __launch_bounds__(256) k_sparse_adj_grad(const AdjGradArgs a, const PegSparse sp, int glog) {
+  const int G = 1 << glog, rows_per_warp = 32 >> glog;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int sub = lane >> glog, lj = lane & (G - 1);
+  const unsigned gmask = G == 32 ? 0xffffffffu : (((1u << G) - 1u) << (sub * G));
+  const int b = blockIdx.y, n = a.n, d = a.d;
+  const int i = (blockIdx.x * 8 + warp) * rows_per_warp + sub;
+  if (i >= n) return;                        // the whole group shares i
+  const float* Gb = a.G + (size_t)b * n * d;
+  const float* Mb = a.M + (size_t)b * n * d;
+  const float* nv = a.node + (size_t)b * 4 * n;
+  const StageScalars& sc = a.sc[b];
+  const float* f = a.fus;
+  const float alpha = 1.f + f[0], beta = 1.f + f[1], gamma = f[2], delta = f[3];
+  const float qi = a.q[(size_t)b * n + i];
+  const float rA = nv[i] + a.tot[2 * b], rD = nv[n + i] + a.tot[2 * b + 1];
+  const int nslab = (d + 4 * G - 1) / (4 * G), c0 = 4 * lj;
+  float4 oi[ADJ_RESIDENT], mi[ADJ_RESIDENT];
+#pragma unroll
+  for (int s = 0; s < ADJ_RESIDENT; ++s) {
+    const int c = s * 4 * G + c0;
+    oi[s] = make_float4(0.f, 0.f, 0.f, 0.f);
+    mi[s] = oi[s];
+    if (s < nslab && c < d) {
+      oi[s] = __ldg(reinterpret_cast<const float4*>(Gb + (size_t)i * d + c));
+      mi[s] = __ldg(reinterpret_cast<const float4*>(Mb + (size_t)i * d + c));
+    }
+  }
+  float4* gc = reinterpret_cast<float4*>(a.g_coef) + (size_t)sc.interval * sp.nnz_stride;
+  const int e0 = sp.row_ptr[(size_t)b * (n + 1) + i], e1 = sp.row_ptr[(size_t)b * (n + 1) + i + 1];
+  for (int base = e0; base < e1; base += G) {
+    const int e = base + lj;
+    const int k = e < e1 ? __ldg(sp.col + e) : 0;
+    const int cnt = min(G, e1 - base);
+    float gij = 0.f, gji = 0.f;
+    for (int jj = 0; jj < cnt; ++jj) {
+      const int j = __shfl_sync(gmask, k, jj, G);
+      const float* Mj = Mb + (size_t)j * d;
+      const float* Gj = Gb + (size_t)j * d;
+      float sij = 0.f, sji = 0.f;
+#pragma unroll
+      for (int s = 0; s < ADJ_RESIDENT; ++s) {
+        const int c = s * 4 * G + c0;
+        if (s < nslab && c < d)
+          adj_dot4(oi[s], mi[s], __ldg(reinterpret_cast<const float4*>(Mj + c)), __ldg(reinterpret_cast<const float4*>(Gj + c)), sij, sji);
+      }
+      for (int s = ADJ_RESIDENT; s < nslab; ++s) {   // rows wider than the resident slabs (the 2he-wide last layer): reload row i
+        const int c = s * 4 * G + c0;
+        if (c < d)
+          adj_dot4(__ldg(reinterpret_cast<const float4*>(Gb + (size_t)i * d + c)), __ldg(reinterpret_cast<const float4*>(Mb + (size_t)i * d + c)),
+                   __ldg(reinterpret_cast<const float4*>(Mj + c)), __ldg(reinterpret_cast<const float4*>(Gj + c)), sij, sji);
+      }
+      for (int o = G >> 1; o > 0; o >>= 1) {
+        sij += __shfl_xor_sync(gmask, sij, o, G);
+        sji += __shfl_xor_sync(gmask, sji, o, G);
+      }
+      if (lj == jj) { gij = sij; gji = sji; }
+    }
+    if (e < e1) {
+      const bool on_diag = k == i;
+      const float gA = alpha * gij + gamma * gji + rA + nv[2 * n + k] + (on_diag ? f[4] * qi : 0.f);
+      const float gD = beta * gij + delta * gji + rD + nv[3 * n + k] + (on_diag ? f[5] * qi : 0.f);
+      float4 v = gc[e];
+      v.x += sc.wA[0] * gA + sc.wD[0] * gD;
+      v.y += sc.wA[1] * gA + sc.wD[1] * gD;
+      v.z += sc.wA[2] * gA + sc.wD[2] * gD;
+      v.w += sc.wA[3] * gA + sc.wD[3] * gD;
+      gc[e] = v;
+    }
+  }
+}
+
+// lanes per row of k_sparse_adj_grad: as k_sparse_contract, at most 8
+inline int sparse_adj_glog(int d) {
+  int g = 0;
+  while (g < 3 && (4 << g) < d) ++g;
+  return g;
+}
+
 // lanes per row of k_sparse_contract: enough float4 slots for d columns, at most a warp
 inline int sparse_glog(int d) {
   int g = 0;

@@ -173,6 +173,7 @@ struct Ctx {
   unsigned int* xticket;   // arrival counter of k_shard_push (in the tickets area)
   int small_C;             // > 0: the cluster-per-graph kernels of peg_small.cuh evaluate f and its VJP (CTAs per graph)
   size_t small_smem;
+  float* g_adj;            // sparse controls (nullable): the VJP also accumulates the cotangent of PegSparse.coef here
 };
 
 // ------------------------------------------------------------------------------------------
@@ -489,6 +490,30 @@ static int feval_fwd(Ctx& c, float t, const float* yin, float* dy, float* const*
   return PEG_OK;
 }
 
+// cotangent of the sparse coefficients through layer l (peg_sparse.cuh).  The node tables live in Za / Zb, which the VJP does not
+// use otherwise: [B][4][n] fits in Za and [B][n] + [B][2] in Zb, since h >= 4.
+static int adj_grad(Ctx& c, int l, const float* M, const float* colM) {
+  const PegDims& d = c.d;
+  const LayerDesc& ld = c.m.layer[l];
+  AdjGradArgs a;
+  a.G = c.w.Obar; a.M = M; a.cbM = colM; a.cbG = c.w.colG;
+  a.fus = c.params + ld.fus_off;
+  a.sc = c.w.sc;
+  a.node = c.w.Za;
+  a.q = c.w.Zb;
+  a.tot = c.w.Zb + (size_t)d.B * d.n;
+  a.g_coef = c.g_adj;
+  a.n = d.n; a.d = ld.dout; a.directed = c.m.directed;
+  k_sparse_adj_node<<<dim3((d.n + 7) / 8, d.B), 256, 0, c.st>>>(a);
+  PEG_LAUNCH_CHECK();
+  k_sparse_adj_tot<<<d.B, 1024, 0, c.st>>>(a);
+  PEG_LAUNCH_CHECK();
+  const int glog = sparse_adj_glog(ld.dout), G = 1 << glog;
+  k_sparse_adj_grad<<<dim3((unsigned)((d.n + 8 * (32 / G) - 1) / (8 * (32 / G))), d.B), 256, 0, c.st>>>(a, *c.ctl.sparse, glog);
+  PEG_LAUNCH_CHECK();
+  return PEG_OK;
+}
+
 // VJP of one evaluation.  zin[l] = input of layer l (l = 0..L-1) as saved by feval_fwd.
 // kbar: cotangent of dy.  Writes ybar (cotangent of the stage input), accumulates g_params.
 // If g_xd != null (control models) also writes the cotangent of control_data.derivative(t).
@@ -564,6 +589,7 @@ static int feval_vjp(Ctx& c, float t, float* const* zin, const float* kbar, floa
       k_fusion_vec_grads<<<grid, 256, 0, c.st>>>(a);
       PEG_LAUNCH_CHECK();
     }
+    if (c.g_adj) PEG_TRY(adj_grad(c, l, M, colM));   // reads Obar: before the Linear backward overwrites it
     {
       dim3 grid((d.n + 31) / 32, d.B);
       float* zb = (l == 0) ? ybar : c.w.Obar;
@@ -658,6 +684,7 @@ static int make_ctx(Ctx& c, peg_stream_t stream, const PegDims* dims, const PegC
   c.fmt = tc_fmt(*dims, ctl->adj_absmax != nullptr);
   c.t_dev = c.dt_dev = nullptr;
   c.tcoef = 0.f;
+  c.g_adj = nullptr;
   c.sh = ctl->shard;
   small_plan(c);
   if (c.sh) {
@@ -983,11 +1010,20 @@ int pegncde_vf_fwd(peg_stream_t stream, const PegDims* dims, const PegControl* c
   return shard_finish(c);
 }
 
-int pegncde_vf_vjp(peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params, float t,
-                   const float* y, const float* g_dy, float* g_y, float* g_params, float* g_xdot, void* workspace,
-                   size_t workspace_bytes) {
+// g_adj (nullable): the cotangent of the sparse coefficients, [T-1, nnz_stride, 4], accumulated
+static int set_adj_grad(Ctx& c, const PegControl* ctl, float* g_adj) {
+  if (!g_adj) return PEG_OK;
+  if (!ctl->sparse) return PEG_ERR_UNSUPPORTED;     // dense controls get no coefficient cotangent
+  if (((uintptr_t)g_adj & 15) != 0) return PEG_ERR_ALIGNMENT;
+  c.g_adj = g_adj;
+  return PEG_OK;
+}
+
+static int vf_vjp(peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params, float t, const float* y,
+                  const float* g_dy, float* g_y, float* g_params, float* g_xdot, float* g_adj, void* workspace, size_t workspace_bytes) {
   Ctx c;
   PEG_TRY(make_ctx(c, stream, dims, ctl, params));
+  PEG_TRY(set_adj_grad(c, ctl, g_adj));
   if (!y || !g_dy || !g_y || !g_params || !workspace) return PEG_ERR_NULL_POINTER;
   if (workspace_bytes < plan(*dims, PEG_WS_VF_VJP, 0, nullptr, nullptr, nullptr)) return PEG_ERR_WORKSPACE;
   SolveWs s;
@@ -1000,6 +1036,18 @@ int pegncde_vf_vjp(peg_stream_t stream, const PegDims* dims, const PegControl* c
   PEG_TRY(feval_fwd(c, t, y, nullptr, save, dims->L - 1));
   PEG_TRY(feval_vjp(c, t, save, g_dy, g_y, g_params, g_xdot));
   return shard_finish(c);
+}
+
+int pegncde_vf_vjp(peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params, float t,
+                   const float* y, const float* g_dy, float* g_y, float* g_params, float* g_xdot, void* workspace,
+                   size_t workspace_bytes) {
+  return vf_vjp(stream, dims, ctl, params, t, y, g_dy, g_y, g_params, g_xdot, nullptr, workspace, workspace_bytes);
+}
+
+int pegncde_vf_vjp_adj(peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params, float t,
+                       const float* y, const float* g_dy, float* g_y, float* g_params, float* g_xdot, float* g_adj_coef,
+                       void* workspace, size_t workspace_bytes) {
+  return vf_vjp(stream, dims, ctl, params, t, y, g_dy, g_y, g_params, g_xdot, g_adj_coef, workspace, workspace_bytes);
 }
 
 int pegncde_step_fwd(peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params, float t,
@@ -1205,12 +1253,13 @@ int pegncde_solve_fwd(peg_stream_t stream, const PegDims* dims, const PegControl
   return shard_finish(c);
 }
 
-int pegncde_solve_bwd(peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params,
-                      const float* step_ts, int32_t steps, const float* y_ckpt, const float* stage_store,
-                      const float* g_yT, const float* g_ckpt, const float* g_stage, float* g_y0, float* g_params,
-                      float* g_xcoef, void* workspace, size_t workspace_bytes) {
+static int solve_bwd(peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params, const float* step_ts,
+                     int32_t steps, const float* y_ckpt, const float* stage_store, const float* g_yT, const float* g_ckpt,
+                     const float* g_stage, float* g_y0, float* g_params, float* g_xcoef, float* g_adj, void* workspace,
+                     size_t workspace_bytes) {
   Ctx c;
   PEG_TRY(make_ctx(c, stream, dims, ctl, params));
+  PEG_TRY(set_adj_grad(c, ctl, g_adj));
   if (!step_ts || !y_ckpt || (!g_yT && !g_ckpt) || !g_y0 || !g_params || !workspace) return PEG_ERR_NULL_POINTER;
   if (steps < 1) return PEG_ERR_BAD_DIMS;
   if (g_xcoef && dims->e == 0) return PEG_ERR_BAD_DIMS;
@@ -1313,6 +1362,22 @@ int pegncde_solve_bwd(peg_stream_t stream, const PegDims* dims, const PegControl
     }
   }
   return shard_finish(c);
+}
+
+int pegncde_solve_bwd(peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params,
+                      const float* step_ts, int32_t steps, const float* y_ckpt, const float* stage_store,
+                      const float* g_yT, const float* g_ckpt, const float* g_stage, float* g_y0, float* g_params,
+                      float* g_xcoef, void* workspace, size_t workspace_bytes) {
+  return solve_bwd(stream, dims, ctl, params, step_ts, steps, y_ckpt, stage_store, g_yT, g_ckpt, g_stage, g_y0, g_params, g_xcoef,
+                   nullptr, workspace, workspace_bytes);
+}
+
+int pegncde_solve_bwd_adj(peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params,
+                          const float* step_ts, int32_t steps, const float* y_ckpt, const float* stage_store,
+                          const float* g_yT, const float* g_ckpt, const float* g_stage, float* g_y0, float* g_params,
+                          float* g_xcoef, float* g_adj_coef, void* workspace, size_t workspace_bytes) {
+  return solve_bwd(stream, dims, ctl, params, step_ts, steps, y_ckpt, stage_store, g_yT, g_ckpt, g_stage, g_y0, g_params, g_xcoef,
+                   g_adj_coef, workspace, workspace_bytes);
 }
 
 const char* pegncde_strerror(int code) {

@@ -33,7 +33,7 @@ import torch
 
 from ._lib import PEG_WS_SOLVE_BWD, PEG_WS_SOLVE_FWD, PEG_WS_STEP, PEG_WS_VF_FWD, check, lib
 from .control import _stream_ptr
-from .vector_field import CDEWrapperVectorField, PermEquivGraphVectorField, resolve_control, workspace
+from .vector_field import CDEWrapperVectorField, PermEquivGraphVectorField, adj_grad_buffer, resolve_control, workspace
 
 
 STREAM_MIN_PIECE_BYTES = 128 << 20   # host coefficient arrays are streamed piece by piece above this size per cubic piece
@@ -130,9 +130,18 @@ def constant_step_table(t0: float, t1: float, dt0: float, rule: str = "state", m
     return np.asarray(out, dtype=np.float32)
 
 
+def _solve_bwd(l, g_adj, *args) -> None:
+    """pegncde_solve_bwd, or pegncde_solve_bwd_adj when the cotangent of the sparse coefficients is asked for (``args`` = the
+    arguments up to g_xcoef, then the workspace pointer and size)."""
+    if g_adj is None:
+        check(l.pegncde_solve_bwd(*args), "pegncde_solve_bwd")
+    else:
+        check(l.pegncde_solve_bwd_adj(*args[:-2], g_adj.data_ptr(), *args[-2:]), "pegncde_solve_bwd_adj")
+
+
 class _SolveFunction(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, y0, flat, x_packed, pc, dims, step_ts, save_steps, store_stages):
+    def forward(ctx, y0, flat, x_packed, adj_packed, pc, dims, step_ts, save_steps, store_stages):
         y0 = y0.contiguous()
         flat = flat.contiguous()
         S = len(step_ts) - 1
@@ -143,7 +152,7 @@ class _SolveFunction(torch.autograd.Function):
         y_ckpt = torch.empty((S + 1,) + tuple(y0.shape), dtype=torch.float32, device=dev)
         host_ts = np.ascontiguousarray(step_ts, dtype=np.float32)
         ctl = pc.struct()
-        need_grad = any(ctx.needs_input_grad[:3])
+        need_grad = any(ctx.needs_input_grad[:4])
         store = None
         if store_stages and need_grad:
             nbytes_store = l.pegncde_stage_store_bytes(dims, S)
@@ -192,14 +201,15 @@ class _SolveFunction(torch.autograd.Function):
         g_y0 = torch.empty_like(y_ckpt[0])
         g_flat = torch.zeros_like(flat)
         g_x = torch.zeros_like(pc.x_coef) if ctx.needs_input_grad[2] else None
+        g_adj = adj_grad_buffer(pc, ctx.needs_input_grad[3])
         ctl = pc.struct()
         store = ctx.store
-        check(l.pegncde_solve_bwd(_stream_ptr(dev), dims, ctl, flat.data_ptr(),
-                                  ctx.host_ts.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), S, y_ckpt.data_ptr(),
-                                  store.data_ptr() if store is not None else None, g_yT.data_ptr(), g_ckpt.data_ptr() if g_ckpt is not None else None, None, g_y0.data_ptr(),
-                                  g_flat.data_ptr(), g_x.data_ptr() if g_x is not None else None, ws.data_ptr(), ws.numel()), "pegncde_solve_bwd")
+        _solve_bwd(l, g_adj, _stream_ptr(dev), dims, ctl, flat.data_ptr(),
+                   ctx.host_ts.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), S, y_ckpt.data_ptr(),
+                   store.data_ptr() if store is not None else None, g_yT.data_ptr(), g_ckpt.data_ptr() if g_ckpt is not None else None, None, g_y0.data_ptr(),
+                   g_flat.data_ptr(), g_x.data_ptr() if g_x is not None else None, ws.data_ptr(), ws.numel())
         ctx.store = None
-        return g_y0, g_flat, g_x, None, None, None, None, None
+        return g_y0, g_flat, g_x, g_adj, None, None, None, None, None
 
 
 def dense_samples_of_table(step_ts: np.ndarray, save_ts: np.ndarray):
@@ -228,7 +238,7 @@ class _FixedDenseFunction(torch.autograd.Function):
     discrete adjoint over the step table, the samples entering as cotangents of their step's start state and stage slopes."""
 
     @staticmethod
-    def forward(ctx, y0, flat, x_packed, pc, dims, step_ts, save_ts):
+    def forward(ctx, y0, flat, x_packed, adj_packed, pc, dims, step_ts, save_ts):
         y0 = y0.contiguous()
         flat = flat.contiguous()
         l = lib()
@@ -279,10 +289,11 @@ class _FixedDenseFunction(torch.autograd.Function):
         g_y0 = torch.empty_like(y_ckpt[0])
         g_flat = torch.zeros_like(flat)
         g_x = torch.zeros_like(pc.x_coef) if ctx.needs_input_grad[2] else None
-        check(l.pegncde_solve_bwd(_stream_ptr(dev), dims, pc.struct(), flat.data_ptr(), host_ts.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), S,
-                                  y_ckpt.data_ptr(), None, None, g_ckpt.data_ptr(), g_stage.data_ptr(), g_y0.data_ptr(), g_flat.data_ptr(),
-                                  g_x.data_ptr() if g_x is not None else None, ws.data_ptr(), ws.numel()), "pegncde_solve_bwd")
-        return g_y0, g_flat, g_x, None, None, None, None
+        g_adj = adj_grad_buffer(pc, ctx.needs_input_grad[3])
+        _solve_bwd(l, g_adj, _stream_ptr(dev), dims, pc.struct(), flat.data_ptr(), host_ts.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), S,
+                   y_ckpt.data_ptr(), None, None, g_ckpt.data_ptr(), g_stage.data_ptr(), g_y0.data_ptr(), g_flat.data_ptr(),
+                   g_x.data_ptr() if g_x is not None else None, ws.data_ptr(), ws.numel())
+        return g_y0, g_flat, g_x, g_adj, None, None, None, None
 
 
 def _stream_pieces(pc, step_ts, run_steps) -> None:
@@ -370,11 +381,12 @@ def diffeqsolve(terms, solver, t0, t1, dt0, y0, args=None, *, saveat: Optional[S
     step_ts = constant_step_table(float(t0), float(t1), float(dt0), controller.rule, max_steps)
     if saveat.ts is not None:   # SaveAt(ts=...) with ConstantStepSize: evolving_out=True of the PGT / TGB models
         save_ts = np.asarray(torch.as_tensor(saveat.ts).detach().cpu().numpy(), dtype=np.float32).reshape(-1)
-        out = _FixedDenseFunction.apply(yb, vf.checked_flat_params(dims), pc.x_packed, pc, dims, step_ts, save_ts)
+        out = _FixedDenseFunction.apply(yb, vf.checked_flat_params(dims), pc.x_packed, pc.adj_packed, pc, dims, step_ts, save_ts)
         S = len(step_ts) - 1
         return Solution(ts=torch.from_numpy(save_ts.copy()), ys=out.squeeze(1) if unb else out,
                         stats={"num_steps": S, "num_accepted_steps": S, "num_rejected_steps": 0})
-    out = _SolveFunction.apply(yb, vf.checked_flat_params(dims), pc.x_packed, pc, dims, step_ts, bool(saveat.steps), bool(getattr(vf, "store_stages", True)))
+    out = _SolveFunction.apply(yb, vf.checked_flat_params(dims), pc.x_packed, pc.adj_packed, pc, dims, step_ts, bool(saveat.steps),
+                               bool(getattr(vf, "store_stages", True)))
     S = len(step_ts) - 1
     if saveat.steps:
         ys = out.squeeze(1) if unb else out
@@ -525,7 +537,7 @@ class _AdaptiveSolveFunction(torch.autograd.Function):
     samples entering as cotangents of the step's start state and of its seven stage slopes."""
 
     @staticmethod
-    def forward(ctx, y0, flat, vf, wrapped, pc, t0, t1, dt0, ctrl, save_ts, max_steps, stats_out):
+    def forward(ctx, y0, flat, adj_packed, vf, wrapped, pc, t0, t1, dt0, ctrl, save_ts, max_steps, stats_out):
         y0 = y0.contiguous()
         flat = flat.contiguous()
         recs, out = _adaptive_batch(vf, wrapped, pc, flat, y0, t0, t1, dt0, ctrl, save_ts, max_steps)
@@ -544,6 +556,7 @@ class _AdaptiveSolveFunction(torch.autograd.Function):
         dev = flat.device
         g_out = g_out.contiguous().to(torch.float32)
         g_flat = torch.zeros_like(flat)
+        g_adj = adj_grad_buffer(ctx.recs[0]["pc1"], ctx.needs_input_grad[2])   # shared by the per-graph views: entries are absolute
         g_y0s = []
         for b, rec in enumerate(ctx.recs):
             dims, pc1, y_ckpt, step_ts = rec["dims"], rec["pc1"], rec["y_ckpt"], rec["step_ts"]
@@ -563,12 +576,12 @@ class _AdaptiveSolveFunction(torch.autograd.Function):
                             g_stage[s, i].add_(gm, alpha=float(w[i]))
             else:
                 g_ckpt[S] = g_out[0, b:b + 1]
-            check(l.pegncde_solve_bwd(_stream_ptr(dev), dims, pc1.struct(), flat.data_ptr(),
-                                      step_ts.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), S, y_ckpt.data_ptr(), None, None,
-                                      g_ckpt.data_ptr(), g_stage.data_ptr() if g_stage is not None else None, g_y0.data_ptr(),
-                                      g_flat.data_ptr(), None, ws.data_ptr(), ws.numel()), "pegncde_solve_bwd")
+            _solve_bwd(l, g_adj, _stream_ptr(dev), dims, pc1.struct(), flat.data_ptr(),
+                       step_ts.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), S, y_ckpt.data_ptr(), None, None,
+                       g_ckpt.data_ptr(), g_stage.data_ptr() if g_stage is not None else None, g_y0.data_ptr(),
+                       g_flat.data_ptr(), None, ws.data_ptr(), ws.numel())
             g_y0s.append(g_y0)
-        return (torch.cat(g_y0s, dim=0), g_flat) + (None,) * 10
+        return (torch.cat(g_y0s, dim=0), g_flat, g_adj) + (None,) * 10
 
 
 def _diffeqsolve_adaptive(vf, wrapped, pc, t0, t1, dt0, yb, unb, ctrl, saveat, max_steps) -> Solution:
@@ -578,7 +591,8 @@ def _diffeqsolve_adaptive(vf, wrapped, pc, t0, t1, dt0, yb, unb, ctrl, saveat, m
     if saveat.ts is not None:
         save_ts = np.asarray(torch.as_tensor(saveat.ts).detach().cpu().numpy(), dtype=np.float32)
     stats_list = []
-    out = _AdaptiveSolveFunction.apply(yb, vf.flat_params(), vf, wrapped, pc, float(t0), float(t1), dt0, ctrl, save_ts, max_steps, stats_list)
+    out = _AdaptiveSolveFunction.apply(yb, vf.flat_params(), pc.adj_packed, vf, wrapped, pc, float(t0), float(t1), dt0, ctrl, save_ts, max_steps,
+                                       stats_list)
     ys = out.squeeze(1) if unb else out
     ts_out = torch.from_numpy(save_ts.copy()) if save_ts is not None else torch.tensor([float(t1)])
     stats = stats_list[0] if unb else {k: [s[k] for s in stats_list] for k in stats_list[0]}

@@ -264,9 +264,14 @@ def resolve_control(control_adj, control_data, device) -> PackedControl:
     return base.with_x((control_data.d, control_data.c, control_data.b, control_data.a))
 
 
+def adj_grad_buffer(pc, needed: bool):
+    """Zeroed cotangent of a sparse control's coefficients (``pegncde_*_adj``), or None when it is not asked for."""
+    return torch.zeros_like(pc.coef) if needed else None
+
+
 class _VFFunction(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, y, flat, vf, pc, dims, t):
+    def forward(ctx, y, flat, adj_packed, vf, pc, dims, t):
         y = y.contiguous()
         flat = flat.contiguous()
         l = lib()
@@ -289,11 +294,15 @@ class _VFFunction(torch.autograd.Function):
         ws = workspace(y.device, nbytes)
         g_y = torch.empty_like(y)
         g_flat = torch.zeros_like(flat)
+        g_adj = adj_grad_buffer(pc, ctx.needs_input_grad[2])
         ctl = pc.struct()
-        check(l.pegncde_vf_vjp(_stream_ptr(y.device), dims, ctl, flat.data_ptr(), ctx.t, y.data_ptr(),
-                               g_dy.contiguous().data_ptr(), g_y.data_ptr(), g_flat.data_ptr(), None, ws.data_ptr(),
-                               ws.numel()), "pegncde_vf_vjp")
-        return g_y, g_flat, None, None, None, None
+        args = (_stream_ptr(y.device), dims, ctl, flat.data_ptr(), ctx.t, y.data_ptr(), g_dy.contiguous().data_ptr(), g_y.data_ptr(),
+                g_flat.data_ptr(), None)
+        if g_adj is None:
+            check(l.pegncde_vf_vjp(*args, ws.data_ptr(), ws.numel()), "pegncde_vf_vjp")
+        else:
+            check(l.pegncde_vf_vjp_adj(*args, g_adj.data_ptr(), ws.data_ptr(), ws.numel()), "pegncde_vf_vjp_adj")
+        return g_y, g_flat, g_adj, None, None, None, None
 
 
 def fused_vector_field(vf: PermEquivGraphVectorField, t, y: torch.Tensor, control_adj, control_data) -> torch.Tensor:
@@ -305,5 +314,5 @@ def fused_vector_field(vf: PermEquivGraphVectorField, t, y: torch.Tensor, contro
     yb = y.unsqueeze(0) if unb else y
     if yb.shape[0] != pc.B:
         raise ValueError(f"state batch {yb.shape[0]} != control batch {pc.B}")
-    out = _VFFunction.apply(yb.to(torch.float32), vf.checked_flat_params(dims), vf, pc, dims, t)
+    out = _VFFunction.apply(yb.to(torch.float32), vf.checked_flat_params(dims), pc.adj_packed, vf, pc, dims, t)
     return out.squeeze(0) if unb else out

@@ -1,6 +1,6 @@
 """Dense planes against sparse (CSR) controls on the benchmark's inputs: prints ONE JSON line.
 
-  python tools/sparse_bench.py [--steps K] [--warmup W] [--workloads a,b,...]
+  python tools/sparse_bench.py [--steps K] [--warmup W] [--workloads a,b,...] [--edge-grads]
 
 The graphs come from bench.py's generator (synth_adjacency); the edge list of a graph is the union of its nonzeros over the
 knots, the edge weights are the snapshot values on it.  For every workload: solver steps/s of forward + adjoint (CUDA-graph replay,
@@ -8,6 +8,11 @@ as bench.py) on the dense control (build_control) and on the sparse one (build_s
 launch from the profiling hooks, nnz per row, HBM bytes per launch (the hooks' algorithmic count) and the V-gather bytes of the
 sparse contraction (2 nnz d 4, mostly served from L2), and the largest relative difference of y(T), dloss/dy0 and the parameter
 gradient between the two controls.  sparse_n65536_h128 has no dense leg: its planes would not fit in device memory.
+
+--edge-grads adds a sparse leg whose coefficients require grad (a leaf in place of the builder's output, so every replayed step
+differentiates the solve w.r.t. them: pegncde_solve_bwd_adj; the once-per-batch Hermite transpose is not part of a step), its ratio
+to the plain sparse leg, and the device time per launch of k_sparse_adj_grad (+ its per-node kernels) against k_sparse_contract<4>
+from torch.profiler in one eager step of its own.
 """
 import argparse
 import ctypes
@@ -69,7 +74,23 @@ def rel(a, b):
     return float((a - b).abs().max() / b.abs().max().clamp_min(1e-30))
 
 
-def measure(name, wl, steps, warmup, dev):
+def kernel_times(step, pc):
+    """device microseconds per launch of the adjoint's sparse kernels in one eager step, from torch.profiler"""
+    from torch.profiler import ProfilerActivity, profile
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        step(pc)
+        torch.cuda.synchronize()
+    out = {}
+    for key, pat in (("contract_bwd", "k_sparse_contract<4>"), ("adj_grad", "k_sparse_adj_grad"), ("adj_node", "k_sparse_adj_node"),
+                     ("adj_tot", "k_sparse_adj_tot")):
+        evs = [e for e in prof.key_averages() if pat in e.key]
+        cnt = sum(e.count for e in evs)
+        tot = sum(getattr(e, "device_time_total", getattr(e, "cuda_time_total", 0.0)) for e in evs)
+        out[key] = dict(launches=cnt, us_per_launch=tot / max(cnt, 1))
+    return out
+
+
+def measure(name, wl, steps, warmup, dev, edge_grads=False):
     n, h, L, T, B = wl["n"], wl["h"], wl["L"], wl["T"], wl["B"]
     ts = torch.arange(T, device=dev, dtype=torch.float32) * (wl["t1"] / (T - 1))
     with_dense = wl.get("dense", True)
@@ -102,6 +123,8 @@ def measure(name, wl, steps, warmup, dev):
     def step(pc):
         for q in params:
             q.grad = None
+        if pc.adj_packed is not None:
+            pc.adj_packed.grad = None
         y = y0.detach().requires_grad_(True)
         yT = P.diffeqsolve(P.ODETerm(vf), P.Tsit5(), 0.0, wl["t1"], wl["dt0"], y, pc, stepsize_controller=P.ConstantStepSize(),
                            saveat=P.SaveAt(t1=True)).ys[-1]
@@ -149,6 +172,15 @@ def measure(name, wl, steps, warmup, dev):
                sparse_gather_bytes_per_launch=2.0 * sparse.nnz * h * 4)
     s_res, s_out = leg(sparse)
     out["sparse"] = s_res
+    if edge_grads:
+        sg = sparse.with_x(None)
+        sg.adj_packed = sparse.coef.detach().clone().requires_grad_(True)
+        g_res, g_out = leg(sg)
+        g_res["kernels"] = kernel_times(step, sg)
+        g_res["g_adj_finite"] = bool(torch.isfinite(sg.adj_packed.grad).all())
+        out["sparse_edge_grads"] = g_res
+        out["edge_grads_throughput_ratio"] = g_res["steps_per_s"] / s_res["steps_per_s"]
+        out["edge_grads_outputs_bit_identical"] = bool(torch.equal(g_out[0], s_out[0]) and torch.equal(g_out[1], s_out[1]))
     if dense is not None:
         d_res, d_out = leg(dense)
         out["dense"] = d_res
@@ -167,12 +199,13 @@ def main():
     ap.add_argument("--steps", type=int, default=5)
     ap.add_argument("--warmup", type=int, default=1)
     ap.add_argument("--workloads", default=",".join(WORKLOADS))
+    ap.add_argument("--edge-grads", action="store_true", help="also time the solve with the cotangent of the sparse coefficients")
     args = ap.parse_args()
     if args.steps < 1:
         ap.error("--steps must be >= 1")
     dev = torch.device("cuda:0")
     info = gpu_info()
-    rows = [measure(nm, WORKLOADS[nm], args.steps, args.warmup, dev) for nm in args.workloads.split(",")]
+    rows = [measure(nm, WORKLOADS[nm], args.steps, args.warmup, dev, args.edge_grads) for nm in args.workloads.split(",")]
     info_end = gpu_info()
     both = [r for r in rows if r["dense"] is not None]
     wins = [r["n"] for r in both if r["sparse_speedup"] > 1.0]
