@@ -68,3 +68,19 @@ def rel_err(a, b):
     a = torch.as_tensor(a).detach().to(torch.float64).cpu()
     b = torch.as_tensor(b).detach().to(torch.float64).cpu()
     return float((a - b).abs().max() / b.abs().max().clamp_min(1e-30))
+
+
+def union_pattern(planes):
+    """planes [..., n, n] -> edge_index [2, E] of the union of nonzeros over the leading axes"""
+    nz = (planes != 0).reshape(-1, planes.shape[-2], planes.shape[-1]).any(dim=0)
+    return torch.nonzero(nz).t().contiguous()
+
+
+def sparse_of_coeffs(ts, coeffs_adj, x_coeffs=None):
+    """reference-layout coefficients (d,c,b,a) each [T-1, n, n, 2] -> SparseControl on the union of nonzeros of their adjacency channel"""
+    import perm_equiv_graph_neural_cdes_b200 as P
+
+    adj = torch.stack([c[..., 1] for c in coeffs_adj])             # [4, T-1, n, n]
+    ei = union_pattern(adj)
+    co = tuple(c[..., 1][:, ei[0], ei[1]].contiguous() for c in coeffs_adj)
+    return P.pack_sparse_control(ts, ei, co, x_coeffs, num_nodes=adj.shape[-1])

@@ -12,7 +12,7 @@ import torch
 import perm_equiv_graph_neural_cdes_b200 as P
 from perm_equiv_graph_neural_cdes_b200 import _lib
 from oracle import reference_path as R
-from tests.helpers import GOLDEN_CASES, device_model, per_operator, product_grads_as_oracle, rel_err
+from tests.helpers import GOLDEN_CASES, device_model, per_operator, product_grads_as_oracle, rel_err, sparse_of_coeffs, union_pattern
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 TC = _lib.PEG_FLAG_TENSOR_CORES
@@ -116,34 +116,20 @@ def test_c_abi_checks_sparse_controls_without_a_device():
 # ---------------------------------------------------------------------------------------------------
 # GPU: helpers
 # ---------------------------------------------------------------------------------------------------
-def _union_pattern(planes):
-    """planes [..., n, n] -> edge_index [2, E] of the union of nonzeros over the leading axes"""
-    nz = (planes != 0).reshape(-1, planes.shape[-2], planes.shape[-1]).any(dim=0)
-    return torch.nonzero(nz).t().contiguous()
-
-
-def _sparse_of_coeffs(ts, coeffs_adj, x_coeffs=None):
-    """reference-layout coefficients (d,c,b,a) each [T-1, n, n, 2] -> SparseControl on the union of nonzeros of their adjacency channel"""
-    adj = torch.stack([c[..., 1] for c in coeffs_adj])             # [4, T-1, n, n]
-    ei = _union_pattern(adj)
-    co = tuple(c[..., 1][:, ei[0], ei[1]].contiguous() for c in coeffs_adj)
-    return P.pack_sparse_control(ts, ei, co, x_coeffs, num_nodes=adj.shape[-1])
-
-
 def _sparse_model(p, cuda, flags):
     """device_model with the adjacency control replaced by its sparse form"""
     vf, term, _ = device_model(p, cuda, flags=flags)
     ts = p.ts.to(torch.float32).to(cuda)
     co = tuple(c.to(torch.float32).to(cuda) for c in p.coeffs_adj)
     xc = None if p.e == 0 else tuple(c.to(torch.float32).to(cuda) for c in p.x_coeffs)
-    sc = _sparse_of_coeffs(ts, co)
+    sc = sparse_of_coeffs(ts, co)
     args = sc if p.e == 0 else [sc, P.CubicInterpolation(ts, xc)]
     return vf, term, args
 
 
 def _snapshot_edges(A):
     """snapshots [T, n, n] -> (edge_index [2, E], edge_weight [T, E]) on the union of nonzeros"""
-    ei = _union_pattern(A)
+    ei = union_pattern(A)
     return ei, A[:, ei[0], ei[1]].contiguous()
 
 
@@ -260,7 +246,7 @@ def test_sparse_directed_vector_field_against_oracle(cuda):
     vf = vf.to(cuda)
     vf.flags = per_operator(TC)
     ts = p.ts.to(torch.float32).to(cuda)
-    sc = _sparse_of_coeffs(ts, tuple(c.to(cuda) for c in p.coeffs_adj))
+    sc = sparse_of_coeffs(ts, tuple(c.to(cuda) for c in p.coeffs_adj))
     y0 = p.y0.to(cuda).requires_grad_(True)
     dy = vf(1.3, y0, sc)
     p64 = R.problem_to(p, torch.float64)
@@ -292,7 +278,7 @@ def test_sparse_sibling_vector_fields_against_oracle(cuda, cls, with_derivative)
     vf = vf.to(cuda)
     vf.flags = per_operator(TC)
     ts = p.ts.to(torch.float32).to(cuda)
-    sc = _sparse_of_coeffs(ts, tuple(c.to(cuda) for c in p.coeffs_adj))
+    sc = sparse_of_coeffs(ts, tuple(c.to(cuda) for c in p.coeffs_adj))
     y0 = p.y0.to(cuda).requires_grad_(True)
     sol = P.diffeqsolve(P.ODETerm(vf), P.Tsit5(), 0.0, 3.0, 0.75, y0, sc)
     (sol.ys[-1] * p.gyT.to(cuda)).sum().backward()
@@ -359,7 +345,7 @@ def test_models_on_sparse_controls_match_dense_controls(cuda):
     vf, term, _ = device_model(p, cuda)
     stats = [P.diffeqsolve(P.ODETerm(vf), P.Tsit5(), float(ts[0]), float(ts[-1]), None, p.y0.to(cuda), ctl,
                            stepsize_controller=P.PIDController(rtol=1e-3, atol=1e-6), saveat=P.SaveAt(ts=ts)).stats
-             for ctl in (P.pack_control(ts, co), _sparse_of_coeffs(ts, co))]
+             for ctl in (P.pack_control(ts, co), sparse_of_coeffs(ts, co))]
     print(f"\nadaptive solve, dense / sparse control: {stats[0]} / {stats[1]}")
     assert stats[0]["num_steps"] == stats[1]["num_steps"], stats
     # The step sizes themselves follow y_err, a difference of nearly equal stage sums: the 1e-7 relative rounding difference of the
@@ -370,7 +356,7 @@ def test_models_on_sparse_controls_match_dense_controls(cuda):
     x0 = torch.randn(150, 1, generator=torch.Generator().manual_seed(1)).to(cuda)
     for controller, tol_y, tol_g in ((None, 1e-2, 2e-2), (P.ConstantStepSize(), 1e-4, 1e-3)):
         res = []
-        for ctl in (P.pack_control(ts, co), _sparse_of_coeffs(ts, co)):
+        for ctl in (P.pack_control(ts, co), sparse_of_coeffs(ts, co)):
             vf, _, _ = device_model(p, cuda)
             model = P.GraphNeuralCDE(16, vf, seed=3, dt0=None if controller is None else 0.25, controller=controller).to(cuda)
             out = model(ts, ctl, x0)
@@ -401,7 +387,7 @@ def test_models_on_sparse_controls_match_dense_controls(cuda):
         for sparse in (False, True):
             vf, _, _ = device_model(p, cuda)
             model = P.PGTGraphNeuralCDE(h, 2, 3, vf, interpolation=interp, seed=1, dt0=0.1).to(cuda)
-            cadj = _sparse_of_coeffs(ts, coeffs) if sparse else dense_in
+            cadj = sparse_of_coeffs(ts, coeffs) if sparse else dense_in
             out = model(ts, cadj, P.CubicInterpolation(ts, xco), x0)
             out.square().sum().backward()
             res.append((out.detach(), [q.grad.clone() for q in model.parameters()]))
@@ -414,7 +400,7 @@ def test_models_on_sparse_controls_match_dense_controls(cuda):
     for sparse in (False, True):
         vf = P.PermEquivGraphVectorField(h, h, 2 * h * 4, 2, 4, n, key=3).to(cuda)
         model = P.TGBGraphNeuralCDE(h, vf, use_mlps=True, seed=2, dt0=0.05).to(cuda)
-        cadj = _sparse_of_coeffs(ts, co) if sparse else P.pack_control(ts, co)
+        cadj = sparse_of_coeffs(ts, co) if sparse else P.pack_control(ts, co)
         out = model(ts, cadj, x_data, xt0, None)
         out.square().mean().backward()
         assert float(model.data_encoder.weight.grad.abs().max()) > 0
@@ -501,7 +487,7 @@ def test_fp64_sparse_restatement_equals_the_oracle(n):
     """pins _sparse_vf64 to the oracle's dense vector field (CPU, fp64) on the union pattern of a synthetic path"""
     p = R.problem_to(R.make_problem(n=n, h=16, e=0, L=3, T=4, t1=3, dt0=0.5, seed=5), torch.float64)
     adj = torch.stack([c[..., 1] for c in p.coeffs_adj])        # [4(d,c,b,a), T-1, n, n]
-    ei = _union_pattern(adj)
+    ei = union_pattern(adj)
     coef = torch.stack([adj[3], adj[2], adj[1], adj[0]], dim=-1)[:, ei[0], ei[1]]   # [T-1, E, 4] (a,b,c,d)
     layers = [(lp.fusion, lp.weight, lp.bias, lp.norm_weight, lp.norm_bias) for lp in p.layers]
     for t in (0.3, 1.0, 2.7):
