@@ -73,7 +73,8 @@ enum {
                                    rounding ~2^-17 per product).  A separately stated looser-tolerance mode: Z_T within 1e-4,
                                    gradients within 2e-3 */
   PEG_FLAG_ADJ_LIGHT = 8,       /* with TENSOR_CORES: the adjoint contraction runs two of its four products single-pass; looser
-                                   stated tolerance on the param1 / param2 gradients (2.5e-3 instead of 1e-3).  Off by default. */
+                                   stated tolerance on the param1 / param2 gradients (2.5e-3 instead of 1e-3).  Off by default.
+                                   Ignored for a static control (PegControl.adj_static) */
   PEG_FLAG_NO_FUSED_SMALL = 64, /* opt out of the small-graph path.  By default, graphs with n < 128 (undirected layer, h <= 128; the
                                    shapes the tcgen05 contraction does not take) run a whole evaluation f(t, y) -- and a whole
                                    VJP -- in ONE fp32 kernel, a thread-block cluster per graph with cluster barriers between
@@ -169,6 +170,15 @@ typedef struct PegControl {
   const PegSparse* sparse; /* NULL = dense planes (adj_coef).  Otherwise the adjacency path is the CSR path of PegSparse: adj_coef may be
                               NULL, adj_absmax is unused, adj_rowsum / adj_diag / adj_total / adj_colsum / tch_coef keep their meaning
                               (the sparse builders fill all of them, adj_colsum included)                                    */
+  const float* adj_static; /* NULL = the adjacency varies in time (adj_coef or sparse).  Otherwise a STATIC control: A(t) = A for all t,
+                              [B, ldn*ldn], one fp32 plane per graph zero padded to ldn x ldn and stored as 32x32 tiles of 4 KB (element
+                              order: peg_tile_off with a single plane; written by pegncde_build_adj_static).  It computes what the dense
+                              control of the snapshots [A] * T computes, bit for bit, while every n x n x d contraction reads 4 n^2 bytes
+                              per graph instead of 16 n^2.  adj_coef may be NULL; adj_rowsum / adj_diag / adj_total / adj_colsum /
+                              adj_absmax keep their [B, T-1, 4, ...] shapes with A's statistics in the `a` slot of every piece and zeros in
+                              b, c, d.  PEG_FLAG_ADJ_LIGHT means nothing for it (there is no A'_s product to lighten).  Not combinable with
+                              sparse or shard, nor differentiable in A (g_adj_coef): PEG_ERR_UNSUPPORTED; 16-byte aligned
+                              (PEG_ERR_ALIGNMENT) */
 } PegControl;
 
 /* ---- parameter packing ---------------------------------------------------------------
@@ -234,6 +244,12 @@ int pegncde_build_adj_sparse(peg_stream_t stream, const PegDims* dims, const Peg
 int pegncde_pack_adj_sparse(peg_stream_t stream, const PegDims* dims, const PegSparse* sp, const int32_t* perm_t, const float* d,
                             const float* c, const float* b, const float* a, float* adj_rowsum, float* adj_diag, float* adj_total,
                             float* adj_colsum, float* tch_coef);
+/* Static control builder: adjacency [B, n, n] (device) -> adj_static [B, ldn*ldn] and the O(n) tables of every one of the T-1 pieces
+ * (adj_rowsum / adj_diag / adj_colsum [B, T-1, 4, n], adj_total / adj_absmax [B, T-1, 4]: A's statistics in the `a` slot, zeros in
+ * b, c, d), tch_coef = (1, 0, 0).  The sums run in the order of the dense pack / colsum kernels, so every table equals the one
+ * pegncde_build_adj writes for the snapshots [A] * T bit for bit.  Every pointer is required. */
+int pegncde_build_adj_static(peg_stream_t stream, const PegDims* dims, const float* adjacency, float* adj_static, float* adj_rowsum,
+                             float* adj_diag, float* adj_total, float* adj_colsum, float* adj_absmax, float* tch_coef);
 /* d,c,b,a each [B, T-1, n, e, 2] -> x_coef [B, T-1, 3, n, 2e] */
 int pegncde_pack_x(peg_stream_t stream, const PegDims* dims, const float* d, const float* c, const float* b,
                    const float* a, float* x_coef);
@@ -365,7 +381,8 @@ uint64_t pegncde_launch_count(void);
  * and returns, per direction (0 = forward contraction, 1 = backward/adjoint contraction): launches seen,
  * launches timed, summed milliseconds of the timed ones and the algorithmic bytes / flops of one launch.  For a sparse control
  * the bytes are its HBM traffic (both orientations' coefficients and columns, row pointers, V, OUT, M in the adjoint); the
- * gathers of V rows (2 nnz d 4 bytes, mostly served from L2) are not included.
+ * gathers of V rows (2 nnz d 4 bytes, mostly served from L2) are not included.  For a static control the plane bytes are 4 n^2 per
+ * graph (one plane) instead of 16 n^2.
  * stride <= 0 disables and frees the events. */
 int pegncde_profile_enable(int32_t stride);
 int pegncde_profile_read(int32_t direction, uint64_t* launches, uint64_t* timed, double* ms_total,

@@ -47,7 +47,7 @@ class PegSparse(Structure):
 
 
 class PegControl(Structure):
-    _fields_ = [(k, c_void_p) for k in ("ts", "adj_coef", "adj_rowsum", "adj_diag", "adj_total", "tch_coef", "x_coef", "adj_colsum", "adj_absmax")] + [("shard", POINTER(PegShard)), ("sparse", POINTER(PegSparse))]
+    _fields_ = [(k, c_void_p) for k in ("ts", "adj_coef", "adj_rowsum", "adj_diag", "adj_total", "tch_coef", "x_coef", "adj_colsum", "adj_absmax")] + [("shard", POINTER(PegShard)), ("sparse", POINTER(PegSparse)), ("adj_static", c_void_p)]
 
 
 class PegError(RuntimeError):
@@ -79,6 +79,7 @@ SIGNATURES = {
     "pegncde_adj_absmax": (c_int, [_P, _DIMS, c_int32, c_int32, _P, _P]),
     "pegncde_build_adj_sparse": (c_int, [_P, _DIMS, POINTER(PegSparse), _P, _P, _P, _P, _P, _P, _P, _P]),
     "pegncde_pack_adj_sparse": (c_int, [_P, _DIMS, POINTER(PegSparse), _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "pegncde_build_adj_static": (c_int, [_P, _DIMS, _P, _P, _P, _P, _P, _P, _P, _P]),
     "pegncde_pack_x": (c_int, [_P, _DIMS, _P, _P, _P, _P, _P]),
     "pegncde_workspace_bytes": (c_size_t, [_DIMS, c_int32, c_int32]),
     "pegncde_vf_fwd": (c_int, [_P, _DIMS, _CTL, _P, c_float, _P, _P, _P, c_size_t]),

@@ -644,3 +644,126 @@ def pack_sparse_control(ts: torch.Tensor, edge_index, coeffs_adj, x_coeffs=None,
         _attach_x(sc, x_coeffs, device)
     sc._keepalive = cf
     return sc
+
+
+# ------------------------------------------------------------------------------------------------------------------------
+# static controls: PegControl.adj_static in pegncde.h
+# ------------------------------------------------------------------------------------------------------------------------
+class StaticControl(PackedControl):
+    """A control whose graph does not change in time: A(t) = A on every piece, paired (optionally) with a time-varying node-signal
+    path on the knots ``ts``.  ``adj_static`` holds ONE tiled fp32 plane per graph (``[B, ldn*ldn]``) instead of four per piece, so it
+    costs ``4 ldn^2`` bytes per graph and every contraction reads a quarter of the bytes of the dense control of ``[A] * T`` -- whose
+    results it reproduces bit for bit.  The O(n) tables keep the dense shapes (A's statistics in slot ``a``, zeros in b, c, d).
+
+    Built by :func:`build_static_control`; used wherever a :class:`PackedControl` is.  Not differentiable in A."""
+
+    def __init__(self, B: int, n: int, T: int, device):
+        self.B, self.n, self.T, self.e, self.ldn = B, n, T, 0, _pad32(n)
+        f = dict(dtype=torch.float32, device=device)
+        self.ts = torch.empty((B, T), **f)
+        self.adj_coef = None
+        self.adj_static = torch.empty((B, self.ldn * self.ldn), **f)
+        self.adj_rowsum = torch.empty((B, T - 1, 4, n), **f)
+        self.adj_diag = torch.empty((B, T - 1, 4, n), **f)
+        self.adj_total = torch.empty((B, T - 1, 4), **f)
+        self.adj_absmax = torch.empty((B, T - 1, 4), **f)
+        self.tch_coef = torch.empty((B, T - 1, 3, n), **f)
+        self.x_coef, self.x_packed = None, None
+        self._adj = {"colsum": torch.empty((B, T - 1, 4, n), **f), "pending": None, "host_ts": None}
+
+    def struct(self) -> PegControl:
+        return PegControl(self.ts.data_ptr(), None, self.adj_rowsum.data_ptr(), self.adj_diag.data_ptr(), self.adj_total.data_ptr(),
+                          self.tch_coef.data_ptr(), self.x_coef.data_ptr() if self.x_coef is not None else None,
+                          self.adj_colsum.data_ptr(), self.adj_absmax.data_ptr(), None, None, self.adj_static.data_ptr())
+
+    def _view(self) -> "StaticControl":
+        v = StaticControl.__new__(StaticControl)
+        v.B, v.n, v.T, v.e, v.ldn = self.B, self.n, self.T, self.e, self.ldn
+        for name in ("ts", "adj_coef", "adj_static", "adj_rowsum", "adj_diag", "adj_total", "adj_absmax", "tch_coef", "x_coef", "x_packed"):
+            setattr(v, name, getattr(self, name))
+        v._adj = self._adj
+        v._keepalive = self
+        return v
+
+    def with_x(self, x_coeffs) -> "StaticControl":
+        """The same plane and tables (shared, no copy) paired with the node-signal coefficients ``x_coeffs``."""
+        v = self._view()
+        _attach_x(v, x_coeffs, self.device)
+        return v
+
+    def select(self, b: int) -> "StaticControl":
+        """View of graph ``b`` as a batch of one (no copy)."""
+        v = self._view()
+        v.B = 1
+        for name in ("ts", "adj_static", "adj_rowsum", "adj_diag", "adj_total", "adj_absmax", "tch_coef"):
+            setattr(v, name, getattr(self, name)[b:b + 1])
+        v.x_coef = self.x_coef[b:b + 1] if self.x_coef is not None else None
+        v.x_packed = None
+        v._adj = {"colsum": self.adj_colsum[b:b + 1], "pending": None, "host_ts": None}
+        return v
+
+    def materialize(self) -> "StaticControl":
+        return self
+
+    def ensure_colsums(self) -> "StaticControl":
+        return self            # the builder always writes the column sums
+
+    def pack_pieces(self, *args, **kwargs):
+        raise TypeError("static controls are built in one go; they have no streamed pieces")
+
+    def plane_maxima(self, *args, **kwargs):
+        raise TypeError("static controls get their plane maxima from build_static_control")
+
+    def static_plane(self) -> torch.Tensor:
+        """Un-tiles ``adj_static`` to the adjacency [B, n, n] (inspection / tests)."""
+        off = tiled_offsets(self.ldn)[0]
+        nt = self.ldn // 32
+        tile = (torch.arange(self.ldn).view(-1, 1) // 32) * nt + torch.arange(self.ldn).view(1, -1) // 32
+        off = off - tile * 4096                          # offset inside a 4-plane tile: [g][q][m][lane][e] with q = 0
+        g = off // 2048
+        off = tile * 1024 + g * 512 + (off - g * 2048)   # the single-plane tile: [g][m][lane][e]
+        dense = self.adj_static[:, off.reshape(-1).to(self.adj_static.device)].reshape(self.B, self.ldn, self.ldn)
+        return dense[:, : self.n, : self.n]
+
+    def dense_planes(self) -> torch.Tensor:
+        """The path as [B, T-1, 4(a,b,c,d), n, n]: A in plane a of every piece, zeros elsewhere (inspection / tests)."""
+        out = torch.zeros((self.B, self.T - 1, 4, self.n, self.n), dtype=torch.float32, device=self.device)
+        out[:, :, 0] = self.static_plane()[:, None]
+        return out
+
+
+def build_static_control(ts: torch.Tensor, adjacency: torch.Tensor, x_t: Optional[torch.Tensor] = None, device=None) -> StaticControl:
+    """A graph that does not change in time -> :class:`StaticControl` (``pegncde_build_adj_static``).  The same results, bit for bit,
+    as ``build_control(ts, adjacency.expand(T, n, n), x_t)`` at a quarter of the plane bytes per contraction and ``1 / (4 (T-1))`` of
+    the control's memory.
+
+    ``adjacency``: ``[n, n]`` or ``[B, n, n]`` (a host tensor is copied to the device once); ``ts``: ``[T]`` or ``[B, T]`` (T >= 2);
+    ``x_t``: optional node signals ``[T, n, e]`` / ``[B, T, n, e]``.  The adjacency gets no gradient: one that requires grad raises."""
+    if not isinstance(adjacency, torch.Tensor):
+        raise TypeError("adjacency must be a torch tensor")
+    if adjacency.requires_grad:
+        raise ValueError("build_static_control: static controls are not differentiable in the adjacency; pass adjacency.detach()")
+    if adjacency.dim() not in (2, 3) or adjacency.shape[-1] != adjacency.shape[-2] or adjacency.shape[-1] < 1:
+        raise ValueError(f"adjacency must be [n, n] or [B, n, n], got {tuple(adjacency.shape)}")
+    if adjacency.dtype.is_complex:
+        raise ValueError(f"adjacency must hold real numbers, got {adjacency.dtype}")
+    device = torch.device(device if device is not None else adjacency.device)
+    if device.type != "cuda":
+        raise RuntimeError("build_static_control needs a CUDA device: the fused path has no CPU fallback")
+    A = _as_batched(adjacency, 2).to(device=device, dtype=torch.float32, non_blocking=True).contiguous()
+    B, n = A.shape[0], A.shape[1]
+    tsb = _as_batched(torch.as_tensor(ts), 1).to(device=device, dtype=torch.float32)
+    T = tsb.shape[-1]
+    if T < 2:
+        raise ValueError("a control path needs at least two knots")
+    if tsb.dim() != 2 or tsb.shape[0] not in (1, B):
+        raise ValueError(f"ts must be [T] or [B={B}, T], got {tuple(ts.shape)}")
+    sc = StaticControl(B, n, T, device)
+    sc.ts.copy_(tsb.expand(B, T))
+    check(lib().pegncde_build_adj_static(_stream_ptr(device), sc.dims(h=4, L=1), A.data_ptr(), sc.adj_static.data_ptr(),
+                                         sc.adj_rowsum.data_ptr(), sc.adj_diag.data_ptr(), sc.adj_total.data_ptr(), sc.adj_colsum.data_ptr(),
+                                         sc.adj_absmax.data_ptr(), sc.tch_coef.data_ptr()), "pegncde_build_adj_static")
+    if x_t is not None:
+        _attach_x(sc, _node_signal_coeffs(sc.ts, x_t, B, T, n, device), device)
+    sc._keepalive = A          # the source lives until the builder has run (stream-ordered)
+    return sc

@@ -64,12 +64,14 @@ __host__ __device__ inline size_t svec_xd(int n, int L) { return (size_t)(3 * L 
 //   * a warp-level 128-bit load of (g, plane, m) is 512 contiguous bytes, and a whole item is 4 x 16 KB blocks;
 //   * every thread ends up holding a full 4x4 micro tile of all four planes, so the transposed orientation
 //     is free in registers, and both orientations store bank-conflict-free into the swizzled operand tiles.
+// A static control (PegControl.adj_static) stores ONE plane per graph in the same order with np = 1: 4-KB tiles
+// [g][m][lane][e], so a warp-level 128-bit load is still 512 contiguous bytes.
 __host__ __device__ inline int peg_npad(int n) { return (n + 31) / 32 * 32; }
-__host__ __device__ inline size_t peg_tile_off(int i, int k, int q, int nt) {
+__host__ __device__ inline size_t peg_tile_off(int i, int k, int q, int nt, int np = 4) {
   const int rt = i >> 5, ct = k >> 5, r = i & 31, c = k & 31;
   const int rq = r >> 2, m = r & 3, cq = c >> 2, e = c & 3;
   const int s = (rq - cq) & 7, g = s >> 2, lane = ((s & 3) << 3) | cq;
-  return ((size_t)rt * nt + ct) * 4096 + (size_t)(((g * 4 + q) * 4 + m) * 128 + lane * 4 + e);
+  return ((size_t)rt * nt + ct) * (1024 * np) + (size_t)(((g * np + q) * 4 + m) * 128 + lane * 4 + e);
 }
 
 // Tsit5 tableau (Tsitouras 2011) -- the tableau behind diffrax.Tsit5.
@@ -99,8 +101,9 @@ inline const Tsit5& tsit5() {
 
 // arguments of the matrix-free contraction (CUDA-core kernel in peg_kernels.cuh, tcgen05 kernel in peg_tc.cu)
 struct ContractArgs {
-  const float* planes;   // adj_coef
-  size_t graph_stride;   // floats per graph = (T-1)*4*n*ldn
+  const float* planes;   // adj_coef, or adj_static for a static control
+  size_t graph_stride;   // floats per graph = (T-1)*4*n*ldn (static: ldn*ldn)
+  int stat;              // static control: `planes` holds one plane per graph that serves every piece (A_s = a, A'_s = 0)
   const StageScalars* sc;
   const float* svec;
   size_t sv_stride;

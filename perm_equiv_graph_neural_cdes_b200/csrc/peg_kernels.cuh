@@ -38,9 +38,11 @@ __global__ void __launch_bounds__(256) k_pack_adj(const float* __restrict__ cd, 
                                                   const float* __restrict__ ts, int n, int npad, int Tm1, int piece0,
                                                   int in_Tm1, float* __restrict__ adj_coef, float* __restrict__ rowsum,
                                                   float* __restrict__ diag, float* __restrict__ total,
-                                                  float* __restrict__ tch, int ncols, int diag_col0) {
+                                                  float* __restrict__ tch, int ncols, int diag_col0, int np) {
   // rectangular shards (row-sharded mode): n rows x ncols columns (ncols a multiple of 32), diagonal at column diag_col0 + i;
-  // the square case is ncols == n, diag_col0 == 0
+  // the square case is ncols == n, diag_col0 == 0.
+  // np = 1 (static control, pegncde_build_adj_static): `snap` is the adjacency [B, n, n] and only its plane `a` = A is written, one
+  // 4-KB tile per 32x32 block and one slab per graph; the tables of piece 0 are filled (the caller copies them to every piece)
   __shared__ __align__(16) float tile[4096];   // the tile in its final element order
   __shared__ float tcol[8][3][32];             // per-warp column sums of the time channel of (b,c,d)
   // blockIdx.y walks `gridDim.y` cubic pieces starting at piece0; the reference-layout source holds in_Tm1 pieces per
@@ -55,15 +57,15 @@ __global__ void __launch_bounds__(256) k_pack_adj(const float* __restrict__ cd, 
   const float* src[4] = {ca, cb, cc, cd};  // (a,b,c,d) order
   float tsum[3] = {0.f, 0.f, 0.f};
   float dt = 1.f, dtp = 1.f;
-  if (snap) {
+  if (snap && np == 4) {
     const float* tb = ts + (size_t)b * (Tm1 + 1);
     dt = tb[iv + 1] - tb[iv];
     dtp = iv > 0 ? tb[iv] - tb[iv - 1] : dt;
   }
   for (int rt = 0; rt < nt; ++rt) {
-    const size_t tile_base = slab * 4 * (size_t)npad * ncpad + ((size_t)rt * ntc + ct) * 4096;
+    const size_t tile_base = (np == 4 ? slab : (size_t)b) * np * (size_t)npad * ncpad + ((size_t)rt * ntc + ct) * (1024 * np);
     if (tiled_in) {
-      for (int idx = threadIdx.x; idx < 1024; idx += 256)
+      for (int idx = threadIdx.x; idx < 256 * np; idx += 256)
         *reinterpret_cast<float4*>(&tile[4 * idx]) = *reinterpret_cast<const float4*>(tiled_in + tile_base + 4 * idx);
       __syncthreads();
     }
@@ -71,7 +73,9 @@ __global__ void __launch_bounds__(256) k_pack_adj(const float* __restrict__ cd, 
       const int r = idx >> 5, c = idx & 31;      // r is warp-uniform, c == lane
       const int i = rt * 32 + r, k = ct * 32 + c;
       float hv[4] = {0.f, 0.f, 0.f, 0.f};
-      if (snap && i < n && k < ncols) {
+      if (np == 1 && i < n && k < ncols) {
+        hv[0] = __ldg(snap + ((size_t)b * n + i) * (size_t)ncols + k);
+      } else if (snap && i < n && k < ncols) {
         const float* Ab = snap + ((size_t)b * (Tm1 + 1) * n + i) * (size_t)ncols + k;
         const size_t knot = (size_t)n * ncols;
         const float y0 = __ldg(Ab + (size_t)iv * knot), y1 = __ldg(Ab + (size_t)(iv + 1) * knot);
@@ -80,8 +84,9 @@ __global__ void __launch_bounds__(256) k_pack_adj(const float* __restrict__ cd, 
       }
 #pragma unroll
       for (int p = 0; p < 4; ++p) {
+        if (p >= np) break;
         float v = 0.f;
-        const int to = (int)peg_tile_off(r, c, p, 1);   // offset inside the tile
+        const int to = (int)peg_tile_off(r, c, p, 1, np);   // offset inside the tile
         if (i < n && k < ncols) {
           if (tiled_in) {
             v = tile[to];
@@ -99,7 +104,7 @@ __global__ void __launch_bounds__(256) k_pack_adj(const float* __restrict__ cd, 
     }
     __syncthreads();
     if (!tiled_in) {
-      for (int idx = threadIdx.x; idx < 1024; idx += 256)
+      for (int idx = threadIdx.x; idx < 256 * np; idx += 256)
         *reinterpret_cast<float4*>(adj_coef + tile_base + 4 * idx) = *reinterpret_cast<const float4*>(&tile[4 * idx]);
     }
     __syncthreads();
@@ -120,27 +125,29 @@ __global__ void __launch_bounds__(256) k_pack_adj(const float* __restrict__ cd, 
 
 // Row sums of the four tiled planes, deterministic: one block per 32-row tile walks the column tiles in order
 // (fixed-order warp reductions, no float atomics), so the packed control -- and every accept / reject decision of an
-// adaptive solve built on it -- is reproducible run to run.  grid (nt, T-1, B), block 256.
+// adaptive solve built on it -- is reproducible run to run.  grid (nt, T-1, B), block 256.  np = 1: the single plane of a static
+// control (one slab per graph, sums of piece `piece0` of the tables), in the same order as plane `a` of a dense one.
 __global__ void __launch_bounds__(256) k_adj_rowsums(const float* __restrict__ adj_coef, int n, int npad, int Tm1, int piece0,
-                                                     float* __restrict__ rowsum, int ncpad) {
+                                                     float* __restrict__ rowsum, int ncpad, int np) {
   __shared__ __align__(16) float tile[4096];
   const int b = blockIdx.z, iv = piece0 + blockIdx.y, rt = blockIdx.x;
   const int nt = ncpad >> 5, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;   // nt = column tiles (ncpad == npad for a square path)
   const size_t slab = (size_t)b * Tm1 + iv;
-  const float* base = adj_coef + slab * 4 * (size_t)npad * ncpad + (size_t)rt * nt * 4096;
+  const float* base = adj_coef + (np == 4 ? slab : (size_t)b) * np * (size_t)npad * ncpad + (size_t)rt * nt * (1024 * np);
   float acc[4][4];
 #pragma unroll
   for (int p = 0; p < 4; ++p)
 #pragma unroll
     for (int rr = 0; rr < 4; ++rr) acc[p][rr] = 0.f;
   for (int ct = 0; ct < nt; ++ct) {
-    for (int idx = threadIdx.x; idx < 1024; idx += 256)
-      *reinterpret_cast<float4*>(&tile[4 * idx]) = *reinterpret_cast<const float4*>(base + (size_t)ct * 4096 + 4 * idx);
+    for (int idx = threadIdx.x; idx < 256 * np; idx += 256)
+      *reinterpret_cast<float4*>(&tile[4 * idx]) = *reinterpret_cast<const float4*>(base + (size_t)ct * (1024 * np) + 4 * idx);
     __syncthreads();
 #pragma unroll
     for (int p = 0; p < 4; ++p)
 #pragma unroll
-      for (int rr = 0; rr < 4; ++rr) acc[p][rr] += warp_sum(tile[peg_tile_off(4 * warp + rr, lane, p, 1)]);
+      for (int rr = 0; rr < 4; ++rr)
+        if (p < np) acc[p][rr] += warp_sum(tile[peg_tile_off(4 * warp + rr, lane, p, 1, np)]);
     __syncthreads();
   }
   if (lane == 0) {
@@ -149,7 +156,7 @@ __global__ void __launch_bounds__(256) k_adj_rowsums(const float* __restrict__ a
 #pragma unroll
       for (int rr = 0; rr < 4; ++rr) {
         const int i = rt * 32 + 4 * warp + rr;
-        if (i < n) rowsum[(slab * 4 + p) * n + i] = acc[p][rr];
+        if (i < n && p < np) rowsum[(slab * 4 + p) * n + i] = acc[p][rr];
       }
   }
 }
@@ -168,19 +175,20 @@ __global__ void __launch_bounds__(256) k_adj_totals(const float* __restrict__ ro
 
 // max |entry| of each of the four planes of one cubic piece.  grid (tile chunks, pieces, B), block 256; fmaxf is order
 // independent, so the atomicMax on the bit pattern (non-negative floats order like unsigned integers) is reproducible.
+// np = 1: the single plane of a static control (slab b), written to slot `a` of piece `piece0`.
 __global__ void __launch_bounds__(256) k_adj_absmax(const float* __restrict__ adj_coef, int npad, int Tm1, int piece0,
-                                                    float* __restrict__ absmax, int ncpad) {
+                                                    float* __restrict__ absmax, int ncpad, int np) {
   __shared__ float sh[8][4];
   const int b = blockIdx.z, iv = piece0 + blockIdx.y;
   const int ntiles = (npad >> 5) * (ncpad >> 5), warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const size_t slab = (size_t)b * Tm1 + iv;
-  const float4* base = reinterpret_cast<const float4*>(adj_coef + slab * 4 * (size_t)npad * ncpad);
+  const float4* base = reinterpret_cast<const float4*>(adj_coef + (np == 4 ? slab : (size_t)b) * np * (size_t)npad * ncpad);
   float mx[4] = {0.f, 0.f, 0.f, 0.f};
   // a tile is 1024 float4: index i -> plane (i >> 7) & 3   ([g][plane][m][lane] with 4 floats per lane)
   for (int t = blockIdx.x; t < ntiles; t += gridDim.x)
-    for (int i = threadIdx.x; i < 1024; i += 256) {
-      const float4 v = __ldg(base + (size_t)t * 1024 + i);
-      const int q = (i >> 7) & 3;       // warp-uniform per iteration? i = tid + 256 k: (i >> 7) & 3 depends on tid >> 7 -> two values per block
+    for (int i = threadIdx.x; i < 256 * np; i += 256) {
+      const float4 v = __ldg(base + (size_t)t * (256 * np) + i);
+      const int q = np == 4 ? (i >> 7) & 3 : 0;       // warp-uniform per iteration? i = tid + 256 k: (i >> 7) & 3 depends on tid >> 7 -> two values per block
       const float m = fmaxf(fmaxf(fabsf(v.x), fabsf(v.y)), fmaxf(fabsf(v.z), fabsf(v.w)));
 #pragma unroll
       for (int qq = 0; qq < 4; ++qq) mx[qq] = (q == qq) ? fmaxf(mx[qq], m) : mx[qq];
@@ -208,30 +216,31 @@ __global__ void k_fill_tch_unit(float* __restrict__ tch, int n, size_t slabs) {
 
 // Column sums of the four tiled planes (directed fusion layer: layers.py:256-345 uses jnp.sum(., axis=0)), deterministic:
 // one block per 32-column tile walks the row tiles in order; thread (warp w, lane c) keeps rows 4w..4w+3 of column c.
-// grid (nt, T-1, B), block 256.
+// grid (nt, T-1, B), block 256.  np = 1: the single plane of a static control (slab b), written to slot `a` of piece blockIdx.y.
 __global__ void __launch_bounds__(256) k_adj_colsums(const float* __restrict__ adj_coef, int n, int npad, int Tm1,
-                                                     float* __restrict__ colsum) {
+                                                     float* __restrict__ colsum, int np) {
   __shared__ __align__(16) float tile[4096];
   __shared__ float part[8][4][32];
   const int b = blockIdx.z, iv = blockIdx.y, ct = blockIdx.x;
   const int nt = npad >> 5, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const size_t slab = (size_t)b * Tm1 + iv;
-  const float* base = adj_coef + slab * 4 * (size_t)npad * npad;
+  const float* base = adj_coef + (np == 4 ? slab : (size_t)b) * np * (size_t)npad * npad;
   float acc[4] = {0.f, 0.f, 0.f, 0.f};
   for (int rt = 0; rt < nt; ++rt) {
-    for (int idx = threadIdx.x; idx < 1024; idx += 256)
-      *reinterpret_cast<float4*>(&tile[4 * idx]) = *reinterpret_cast<const float4*>(base + ((size_t)rt * nt + ct) * 4096 + 4 * idx);
+    for (int idx = threadIdx.x; idx < 256 * np; idx += 256)
+      *reinterpret_cast<float4*>(&tile[4 * idx]) = *reinterpret_cast<const float4*>(base + ((size_t)rt * nt + ct) * (1024 * np) + 4 * idx);
     __syncthreads();
 #pragma unroll
     for (int p = 0; p < 4; ++p)
 #pragma unroll
-      for (int rr = 0; rr < 4; ++rr) acc[p] += tile[peg_tile_off(4 * warp + rr, lane, p, 1)];
+      for (int rr = 0; rr < 4; ++rr)
+        if (p < np) acc[p] += tile[peg_tile_off(4 * warp + rr, lane, p, 1, np)];
     __syncthreads();
   }
 #pragma unroll
   for (int p = 0; p < 4; ++p) part[warp][p][lane] = acc[p];
   __syncthreads();
-  if (warp < 4) {   // plane = warp, column = lane: add the 8 row groups in a fixed order
+  if (warp < np) {   // plane = warp, column = lane: add the 8 row groups in a fixed order
     float t = 0.f;
 #pragma unroll
     for (int w8 = 0; w8 < 8; ++w8) t += part[w8][warp][lane];
@@ -905,7 +914,9 @@ __device__ __forceinline__ void contract_epilogue4(const ContractArgs& a, int b,
   *reinterpret_cast<float4*>(a.out + ((size_t)b * n + gi) * d + gc) = make_float4(o[0], o[1], o[2], o[3]);
 }
 
-template <int NACC>
+// STAT: static control (ContractArgs.stat): one plane per graph, read for every piece; planes b, c, d are exact zeros, so the
+// arithmetic below is the dense control's on the snapshots [A] * T and the result is the same bit for bit
+template <int NACC, bool STAT = false>
 __global__ void __launch_bounds__(256) k_dual_contract(ContractArgs a) {
   constexpr int NS = (NACC == 1) ? 2 : 4;
   __shared__ __align__(16) float S[NS][CT_KC][CT_LD];
@@ -928,7 +939,8 @@ __global__ void __launch_bounds__(256) k_dual_contract(ContractArgs a) {
     }
   }
   const int npad = a.ldn, nt = npad >> 5;
-  const float* P = a.planes + (size_t)b * a.graph_stride + (size_t)sc.interval * 4 * npad * npad;
+  const float* P = a.planes + (size_t)b * a.graph_stride + (STAT ? 0 : (size_t)sc.interval * 4 * npad * npad);
+  constexpr int NPL = STAT ? 1 : 4;
   const float* Vb = a.V + (size_t)b * n * d;
 
   float acc[NACC][4][4];
@@ -952,7 +964,7 @@ __global__ void __launch_bounds__(256) k_dual_contract(ContractArgs a) {
       for (int q = 0; q < 4; ++q) p[q] = make_float4(0.f, 0.f, 0.f, 0.f);
       if (gi < npad && gk < npad) {   // padding is zero-filled by the pack pre-pass
 #pragma unroll
-        for (int q = 0; q < 4; ++q) p[q] = *reinterpret_cast<const float4*>(P + peg_tile_off(gi, gk, q, nt));
+        for (int q = 0; q < NPL; ++q) p[q] = *reinterpret_cast<const float4*>(P + peg_tile_off(gi, gk, q, nt, NPL));
       }
       float x0[4], x1[4];
       const float* pf = reinterpret_cast<const float*>(p);
@@ -976,7 +988,7 @@ __global__ void __launch_bounds__(256) k_dual_contract(ContractArgs a) {
       for (int q = 0; q < 4; ++q) p[q] = make_float4(0.f, 0.f, 0.f, 0.f);
       if (gk < npad && gi < npad) {
 #pragma unroll
-        for (int q = 0; q < 4; ++q) p[q] = *reinterpret_cast<const float4*>(P + peg_tile_off(gk, gi, q, nt));
+        for (int q = 0; q < NPL; ++q) p[q] = *reinterpret_cast<const float4*>(P + peg_tile_off(gk, gi, q, nt, NPL));
       }
       const float* pf = reinterpret_cast<const float*>(p);
       float y0[4], y1[4];

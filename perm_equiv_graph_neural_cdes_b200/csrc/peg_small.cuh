@@ -139,12 +139,21 @@ __device__ void small_prep(const SmallArgs& a, int b, int rank, const SmallSm& s
   __syncthreads();
 }
 
+// planes of graph b for the stage's cubic piece; STAT (static control, PegControl.adj_static): the one plane of graph b, which
+// serves every piece -- planes b, c, d are exact zeros, so the kernels below compute what the dense control of [A] * T computes
+template <bool STAT>
+__device__ __forceinline__ const float* small_planes(const SmallArgs& a, int b, int interval) {
+  if (STAT) return a.ctl.adj_static + (size_t)b * a.npad * a.npad;
+  return a.ctl.adj_coef + ((size_t)b * (a.T - 1) + interval) * 4 * (size_t)a.npad * a.npad;
+}
+
 // resident mode: A_s = sum_p wA[p] plane_p and A'_s = sum_p wD[p] plane_p of the stage's cubic piece, once per kernel.  The tiled
 // planes are read in storage order (a warp's 128-bit loads are 512 contiguous bytes); thread (g, m, lane) of a 32x32 tile holds
-// row 4 rq + m, columns 4 cq .. 4 cq + 3 of all four planes (peg_tile_off).
+// row 4 rq + m, columns 4 cq .. 4 cq + 3 of all four planes (peg_tile_off).  STAT: the plane is copied (A_s = a, A'_s = 0).
+template <bool STAT>
 __device__ void small_build_A(const SmallArgs& a, int b, const StageScalars* S, const SmallSm& sm) {
   const int tid = threadIdx.x, n16 = (a.n + 15) / 16 * 16, nt = a.npad >> 5, tiles = (n16 + 31) >> 5, P = sm.P;
-  const float* Pl = a.ctl.adj_coef + ((size_t)b * (a.T - 1) + S->interval) * 4 * (size_t)a.npad * a.npad;
+  const float* Pl = small_planes<STAT>(a, b, S->interval);
   const int g = tid >> 7, m = (tid >> 5) & 3, lane = tid & 31;
   const int s_ = (g << 2) | (lane >> 3), cq = lane & 7, rq = (s_ + cq) & 7;
   const int r = rq * 4 + m, c = cq * 4;
@@ -152,6 +161,19 @@ __device__ void small_build_A(const SmallArgs& a, int b, const StageScalars* S, 
 #pragma unroll 2
   for (int t = 0; t < tiles * tiles; ++t) {
     const int rt = t / tiles, ct = t - rt * tiles;
+    if (STAT) {
+      const float4 p0 = __ldg(reinterpret_cast<const float4*>(Pl + ((size_t)rt * nt + ct) * 1024 + (size_t)(g * 4 + m) * 128 + lane * 4));
+      const int gi = rt * 32 + r, gk = ct * 32 + c;
+      if (gi < n16 && gk < n16) {
+        const float e0[4] = {p0.x, p0.y, p0.z, p0.w};
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          sm.As[gi * P + gk + j] = e0[j];
+          sm.Ad[gi * P + gk + j] = 0.f;
+        }
+      }
+      continue;
+    }
     const float* tb = Pl + ((size_t)rt * nt + ct) * 4096 + (size_t)(g * 16 + m) * 128 + lane * 4;
     const float4 p0 = __ldg(reinterpret_cast<const float4*>(tb));
     const float4 p1 = __ldg(reinterpret_cast<const float4*>(tb + 512));
@@ -321,7 +343,7 @@ struct SmallItem {
 
 // ---- phase B / B': one (row block, column block) item of the matrix-free contraction (k_dual_contract, V from shared memory,
 // planes prefetched into registers one K chunk ahead).  NACC = 1 forward, 4 adjoint (+ all fusion-scalar gradients of the layer).
-template <int NACC>
+template <int NACC, bool STAT>
 __device__ void small_contract_item(const SmallItem& it, const StageScalars* S, const SmallSm& sm) {
   constexpr int NS = (NACC == 1) ? 2 : 4;
   float (*Sm_)[SG_KC][SG_LD] = reinterpret_cast<float (*)[SG_KC][SG_LD]>(sm.S);
@@ -354,10 +376,11 @@ __device__ void small_contract_item(const SmallItem& it, const StageScalars* S, 
     const bool okd = gi < npad && gk < npad;
     const int gk2 = k0 + tkr, gi2 = i0 + 4 * tiq;
     const bool okt = gk2 < npad && gi2 < npad;
+    constexpr int NPL = STAT ? 1 : 4;   // a static control has plane a only: b, c, d stay exact zeros
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
-      pd[q] = okd ? __ldg(reinterpret_cast<const float4*>(it.P + peg_tile_off(gi, gk, q, nt))) : make_float4(0.f, 0.f, 0.f, 0.f);
-      pt[q] = okt ? __ldg(reinterpret_cast<const float4*>(it.P + peg_tile_off(gk2, gi2, q, nt))) : make_float4(0.f, 0.f, 0.f, 0.f);
+      pd[q] = (okd && q < NPL) ? __ldg(reinterpret_cast<const float4*>(it.P + peg_tile_off(gi, gk, q, nt, NPL))) : make_float4(0.f, 0.f, 0.f, 0.f);
+      pt[q] = (okt && q < NPL) ? __ldg(reinterpret_cast<const float4*>(it.P + peg_tile_off(gk2, gi2, q, nt, NPL))) : make_float4(0.f, 0.f, 0.f, 0.f);
     }
   };
   auto stage = [&](int k0) {
@@ -693,6 +716,7 @@ __device__ void small_phase_linear(const SmallArgs& a, int l, const float* Z, fl
 }
 
 // forward contraction of layer l: V = Mg [n][dout] -> out [n][dout]
+template <bool STAT>
 __device__ void small_phase_contract_fwd(const SmallArgs& a, int b, int l, const float* Mg, float* out, int relu, int scale_tg,
                                          int rank, const StageScalars* S, const SmallSm& sm) {
   const LayerDesc& ld = a.model.layer[l];
@@ -700,7 +724,7 @@ __device__ void small_phase_contract_fwd(const SmallArgs& a, int b, int l, const
   int lo, hi;
   small_range(nrb * ncb, rank, a.C, lo, hi);
   SmallItem it;
-  it.P = a.ctl.adj_coef + ((size_t)b * (a.T - 1) + S->interval) * 4 * (size_t)a.npad * a.npad;
+  it.P = small_planes<STAT>(a, b, S->interval);
   it.npad = a.npad; it.n = n; it.d = ld.dout;
   it.fus = a.params + ld.fus_off;
   it.vvec = sm.vec + (3 * l + 0) * sm.nv;
@@ -717,13 +741,14 @@ __device__ void small_phase_contract_fwd(const SmallArgs& a, int b, int l, const
     it.c0 = cbi * SG_WB; it.wb = min(SG_WB, ld.dout - it.c0);
     it.i0 = rbi * rbsz; it.rows_end = min(n, it.i0 + rbsz);
     if (cbi != cur) { small_load_V(Mg, n, ld.dout, it.c0, it.wb, sm.vec + (3 * l + 2) * sm.nv, nullptr, sm); cur = cbi; }
-    small_contract_item<1>(it, S, sm);
+    small_contract_item<1, STAT>(it, S, sm);
   }
 }
 
 // =====================================================================================
 // dy = f(t, yin) for graph blockIdx.x / C; grid (B * C), cluster (C), block 256
 // =====================================================================================
+template <bool STAT>
 __global__ void __launch_bounds__(SG_THREADS, 1) k_small_fwd(const SmallArgs a) {
   extern __shared__ __align__(16) float sg_smem[];
   __shared__ StageScalars S;
@@ -732,7 +757,7 @@ __global__ void __launch_bounds__(SG_THREADS, 1) k_small_fwd(const SmallArgs a) 
   const SmallSm sm = small_carve(sg_smem, a.n, a.L);
   const int n = a.n, h = a.h, L = a.L, dmax = a.model.dmax;
   small_prep(a, b, rank, sm, &S);
-  if (sm.As) small_build_A(a, b, &S, sm);
+  if (sm.As) small_build_A<STAT>(a, b, &S, sm);
   float* Mg = a.M + (size_t)b * n * dmax;
   const float* Zin = a.yin + (size_t)b * n * h;
   for (int l = 0; l < a.nlayers; ++l) {
@@ -743,7 +768,7 @@ __global__ void __launch_bounds__(SG_THREADS, 1) k_small_fwd(const SmallArgs a) 
     float* out;
     if (!last) out = (a.save[l + 1] ? a.save[l + 1] : ((l & 1) ? a.Zb : a.Za)) + (size_t)b * n * h;
     else out = a.e > 0 ? a.OL + (size_t)b * n * dmax : a.dy + (size_t)b * n * h;
-    small_phase_contract_fwd(a, b, l, Mg, out, last ? 0 : 1, last ? 1 : 0, rank, &S, sm);
+    small_phase_contract_fwd<STAT>(a, b, l, Mg, out, last ? 0 : 1, last ? 1 : 0, rank, &S, sm);
     __threadfence();
     cluster.sync();
     Zin = out;
@@ -767,6 +792,7 @@ __global__ void __launch_bounds__(SG_THREADS, 1) k_small_fwd(const SmallArgs a) 
 // =====================================================================================
 // VJP of one evaluation (feval_vjp): ybar = J_y^T kbar, g_params += J_theta^T kbar, optionally g_xd
 // =====================================================================================
+template <bool STAT>
 __global__ void __launch_bounds__(SG_THREADS, 1) k_small_vjp(const SmallArgs a) {
   extern __shared__ __align__(16) float sg_smem[];
   __shared__ StageScalars S;
@@ -776,7 +802,7 @@ __global__ void __launch_bounds__(SG_THREADS, 1) k_small_vjp(const SmallArgs a) 
   const int n = a.n, h = a.h, L = a.L, dmax = a.model.dmax, e2 = 2 * a.e;
   const int dL = a.model.layer[L - 1].dout;
   small_prep(a, b, rank, sm, &S);
-  if (sm.As) small_build_A(a, b, &S, sm);
+  if (sm.As) small_build_A<STAT>(a, b, &S, sm);
   float* Mg = a.M + (size_t)b * n * dmax;
   float* Ng = a.N + (size_t)b * n * h;
   float* Og = a.Obar + (size_t)b * n * dmax;
@@ -791,7 +817,7 @@ __global__ void __launch_bounds__(SG_THREADS, 1) k_small_vjp(const SmallArgs a) 
     small_phase_linear(a, l, a.zin[l] + (size_t)b * n * h, Mg, nullptr, rank, sm);
     __threadfence();
     cluster.sync();
-    small_phase_contract_fwd(a, b, l, Mg, OLg, 0, 1, rank, &S, sm);
+    small_phase_contract_fwd<STAT>(a, b, l, Mg, OLg, 0, 1, rank, &S, sm);
     __threadfence();
     cluster.sync();
     float* gx = a.g_xd + (size_t)b * n * e2;
@@ -829,7 +855,7 @@ __global__ void __launch_bounds__(SG_THREADS, 1) k_small_vjp(const SmallArgs a) 
       int lo, hi;
       small_range(nrb * ncb, rank, a.C, lo, hi);
       SmallItem it;
-      it.P = a.ctl.adj_coef + ((size_t)b * (a.T - 1) + S.interval) * 4 * (size_t)a.npad * a.npad;
+      it.P = small_planes<STAT>(a, b, S.interval);
       it.npad = a.npad; it.n = n; it.d = ld.dout;
       it.fus = a.params + ld.fus_off;
       it.vvec = sm.vec + (3 * l + 0) * sm.nv;
@@ -847,7 +873,7 @@ __global__ void __launch_bounds__(SG_THREADS, 1) k_small_vjp(const SmallArgs a) 
         it.i0 = rbi * rbsz; it.rows_end = min(n, it.i0 + rbsz);
         it.first_row_block = rbi == 0;
         if (cbi != cur) { small_load_V(Og, n, ld.dout, it.c0, it.wb, sm.vec + (3 * l + 1) * sm.nv, Mg, sm); cur = cbi; }
-        small_contract_item<4>(it, &S, sm);
+        small_contract_item<4, STAT>(it, &S, sm);
       }
     }
     __threadfence();

@@ -147,19 +147,25 @@ __device__ __forceinline__ int bfp_min_exponent(const int* __restrict__ ve, int 
 // FMT 0 = 3xTF32 operands (fp32 words, SWIZZLE_128B tiles, kind::tf32: error ~2^-22 per product);
 // FMT 1 = bf16x2 operands (x = hi + lo, both bf16; hi*hi + lo*hi + hi*lo on kind::f16 at twice the tf32 rate and half the
 //         shared-memory traffic; SWIZZLE_64B tiles of 8 KB; error ~2^-17 per product, fp32 accumulate in TMEM)
-template <int KIND, int FMT>
+// STAT = static control (ContractArgs.stat): the converters load ONE plane (4 LDG.128 per thread per item instead of 16) that serves
+// every piece, and X = alpha A, Y = gamma A (forward) / A_s = A (adjoint) need no cubic combine.  A'_s = 0, so the adjoint has one
+// A-operand variant per item: its A'_s products and their accumulators are gone and the epilogue reads exact zeros in their place.
+// The K order of every accumulator is the dense kernel's, so the result equals the dense control of [A] * T bit for bit.
+template <int KIND, int FMT, bool STAT = false>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__ CUtensorMap map_lo, const TcParams p) {
   constexpr bool BWD = KIND != 0, LIGHT = KIND == 2;
   constexpr bool F16 = FMT != PEG_FMT_TF32X3;       // 16-bit parts: bf16x2 or fp16x2
   constexpr bool BFP = FMT == PEG_FMT_FP16X2;       // block floating point (see PEG_FMT_FP16X2)
   static_assert(!(F16 && LIGHT), "the LIGHT adjoint exists for the tf32 operand format only");
+  static_assert(!(STAT && LIGHT), "a static control has no A'_s product to lighten");
+  constexpr int NPL = STAT ? 1 : 4;                 // coefficient planes per tile
 
   constexpr int ATILE = F16 ? TC_BM * TC_BK * 2 : TC_ATILE;   // one A-operand tile (hi or lo part)
   constexpr int ESZ = F16 ? 2 : 4;                            // operand element size
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   __shared__ float fsum[8][16];    // adjoint epilogue: per-warp partials of the fusion-scalar gradients
-  constexpr int NA = BWD ? 2 : 1;  // A-operand variants per item: fwd = combined X or Y; bwd = (A_s, A'_s)
+  constexpr int NA = (BWD && !STAT) ? 2 : 1;  // A-operand variants per item: fwd = combined X or Y; bwd = (A_s, A'_s); static bwd = A
   const ContractArgs& a = p.a;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int b = blockIdx.z, I = p.mode == 1 ? (int)blockIdx.x / p.ksplit : (int)blockIdx.x, ntile = blockIdx.y;
@@ -288,20 +294,22 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
         w[0][q] = lc.cA * sc.wA[q] + lc.cD * sc.wD[q];
         w[NA - 1][q] = lc.sepA ? sc.wA[q] : sc.wD[q];
       } else if (BWD) {
-        w[0][q] = sc.wA[q]; w[NA - 1][q] = sc.wD[q];
+        w[0][q] = sc.wA[q];
+        if (NA > 1) w[NA - 1][q] = sc.wD[q];   // static: A_s only
       } else {
         w[0][q] = grp == 0 ? alpha * sc.wA[q] + beta * sc.wD[q]     // X = (1+p1_0) A + (1+p1_1) A'
                            : gamma * sc.wA[q] + delta * sc.wD[q];   // Y = p2_0 A + p2_1 A'
       }
     }
     const int ntr = a.ldn >> 5, nt = a.ldk >> 5;      // row tiles of this rank's strip, tiles per row of tiles (= K chunks)
-    const float* P = ((grp == 1 && sharded) ? a.planes_t : a.planes) + (size_t)b * a.graph_stride + (size_t)sc.interval * 4 * a.ldn * a.ldk;
+    const float* P = ((grp == 1 && sharded) ? a.planes_t : a.planes) + (size_t)b * a.graph_stride +
+                     (STAT ? 0 : (size_t)sc.interval * 4 * a.ldn * a.ldk);
     // Tiled plane layout (peg_common.cuh): an item is four 16-KB tiles; warp w loads half (g) of tile u, every
     // warp-level LDG.128 is 512 contiguous bytes and the thread ends up with the 4x4 micro tile (rq, cq) of all
     // four planes: buf[plane*4 + m] = row 4*rq + m, columns 4*cq .. 4*cq+3 of the 32x32 tile.
     const int cv_u = w8 >> 1, cv_g = w8 & 1;
     const int cv_cq = lane & 7, cv_rq = ((lane & 7) + 4 * cv_g + (lane >> 3)) & 7;
-    const int cv_off = cv_g * 2048 + lane * 4;   // float offset of (g, plane 0, m 0, lane) inside a tile
+    const int cv_off = cv_g * (512 * NPL) + lane * 4;   // float offset of (g, plane 0, m 0, lane) inside a tile
 
     // One register buffer per thread (16 x LDG.128 = the thread's 4x4 micro tile of all four planes): a group issues the
     // loads of its next item right after publishing the current one; the two groups run out of phase, so ~2 items
@@ -315,26 +323,26 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
       if constexpr (F16) {
         // row tiles beyond the padded matrix (last 128-row block of a ragged n: 4 I + u >= nt, a per-warp, loop-invariant condition)
         // are read from row tile 0 and their weights are zero: no zero-fill path, the loads stay unconditional
-        const float* base = P + ((size_t)rt * nt + ct) * 4096 + cv_off;
+        const float* base = P + ((size_t)rt * nt + ct) * (1024 * NPL) + cv_off;
         const float* base_even = base + sw * 128;
         const float* base_odd = base - sw * 128;
 #pragma unroll
-        for (int q = 0; q < 4; ++q)
+        for (int q = 0; q < NPL; ++q)
 #pragma unroll
           for (int m = 0; m < 4; ++m) buf[q * 4 + m] = ldg_stream(((m & 1) ? base_odd : base_even) + (q * 4 + m) * 128);
         return;
       }
       if (rt < (tposed ? nt : ntr) && ct < (tposed ? ntr : nt)) {
-        const float* base = P + ((size_t)rt * nt + ct) * 4096 + cv_off;
+        const float* base = P + ((size_t)rt * nt + ct) * (1024 * NPL) + cv_off;
         const float* base_even = base + sw * 128;   // register row m <- tile row m ^ sw: even m read one row up, odd m one row down
         const float* base_odd = base - sw * 128;
 #pragma unroll
-        for (int q = 0; q < 4; ++q)
+        for (int q = 0; q < NPL; ++q)
 #pragma unroll
           for (int m = 0; m < 4; ++m) buf[q * 4 + m] = ldg_stream(((m & 1) ? base_odd : base_even) + (q * 4 + m) * 128);
       } else {
 #pragma unroll
-        for (int q = 0; q < 16; ++q) buf[q] = make_float4(0.f, 0.f, 0.f, 0.f);
+        for (int q = 0; q < 4 * NPL; ++q) buf[q] = make_float4(0.f, 0.f, 0.f, 0.f);
       }
     };
     // item j -> its plane tile: direct = rows of block I x chunk kc, transposed = chunk kc x columns of block I
@@ -386,7 +394,12 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
 #pragma unroll
         for (int m = 0; m < 4; ++m) {
           const float4 e0 = buf[0 * 4 + m], e1 = buf[1 * 4 + m], e2 = buf[2 * 4 + m], e3 = buf[3 * 4 + m];
-          if (BWD && !LIGHT && v == NA - 1) {   // A'_s = b + 2 s c + 3 s^2 d: the derivative has no `a` term (wD[0] == 0)
+          if (STAT) {   // one plane: the combine of the dense kernel with exact-zero planes b, c, d
+            t[v][4 * m + 0] = w0 * e0.x;
+            t[v][4 * m + 1] = w0 * e0.y;
+            t[v][4 * m + 2] = w0 * e0.z;
+            t[v][4 * m + 3] = w0 * e0.w;
+          } else if (BWD && !LIGHT && v == NA - 1) {   // A'_s = b + 2 s c + 3 s^2 d: the derivative has no `a` term (wD[0] == 0)
             t[v][4 * m + 0] = w1 * e1.x + w2 * e2.x + w3 * e3.x;
             t[v][4 * m + 1] = w1 * e1.y + w2 * e2.y + w3 * e3.y;
             t[v][4 * m + 2] = w1 * e1.z + w2 * e2.z + w3 * e3.z;
@@ -446,7 +459,8 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
 
     auto comb = [&](int v, float e0, float e1, float e2, float e3) -> float {
       float r;
-      if (BWD && v == NA - 1) r = w[v][1] * e1 + w[v][2] * e2 + w[v][3] * e3;    // A'_s has no `a` term (wD[0] == 0)
+      if (STAT) r = w[v][0] * e0;                                                   // one plane (b, c, d are exact zeros)
+      else if (BWD && v == NA - 1) r = w[v][1] * e1 + w[v][2] * e2 + w[v][3] * e3;    // A'_s has no `a` term (wD[0] == 0)
       else r = w[v][0] * e0 + w[v][1] * e1 + w[v][2] * e2 + w[v][3] * e3;
       return BFP ? r * fitem[v] : r;
     };
@@ -654,10 +668,14 @@ k_tc_contract(const __grid_constant__ CUtensorMap map_hi, const __grid_constant_
           }
         };
         ld16(0, r0);
-        if (BWD) { ld16(1, r1); ld16(2, r2); ld16(3, r3); }
+        if (BWD) { ld16(1, r1); ld16(2, r2); ld16(3, r3); }     // static: the A'_s slots of `partial` stay zero
       } else {
         tmem_ld16(taddr, r0);
-        if (BWD) {
+        if (BWD && STAT) {   // A'_s = 0: its products are exact zeros and were not computed
+          tmem_ld16(taddr + 2 * nd, r2);
+#pragma unroll
+          for (int u = 0; u < 16; ++u) r1[u] = r3[u] = 0u;
+        } else if (BWD) {
           tmem_ld16(taddr + nd, r1);
           tmem_ld16(taddr + 2 * nd, r2);
           tmem_ld16(taddr + 3 * nd, r3);
@@ -936,7 +954,7 @@ int tc_contract(cudaStream_t st, const PegDims& dm, const TcWs& w, const Contrac
   p.nd = pick_nd(d, bwd ? 128 : 256);
   p.nsplit = (dm.flags & PEG_FLAG_TF32_FAST) ? 1 : 3;
   p.nkc = ldk / 32;
-  const int na = bwd ? 2 : 1, sp = (f16 || p.nsplit == 3) ? 2 : 1;
+  const int na = (bwd && !a.stat) ? 2 : 1, sp = (f16 || p.nsplit == 3) ? 2 : 1;
   const int a_bytes = na * sp * (f16 ? TC_ATILE / 2 : TC_ATILE), b_bytes = sp * p.nd * TC_BK * (f16 ? 2 : 4);
   // smem rings: two B slots (one per pair in flight), the rest of ~208 KB goes to A slots (even count, at most 4)
   int sb = 2;
@@ -990,11 +1008,13 @@ int tc_contract(cudaStream_t st, const PegDims& dm, const TcWs& w, const Contrac
   // PEG_FLAG_ADJ_LIGHT (two of the four adjoint products single-pass): measured on B200 at n=2048, d=128, B=9 the adjoint launch
   // goes 213 -> 199 us (+5 % solver steps/s) but the param1/param2 gradients of a whole solve are off by up to 2.5e-3 (the rounding
   // of the slowly varying planes is correlated across launches, it does not average out) -> an accuracy mode the caller asks for
+  // (a static control never takes ADJ_LIGHT: make_ctx clears it)
   const int kind = bwd ? ((dm.flags & PEG_FLAG_ADJ_LIGHT) ? 2 : 1) : 0;   // tc_fmt() is 3xTF32 whenever ADJ_LIGHT is set
-  // the instantiation for (kind, format): 0..2 = 3xTF32 forward / adjoint / LIGHT adjoint, then bf16x2 and fp16x2 forward / adjoint
-  const int inst = fmt == PEG_FMT_TF32X3 ? kind : 3 + 2 * (fmt - 1) + kind;
+  // the instantiation for (kind, format): 0..2 = 3xTF32 forward / adjoint / LIGHT adjoint, then bf16x2 and fp16x2 forward / adjoint;
+  // 7..12 = the static-control forward / adjoint of 3xTF32, bf16x2, fp16x2
+  const int inst = a.stat ? 7 + 2 * fmt + kind : (fmt == PEG_FMT_TF32X3 ? kind : 3 + 2 * (fmt - 1) + kind);
   {
-    static std::atomic<unsigned> done[7] = {{0u}, {0u}, {0u}, {0u}, {0u}, {0u}, {0u}};
+    static std::atomic<unsigned> done[13] = {};
     switch (inst) {
       case 0: PEG_TRY(optin_smem(k_tc_contract<0, 0>, done[0])); break;
       case 1: PEG_TRY(optin_smem(k_tc_contract<1, 0>, done[1])); break;
@@ -1002,7 +1022,13 @@ int tc_contract(cudaStream_t st, const PegDims& dm, const TcWs& w, const Contrac
       case 3: PEG_TRY(optin_smem(k_tc_contract<0, 1>, done[3])); break;
       case 4: PEG_TRY(optin_smem(k_tc_contract<1, 1>, done[4])); break;
       case 5: PEG_TRY(optin_smem(k_tc_contract<0, 2>, done[5])); break;
-      default: PEG_TRY(optin_smem(k_tc_contract<1, 2>, done[6])); break;
+      case 6: PEG_TRY(optin_smem(k_tc_contract<1, 2>, done[6])); break;
+      case 7: PEG_TRY(optin_smem(k_tc_contract<0, 0, true>, done[7])); break;
+      case 8: PEG_TRY(optin_smem(k_tc_contract<1, 0, true>, done[8])); break;
+      case 9: PEG_TRY(optin_smem(k_tc_contract<0, 1, true>, done[9])); break;
+      case 10: PEG_TRY(optin_smem(k_tc_contract<1, 1, true>, done[10])); break;
+      case 11: PEG_TRY(optin_smem(k_tc_contract<0, 2, true>, done[11])); break;
+      default: PEG_TRY(optin_smem(k_tc_contract<1, 2, true>, done[12])); break;
     }
   }
   cudaLaunchConfig_t cfg;
@@ -1019,7 +1045,13 @@ int tc_contract(cudaStream_t st, const PegDims& dm, const TcWs& w, const Contrac
       case 3: return cudaLaunchKernelEx(&cfg, k_tc_contract<0, 1>, mhi, mlo, p);
       case 4: return cudaLaunchKernelEx(&cfg, k_tc_contract<1, 1>, mhi, mlo, p);
       case 5: return cudaLaunchKernelEx(&cfg, k_tc_contract<0, 2>, mhi, mlo, p);
-      default: return cudaLaunchKernelEx(&cfg, k_tc_contract<1, 2>, mhi, mlo, p);
+      case 6: return cudaLaunchKernelEx(&cfg, k_tc_contract<1, 2>, mhi, mlo, p);
+      case 7: return cudaLaunchKernelEx(&cfg, k_tc_contract<0, 0, true>, mhi, mlo, p);
+      case 8: return cudaLaunchKernelEx(&cfg, k_tc_contract<1, 0, true>, mhi, mlo, p);
+      case 9: return cudaLaunchKernelEx(&cfg, k_tc_contract<0, 1, true>, mhi, mlo, p);
+      case 10: return cudaLaunchKernelEx(&cfg, k_tc_contract<1, 1, true>, mhi, mlo, p);
+      case 11: return cudaLaunchKernelEx(&cfg, k_tc_contract<0, 2, true>, mhi, mlo, p);
+      default: return cudaLaunchKernelEx(&cfg, k_tc_contract<1, 2, true>, mhi, mlo, p);
     }
   };
   const cudaError_t le = launch();

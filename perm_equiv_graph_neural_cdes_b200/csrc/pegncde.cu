@@ -319,8 +319,9 @@ static int contract(Ctx& c, int l, bool bwd, const float* V, const float* Mref, 
                     bool relu, bool scale_tg, float* g_fus, bool vt_ready, const float* cbM = nullptr, bool cbM_global = false) {
   const LayerDesc& ld = c.m.layer[l];
   ContractArgs a;
-  a.planes = c.ctl.adj_coef;
-  a.graph_stride = (size_t)(c.d.T - 1) * 4 * c.d.ldn * c.d.ldn;
+  a.stat = c.ctl.adj_static ? 1 : 0;
+  a.planes = a.stat ? c.ctl.adj_static : c.ctl.adj_coef;
+  a.graph_stride = a.stat ? (size_t)c.d.ldn * c.d.ldn : (size_t)(c.d.T - 1) * 4 * c.d.ldn * c.d.ldn;
   a.sc = c.w.sc;
   a.svec = c.w.svec;
   a.sv_stride = c.sv_stride;
@@ -344,10 +345,10 @@ static int contract(Ctx& c, int l, bool bwd, const float* V, const float* Mref, 
   a.n_glob = c.sh ? c.sh->n_glob : c.d.n;
   a.row_block0 = c.sh ? c.sh->row0 / 128 : 0;
   if (c.sh) a.graph_stride = (size_t)(c.d.T - 1) * 4 * c.d.ldn * a.ldk;
-  // algorithmic work of one launch: the four coefficient planes are traversed once (16 n^2 B per graph),
-  // V is read and OUT written once; 2 (fwd) or 4 (bwd) n x n x d products.
+  // algorithmic work of one launch: the four coefficient planes are traversed once (16 n^2 B per graph; a static control's one
+  // plane: 4 n^2 B), V is read and OUT written once; 2 (fwd) or 4 (bwd) n x n x d products.
   const double nn = (double)c.d.n * c.d.n, nd = (double)c.d.n * ld.dout;
-  double bytes = c.d.B * (16.0 * nn + 4.0 * nd * (bwd ? 3.0 : 2.0));
+  double bytes = c.d.B * ((a.stat ? 4.0 : 16.0) * nn + 4.0 * nd * (bwd ? 3.0 : 2.0));
   double flops = c.d.B * (bwd ? 8.0 : 4.0) * nn * ld.dout;
   if (c.ctl.sparse) {
     // sparse path: both orientations' coefficients (one piece) and columns, both row-pointer arrays, V and OUT once (+ M in the
@@ -383,10 +384,14 @@ static int contract(Ctx& c, int l, bool bwd, const float* V, const float* Mref, 
     if (rc == PEG_OK) g_launches.fetch_add(vt_ready ? 1 : (c.w.tc.fmt == PEG_FMT_FP16X2 ? 3 : 2));
   } else {
     dim3 grid((c.d.n + CT_TI - 1) / CT_TI, (ld.dout + CT_TC - 1) / CT_TC, c.d.B);
-    if (!bwd)
+    if (a.stat) {
+      if (!bwd) k_dual_contract<1, true><<<grid, 256, 0, c.st>>>(a);
+      else k_dual_contract<4, true><<<grid, 256, 0, c.st>>>(a);
+    } else if (!bwd) {
       k_dual_contract<1><<<grid, 256, 0, c.st>>>(a);
-    else
+    } else {
       k_dual_contract<4><<<grid, 256, 0, c.st>>>(a);
+    }
     g_launches.fetch_add(1);
     cudaError_t e = cudaPeekAtLastError();
     if (e != cudaSuccess) { g_last_cuda = (int)e; (void)cudaGetLastError(); rc = PEG_ERR_CUDA; }
@@ -411,10 +416,15 @@ static void small_plan(Ctx& c) {
   if (smem > 220 * 1024) return;
   int dev = 0, sm_count = 0;
   if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) { (void)cudaGetLastError(); return; }
-  static std::atomic<unsigned> smem_done[2] = {{0u}, {0u}}, cluster_done[2] = {{0u}, {0u}};
-  if (optin_smem(k_small_fwd, smem_done[0]) != PEG_OK || optin_smem(k_small_vjp, smem_done[1]) != PEG_OK) return;
-  const bool nonportable = optin_nonportable_cluster(k_small_fwd, cluster_done[0]) == PEG_OK &&
-                           optin_nonportable_cluster(k_small_vjp, cluster_done[1]) == PEG_OK;
+  // a static control is planned exactly like a dense one (same cluster width): only the kernels' plane loads differ
+  static std::atomic<unsigned> smem_done[4] = {}, cluster_done[4] = {};
+  const bool stat = c.ctl.adj_static != nullptr;
+  auto fwd = stat ? k_small_fwd<true> : k_small_fwd<false>;
+  auto vjp = stat ? k_small_vjp<true> : k_small_vjp<false>;
+  const int k0 = stat ? 2 : 0;
+  if (optin_smem(fwd, smem_done[k0]) != PEG_OK || optin_smem(vjp, smem_done[k0 + 1]) != PEG_OK) return;
+  const bool nonportable = optin_nonportable_cluster(fwd, cluster_done[k0]) == PEG_OK &&
+                           optin_nonportable_cluster(vjp, cluster_done[k0 + 1]) == PEG_OK;
   // CTAs per graph: as many as keep the batch within one wave of SMs, no more than the widest phase has work items
   const int dL = c.m.layer[d.L - 1].dout;
   const int items = ((d.n + SG_RB - 1) / SG_RB) * ((dL + SG_WB - 1) / SG_WB);
@@ -446,7 +456,9 @@ static int small_launch(Ctx& c, const SmallArgs& a, bool vjp) {
   at[0].val.clusterDim.x = (unsigned)c.small_C; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
   cfg.attrs = at;
   cfg.numAttrs = 1;
-  const cudaError_t e = vjp ? cudaLaunchKernelEx(&cfg, k_small_vjp, a) : cudaLaunchKernelEx(&cfg, k_small_fwd, a);
+  const bool stat = c.ctl.adj_static != nullptr;
+  const cudaError_t e = vjp ? cudaLaunchKernelEx(&cfg, stat ? k_small_vjp<true> : k_small_vjp<false>, a)
+                            : cudaLaunchKernelEx(&cfg, stat ? k_small_fwd<true> : k_small_fwd<false>, a);
   g_launches.fetch_add(1);
   if (e != cudaSuccess) { g_last_cuda = (int)e; (void)cudaGetLastError(); return PEG_ERR_CUDA; }
   return PEG_OK;
@@ -664,11 +676,15 @@ static int check_sparse(const PegSparse* sp) {
 static int make_ctx(Ctx& c, peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params) {
   PEG_TRY(check_dims(dims));
   if (!ctl || !params) return PEG_ERR_NULL_POINTER;
-  if (!ctl->ts || (!ctl->adj_coef && !ctl->sparse) || !ctl->adj_rowsum || !ctl->adj_diag || !ctl->adj_total || !ctl->tch_coef)
+  if (!ctl->ts || (!ctl->adj_coef && !ctl->sparse && !ctl->adj_static) || !ctl->adj_rowsum || !ctl->adj_diag || !ctl->adj_total ||
+      !ctl->tch_coef)
     return PEG_ERR_NULL_POINTER;
   if (dims->e > 0 && !ctl->x_coef) return PEG_ERR_NULL_POINTER;
   if ((dims->flags & PEG_FLAG_DIRECTED) && !ctl->adj_colsum) return PEG_ERR_NULL_POINTER;
-  if (ctl->sparse) {
+  if (ctl->adj_static) {
+    if (ctl->sparse || ctl->shard) return PEG_ERR_UNSUPPORTED;   // a static control is one dense plane on one GPU
+    if (((uintptr_t)ctl->adj_static & 15) != 0) return PEG_ERR_ALIGNMENT;
+  } else if (ctl->sparse) {
     if (ctl->shard) return PEG_ERR_UNSUPPORTED;     // row-sharded sparse controls are not implemented
     PEG_TRY(check_sparse(ctl->sparse));
   } else if (((uintptr_t)ctl->adj_coef & 15) != 0) {
@@ -676,12 +692,13 @@ static int make_ctx(Ctx& c, peg_stream_t stream, const PegDims* dims, const PegC
   }
   c.st = (cudaStream_t)stream;
   c.d = *dims;
+  if (ctl->adj_static) c.d.flags &= ~PEG_FLAG_ADJ_LIGHT;   // no A'_s product to lighten: the static adjoint is the exact one
   c.ctl = *ctl;
   c.params = params;
   c.m = make_model(*dims);
   c.sv_stride = svec_stride(dims->n, dims->L, dims->e);
   c.use_tc = (dims->flags & PEG_FLAG_TENSOR_CORES) != 0;
-  c.fmt = tc_fmt(*dims, ctl->adj_absmax != nullptr);
+  c.fmt = tc_fmt(c.d, ctl->adj_absmax != nullptr);
   c.t_dev = c.dt_dev = nullptr;
   c.tcoef = 0.f;
   c.g_adj = nullptr;
@@ -860,11 +877,11 @@ static int pack_common(peg_stream_t stream, const PegDims* dims, const float* d,
   const bool unit_time = planar || snap;   // no time channel in the source: d(time)/dt == 1
   grid.x = ncpad / 32;                    // one block per column of tiles
   k_pack_adj<<<grid, 256, 0, st>>>(d, c, b, a, planar, snap, ts, dims->n, dims->ldn, Tm1, piece0, count, adj_coef, adj_rowsum,
-                                   adj_diag, adj_total, tch_coef, ncols, diag_col0);
+                                   adj_diag, adj_total, tch_coef, ncols, diag_col0, 4);
   PEG_LAUNCH_CHECK();
   if (adj_rowsum && adj_total) {   // row sums and totals of the tiled planes, reduced in a fixed order (deterministic)
     const float* tiled = planar ? planar : adj_coef;
-    k_adj_rowsums<<<dim3(nt, count, dims->B), 256, 0, st>>>(tiled, dims->n, dims->ldn, Tm1, piece0, adj_rowsum, ncpad);
+    k_adj_rowsums<<<dim3(nt, count, dims->B), 256, 0, st>>>(tiled, dims->n, dims->ldn, Tm1, piece0, adj_rowsum, ncpad, 4);
     PEG_LAUNCH_CHECK();
     k_adj_totals<<<dim3(4 * count, dims->B), 256, 0, st>>>(adj_rowsum, dims->n, Tm1, piece0, adj_total);
     PEG_LAUNCH_CHECK();
@@ -911,7 +928,7 @@ int pegncde_adj_colsums(peg_stream_t stream, const PegDims* dims, const float* a
   PEG_TRY(check_dims(dims));
   if (!adj_coef || !adj_colsum) return PEG_ERR_NULL_POINTER;
   const int nt = dims->ldn / 32;
-  k_adj_colsums<<<dim3(nt, dims->T - 1, dims->B), 256, 0, (cudaStream_t)stream>>>(adj_coef, dims->n, dims->ldn, dims->T - 1, adj_colsum);
+  k_adj_colsums<<<dim3(nt, dims->T - 1, dims->B), 256, 0, (cudaStream_t)stream>>>(adj_coef, dims->n, dims->ldn, dims->T - 1, adj_colsum, 4);
   PEG_LAUNCH_CHECK();
   return PEG_OK;
 }
@@ -926,7 +943,7 @@ int pegncde_adj_absmax(peg_stream_t stream, const PegDims* dims, int32_t piece_b
   PEG_CUDA(cudaMemset2DAsync(adj_absmax + (size_t)piece_begin * 4, (size_t)Tm1 * 4 * sizeof(float), 0, (size_t)piece_count * 4 * sizeof(float),
                              dims->B, st));
   const int nt = dims->ldn / 32, ntiles = nt * nt;
-  k_adj_absmax<<<dim3(ntiles < 64 ? ntiles : 64, piece_count, dims->B), 256, 0, st>>>(adj_coef, dims->ldn, Tm1, piece_begin, adj_absmax, dims->ldn);
+  k_adj_absmax<<<dim3(ntiles < 64 ? ntiles : 64, piece_count, dims->B), 256, 0, st>>>(adj_coef, dims->ldn, Tm1, piece_begin, adj_absmax, dims->ldn, 4);
   PEG_LAUNCH_CHECK();
   return PEG_OK;
 }
@@ -943,9 +960,62 @@ int pegncde_build_adj_rect(peg_stream_t stream, const PegDims* dims, int32_t n_c
     const int Tm1 = dims->T - 1, ncpad = peg_npad(n_cols);
     PEG_CUDA(cudaMemsetAsync(adj_absmax, 0, (size_t)dims->B * Tm1 * 4 * sizeof(float), st));
     const int ntiles = (dims->ldn / 32) * (ncpad / 32);
-    k_adj_absmax<<<dim3(ntiles < 64 ? ntiles : 64, Tm1, dims->B), 256, 0, st>>>(adj_coef, dims->ldn, Tm1, 0, adj_absmax, ncpad);
+    k_adj_absmax<<<dim3(ntiles < 64 ? ntiles : 64, Tm1, dims->B), 256, 0, st>>>(adj_coef, dims->ldn, Tm1, 0, adj_absmax, ncpad, 4);
     PEG_LAUNCH_CHECK();
   }
+  return PEG_OK;
+}
+
+// every piece of a static control's tables = piece 0: t [B][Tm1][per] <- t[b][0] for pieces 1 .. Tm1-1
+__global__ void k_repeat_piece0(float* __restrict__ t, size_t per, int Tm1, int B) {
+  const size_t total = (size_t)B * (Tm1 - 1) * per;
+  for (size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x) {
+    const size_t j = idx % per, r = idx / per, b = r / (Tm1 - 1), iv = 1 + r % (Tm1 - 1);
+    t[(b * Tm1 + iv) * per + j] = t[b * Tm1 * per + j];
+  }
+}
+
+int pegncde_build_adj_static(peg_stream_t stream, const PegDims* dims, const float* adjacency, float* adj_static, float* adj_rowsum,
+                             float* adj_diag, float* adj_total, float* adj_colsum, float* adj_absmax, float* tch_coef) {
+  PEG_TRY(check_dims(dims));
+  if (!adjacency || !adj_static || !adj_rowsum || !adj_diag || !adj_total || !adj_colsum || !adj_absmax || !tch_coef)
+    return PEG_ERR_NULL_POINTER;
+  if (((uintptr_t)adj_static & 15) != 0) return PEG_ERR_ALIGNMENT;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int B = dims->B, n = dims->n, npad = dims->ldn, nt = npad / 32, Tm1 = dims->T - 1;
+  const size_t vec = (size_t)B * Tm1 * 4 * n, sc = (size_t)B * Tm1 * 4;
+  // slots b, c, d of every table stay zero (A' = 0); slot a of piece 0 is written by the dense kernels run with one plane, in their
+  // summation order, then repeated for every piece
+  PEG_CUDA(cudaMemsetAsync(adj_rowsum, 0, vec * sizeof(float), st));
+  PEG_CUDA(cudaMemsetAsync(adj_diag, 0, vec * sizeof(float), st));
+  PEG_CUDA(cudaMemsetAsync(adj_colsum, 0, vec * sizeof(float), st));
+  PEG_CUDA(cudaMemsetAsync(adj_absmax, 0, sc * sizeof(float), st));
+  k_pack_adj<<<dim3(nt, 1, B), 256, 0, st>>>(nullptr, nullptr, nullptr, nullptr, nullptr, adjacency, nullptr, n, npad, Tm1, 0, 1,
+                                             adj_static, nullptr, adj_diag, nullptr, nullptr, n, 0, 1);
+  PEG_LAUNCH_CHECK();
+  k_adj_rowsums<<<dim3(nt, 1, B), 256, 0, st>>>(adj_static, n, npad, Tm1, 0, adj_rowsum, npad, 1);
+  PEG_LAUNCH_CHECK();
+  k_adj_totals<<<dim3(4, B), 256, 0, st>>>(adj_rowsum, n, Tm1, 0, adj_total);
+  PEG_LAUNCH_CHECK();
+  k_adj_colsums<<<dim3(nt, 1, B), 256, 0, st>>>(adj_static, n, npad, Tm1, adj_colsum, 1);
+  PEG_LAUNCH_CHECK();
+  k_adj_absmax<<<dim3(nt * nt < 64 ? nt * nt : 64, 1, B), 256, 0, st>>>(adj_static, npad, Tm1, 0, adj_absmax, npad, 1);
+  PEG_LAUNCH_CHECK();
+  if (Tm1 > 1) {
+    float* per_n[3] = {adj_rowsum, adj_diag, adj_colsum};
+    for (float* t : per_n) {
+      k_repeat_piece0<<<(unsigned)std::min<size_t>(4096, ((size_t)B * (Tm1 - 1) * 4 * n + 255) / 256), 256, 0, st>>>(t, (size_t)4 * n, Tm1, B);
+      PEG_LAUNCH_CHECK();
+    }
+    float* per_4[2] = {adj_total, adj_absmax};
+    for (float* t : per_4) {
+      k_repeat_piece0<<<(unsigned)std::min<size_t>(4096, ((size_t)B * (Tm1 - 1) * 4 + 255) / 256), 256, 0, st>>>(t, 4, Tm1, B);
+      PEG_LAUNCH_CHECK();
+    }
+  }
+  const size_t cnt = (size_t)B * Tm1 * 3 * n;
+  k_fill_tch_unit<<<(unsigned)((cnt + 255) / 256), 256, 0, st>>>(tch_coef, n, (size_t)B * Tm1);
+  PEG_LAUNCH_CHECK();
   return PEG_OK;
 }
 

@@ -107,6 +107,8 @@ class PackedControl:
 def fused_control(ts, coeffs_adj, x_coeffs, hidden_dim, num_layers, flags=PEG_FLAG_TENSOR_CORES):
     if hasattr(coeffs_adj, "row_ptr_t"):
         raise TypeError("the JAX handlers take dense coefficient arrays; sparse (CSR) controls run through the torch API only")
+    if hasattr(coeffs_adj, "adj_static"):
+        raise TypeError("the JAX handlers take dense coefficient arrays; static controls run through the torch API only")
     d = jnp.ndim(coeffs_adj[0])
     cadj = [c if d == 5 else c[None] for c in coeffs_adj]
     cx = None if x_coeffs is None else [c if jnp.ndim(c) == 5 else c[None] for c in x_coeffs]
