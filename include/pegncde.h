@@ -177,8 +177,8 @@ typedef struct PegControl {
                               per graph instead of 16 n^2.  adj_coef may be NULL; adj_rowsum / adj_diag / adj_total / adj_colsum /
                               adj_absmax keep their [B, T-1, 4, ...] shapes with A's statistics in the `a` slot of every piece and zeros in
                               b, c, d.  PEG_FLAG_ADJ_LIGHT means nothing for it (there is no A'_s product to lighten).  Not combinable with
-                              sparse or shard, nor differentiable in A (g_adj_coef): PEG_ERR_UNSUPPORTED; 16-byte aligned
-                              (PEG_ERR_ALIGNMENT) */
+                              sparse or shard, nor with g_adj_coef: PEG_ERR_UNSUPPORTED; 16-byte aligned (PEG_ERR_ALIGNMENT).
+                              Differentiable in A through pegncde_vf_vjp_adj_static / pegncde_solve_bwd_adj_static */
 } PegControl;
 
 /* ---- parameter packing ---------------------------------------------------------------
@@ -277,6 +277,16 @@ int pegncde_vf_vjp(peg_stream_t stream, const PegDims* dims, const PegControl* c
 int pegncde_vf_vjp_adj(peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params, float t,
                        const float* y, const float* g_dy, float* g_y, float* g_params, float* g_xdot, float* g_adj_coef,
                        void* workspace, size_t workspace_bytes);
+/* pegncde_vf_vjp plus the gradient of a static control's adjacency: g_adj_static [B, ldn, ldn] row-major fp32 (row pitch ldn)
+ * ACCUMULATES d loss / d A (caller zeroes it); only entries i, j < n are touched.  The control's statistics (row / column sums,
+ * diagonal, total) are functions of A and are differentiated through.  Every entry has one owner per layer and the launches are
+ * stream-ordered, so the result is reproducible bit for bit.  The small-graph cluster kernels compute no adjacency gradient: a call
+ * with g_adj_static runs the per-operator path, and its other outputs equal those of pegncde_vf_vjp with PEG_FLAG_NO_FUSED_SMALL.
+ * Same workspace as pegncde_vf_vjp.  A control that is not static with a non-NULL g_adj_static returns PEG_ERR_UNSUPPORTED, a
+ * pointer that is not 16-byte aligned PEG_ERR_ALIGNMENT; with g_adj_static == NULL the call is pegncde_vf_vjp. */
+int pegncde_vf_vjp_adj_static(peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params, float t,
+                              const float* y, const float* g_dy, float* g_y, float* g_params, float* g_xdot, float* g_adj_static,
+                              void* workspace, size_t workspace_bytes);
 
 /* ---- one Tsit5 step (adaptive controllers stay on the host) ----------------------------- */
 /* k1 = f(t, y) when k1_valid == 0 (first step) else taken from k1 (FSAL).  Writes y1, y_err
@@ -367,6 +377,14 @@ int pegncde_solve_bwd_adj(peg_stream_t stream, const PegDims* dims, const PegCon
                           const float* step_ts, int32_t steps, const float* y_ckpt, const float* stage_store,
                           const float* g_yT, const float* g_ckpt, const float* g_stage, float* g_y0, float* g_params,
                           float* g_xcoef, float* g_adj_coef, void* workspace, size_t workspace_bytes);
+/* pegncde_solve_bwd plus g_adj_static (nullable, static controls only) [B, ldn, ldn]: ACCUMULATES d loss / d A over every stage of
+ * every step, as pegncde_vf_vjp_adj_static does for one evaluation (same checks, same path rule: with g_adj_static the adjoint runs
+ * the per-operator path, and its other outputs equal pegncde_solve_bwd's with PEG_FLAG_NO_FUSED_SMALL).  The per-graph views of
+ * a batch (B = 1 controls) write their graph's slice of one shared buffer (offset b * ldn * ldn). */
+int pegncde_solve_bwd_adj_static(peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params,
+                                 const float* step_ts, int32_t steps, const float* y_ckpt, const float* stage_store,
+                                 const float* g_yT, const float* g_ckpt, const float* g_stage, float* g_y0, float* g_params,
+                                 float* g_xcoef, float* g_adj_static, void* workspace, size_t workspace_bytes);
 
 /* ---- introspection ------------------------------------------------------------------------ */
 const char* pegncde_strerror(int code);

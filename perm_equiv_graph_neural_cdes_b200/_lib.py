@@ -85,6 +85,7 @@ SIGNATURES = {
     "pegncde_vf_fwd": (c_int, [_P, _DIMS, _CTL, _P, c_float, _P, _P, _P, c_size_t]),
     "pegncde_vf_vjp": (c_int, [_P, _DIMS, _CTL, _P, c_float, _P, _P, _P, _P, _P, _P, c_size_t]),
     "pegncde_vf_vjp_adj": (c_int, [_P, _DIMS, _CTL, _P, c_float, _P, _P, _P, _P, _P, _P, _P, c_size_t]),
+    "pegncde_vf_vjp_adj_static": (c_int, [_P, _DIMS, _CTL, _P, c_float, _P, _P, _P, _P, _P, _P, _P, c_size_t]),
     "pegncde_step_fwd": (c_int, [_P, _DIMS, _CTL, _P, c_float, c_float, _P, _P, c_int32, _P, _P, _P, _P, _P, c_size_t]),
     "pegncde_step_fwd_batched": (c_int, [_P, _DIMS, _CTL, _P, _P, _P, _P, _P, c_int32, _P, _P, _P, _P, _P, c_size_t]),
     "pegncde_adaptive_control": (c_int, [_P, _DIMS, _P, c_float, c_float, c_float, c_float, c_float, c_float, c_int32, _P, c_int32, c_int32,
@@ -96,6 +97,7 @@ SIGNATURES = {
     "pegncde_stage_store_bytes": (c_size_t, [_DIMS, c_int32]),
     "pegncde_solve_bwd": (c_int, [_P, _DIMS, _CTL, _P, POINTER(c_float), c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P, c_size_t]),
     "pegncde_solve_bwd_adj": (c_int, [_P, _DIMS, _CTL, _P, POINTER(c_float), c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, c_size_t]),
+    "pegncde_solve_bwd_adj_static": (c_int, [_P, _DIMS, _CTL, _P, POINTER(c_float), c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, c_size_t]),
     "pegncde_strerror": (c_char_p, [c_int]),
     "pegncde_last_cuda_error": (c_int, []),
     "pegncde_version": (c_char_p, []),

@@ -107,7 +107,7 @@ class PackedControl:
 
     Built once per batch; owns the device tensors and hands raw pointers to the C-ABI."""
 
-    adj_packed = None   # differentiable source of the adjacency coefficients: sparse controls only (SparseControl)
+    adj_packed = None   # differentiable source of the adjacency: sparse (SparseControl) and static (StaticControl) controls only
 
     def __init__(self, B: int, n: int, T: int, e: int, device):
         self.B, self.n, self.T, self.e = B, n, T, e
@@ -655,7 +655,9 @@ class StaticControl(PackedControl):
     costs ``4 ldn^2`` bytes per graph and every contraction reads a quarter of the bytes of the dense control of ``[A] * T`` -- whose
     results it reproduces bit for bit.  The O(n) tables keep the dense shapes (A's statistics in slot ``a``, zeros in b, c, d).
 
-    Built by :func:`build_static_control`; used wherever a :class:`PackedControl` is.  Not differentiable in A."""
+    Built by :func:`build_static_control`; used wherever a :class:`PackedControl` is.  Built with ``differentiable=True`` from an
+    adjacency that requires grad, ``adj_packed`` is the batched fp32 A ``[B, n, n]`` on the autograd tape: the solves and vector
+    fields then return d loss / d A (``pegncde_*_adj_static``) and it flows back to the caller's tensors."""
 
     def __init__(self, B: int, n: int, T: int, device):
         self.B, self.n, self.T, self.e, self.ldn = B, n, T, 0, _pad32(n)
@@ -669,6 +671,7 @@ class StaticControl(PackedControl):
         self.adj_absmax = torch.empty((B, T - 1, 4), **f)
         self.tch_coef = torch.empty((B, T - 1, 3, n), **f)
         self.x_coef, self.x_packed = None, None
+        self.adj_packed = None
         self._adj = {"colsum": torch.empty((B, T - 1, 4, n), **f), "pending": None, "host_ts": None}
 
     def struct(self) -> PegControl:
@@ -679,7 +682,8 @@ class StaticControl(PackedControl):
     def _view(self) -> "StaticControl":
         v = StaticControl.__new__(StaticControl)
         v.B, v.n, v.T, v.e, v.ldn = self.B, self.n, self.T, self.e, self.ldn
-        for name in ("ts", "adj_coef", "adj_static", "adj_rowsum", "adj_diag", "adj_total", "adj_absmax", "tch_coef", "x_coef", "x_packed"):
+        for name in ("ts", "adj_coef", "adj_static", "adj_rowsum", "adj_diag", "adj_total", "adj_absmax", "tch_coef", "x_coef", "x_packed",
+                     "adj_packed"):
             setattr(v, name, getattr(self, name))
         v._adj = self._adj
         v._keepalive = self
@@ -692,11 +696,12 @@ class StaticControl(PackedControl):
         return v
 
     def select(self, b: int) -> "StaticControl":
-        """View of graph ``b`` as a batch of one (no copy)."""
+        """View of graph ``b`` as a batch of one (no copy; ``adj_packed`` is sliced on the tape)."""
         v = self._view()
         v.B = 1
         for name in ("ts", "adj_static", "adj_rowsum", "adj_diag", "adj_total", "adj_absmax", "tch_coef"):
             setattr(v, name, getattr(self, name)[b:b + 1])
+        v.adj_packed = self.adj_packed[b:b + 1] if self.adj_packed is not None else None
         v.x_coef = self.x_coef[b:b + 1] if self.x_coef is not None else None
         v.x_packed = None
         v._adj = {"colsum": self.adj_colsum[b:b + 1], "pending": None, "host_ts": None}
@@ -732,17 +737,21 @@ class StaticControl(PackedControl):
         return out
 
 
-def build_static_control(ts: torch.Tensor, adjacency: torch.Tensor, x_t: Optional[torch.Tensor] = None, device=None) -> StaticControl:
+def build_static_control(ts: torch.Tensor, adjacency: torch.Tensor, x_t: Optional[torch.Tensor] = None, device=None, *,
+                         differentiable: bool = False) -> StaticControl:
     """A graph that does not change in time -> :class:`StaticControl` (``pegncde_build_adj_static``).  The same results, bit for bit,
     as ``build_control(ts, adjacency.expand(T, n, n), x_t)`` at a quarter of the plane bytes per contraction and ``1 / (4 (T-1))`` of
     the control's memory.
 
     ``adjacency``: ``[n, n]`` or ``[B, n, n]`` (a host tensor is copied to the device once); ``ts``: ``[T]`` or ``[B, T]`` (T >= 2);
-    ``x_t``: optional node signals ``[T, n, e]`` / ``[B, T, n, e]``.  The adjacency gets no gradient: one that requires grad raises."""
+    ``x_t``: optional node signals ``[T, n, e]`` / ``[B, T, n, e]``.
+
+    ``differentiable=True``: an adjacency that requires grad (a learned ``[n, n]`` parameter, ``softmax(relu(E E^T))``, ...) receives
+    d loss / d A through every solve and vector field run on this control.  Without it an adjacency that requires grad raises."""
     if not isinstance(adjacency, torch.Tensor):
         raise TypeError("adjacency must be a torch tensor")
-    if adjacency.requires_grad:
-        raise ValueError("build_static_control: static controls are not differentiable in the adjacency; pass adjacency.detach()")
+    if adjacency.requires_grad and not differentiable:
+        raise ValueError("build_static_control: pass differentiable=True to learn the adjacency, or adjacency.detach()")
     if adjacency.dim() not in (2, 3) or adjacency.shape[-1] != adjacency.shape[-2] or adjacency.shape[-1] < 1:
         raise ValueError(f"adjacency must be [n, n] or [B, n, n], got {tuple(adjacency.shape)}")
     if adjacency.dtype.is_complex:
@@ -763,6 +772,8 @@ def build_static_control(ts: torch.Tensor, adjacency: torch.Tensor, x_t: Optiona
     check(lib().pegncde_build_adj_static(_stream_ptr(device), sc.dims(h=4, L=1), A.data_ptr(), sc.adj_static.data_ptr(),
                                          sc.adj_rowsum.data_ptr(), sc.adj_diag.data_ptr(), sc.adj_total.data_ptr(), sc.adj_colsum.data_ptr(),
                                          sc.adj_absmax.data_ptr(), sc.tch_coef.data_ptr()), "pegncde_build_adj_static")
+    if A.requires_grad:
+        sc.adj_packed = A      # [B, n, n] fp32 on the tape: the gradient kernels return d loss / d A in this layout
     if x_t is not None:
         _attach_x(sc, _node_signal_coeffs(sc.ts, x_t, B, T, n, device), device)
     sc._keepalive = A          # the source lives until the builder has run (stream-ordered)

@@ -351,6 +351,99 @@ __global__ void __launch_bounds__(256) k_sparse_adj_grad(const AdjGradArgs a, co
   }
 }
 
+// =====================================================================================
+// Gradient of a static control's adjacency (pegncde_vf_vjp_adj_static / pegncde_solve_bwd_adj_static).  A static control has
+// A_s = A and A'_s = 0 on every piece (wA[0] = 1, wD[0] = 0), so only the gA half above reaches it, for every (i, j) < n:
+//   G_ij += (1 + p1) <Obar_i, M_j> + p2 <Obar_j, M_i> + [i == j] p3 q_i + rowA_i + totA + colA_j
+// The n x n part is one product per graph, X Y^T with X = [Obar | M] and Y = [(1 + p1) M | p2 Obar] (K = 2d, both K-major).
+// k_adj_grad is its fp32 FFMA form; k_tc_adj_grad (peg_tc.cu) its tcgen05 form.  The per-node and per-graph terms come from
+// k_sparse_adj_node / k_sparse_adj_tot.  One owner per element and stream-ordered launches: no atomics, reproducible bit for bit.
+// =====================================================================================
+constexpr int AG_TILE = 64;   // output rows / columns per CTA
+constexpr int AG_KC = 16;     // K chunk
+
+// element k of row r of X (xside) or of Y, zero past K = 2d; k is a multiple of 4 and d % 4 == 0, so a float4 never straddles
+__device__ __forceinline__ float4 adj_operand(const float* Gb, const float* Mb, int r, int k, int n, int d, bool xside, float alpha,
+                                              float gamma) {
+  if (r >= n || k >= 2 * d) return make_float4(0.f, 0.f, 0.f, 0.f);
+  const bool first = k < d;
+  const float* src = (first == xside ? Gb : Mb) + (size_t)r * d + (first ? k : k - d);
+  float4 v = __ldg(reinterpret_cast<const float4*>(src));
+  if (!xside) {
+    const float s = first ? alpha : gamma;
+    v.x *= s; v.y *= s; v.z *= s; v.w *= s;
+  }
+  return v;
+}
+
+// the epilogue's rank-one and diagonal terms for row i, columns j .. j+3 (all < n), added to the product
+__device__ __forceinline__ float4 adj_epilogue(float4 acc, int i, int j, float ri, float dq, const float* colA) {
+  acc.x += ri + colA[j] + (i == j ? dq : 0.f);
+  acc.y += ri + colA[j + 1] + (i == j + 1 ? dq : 0.f);
+  acc.z += ri + colA[j + 2] + (i == j + 2 ? dq : 0.f);
+  acc.w += ri + colA[j + 3] + (i == j + 3 ? dq : 0.f);
+  return acc;
+}
+
+// grid (ceil(n/64), ceil(n/64), B), block 256: each thread owns 4 x 4 outputs (rows 4 ty.., columns 4 tx..), the K loop runs in
+// chunks of 16 through shared memory (stored k-major, so the inner loop reads float4s).  g [B, ldn, ldn] row-major, accumulated.
+__global__ void __launch_bounds__(256) k_adj_grad(const AdjGradArgs a, float* __restrict__ g, int ldn) {
+  __shared__ __align__(16) float xs[AG_KC][AG_TILE + 4];
+  __shared__ __align__(16) float ys[AG_KC][AG_TILE + 4];
+  const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
+  const int b = blockIdx.z, n = a.n, d = a.d;
+  const int i0 = blockIdx.x * AG_TILE, j0 = blockIdx.y * AG_TILE;
+  const float* Gb = a.G + (size_t)b * n * d;
+  const float* Mb = a.M + (size_t)b * n * d;
+  const float alpha = 1.f + a.fus[0], gamma = a.fus[2];
+  const int lr = tid >> 2, lk = 4 * (tid & 3);       // loader: row lr of the tile, columns lk .. lk+3 of the chunk
+  float acc[4][4];
+#pragma unroll
+  for (int u = 0; u < 4; ++u)
+#pragma unroll
+    for (int v = 0; v < 4; ++v) acc[u][v] = 0.f;
+  for (int k0 = 0; k0 < 2 * d; k0 += AG_KC) {
+    const float4 xv = adj_operand(Gb, Mb, i0 + lr, k0 + lk, n, d, true, alpha, gamma);
+    const float4 yv = adj_operand(Gb, Mb, j0 + lr, k0 + lk, n, d, false, alpha, gamma);
+    __syncthreads();
+    xs[lk][lr] = xv.x; xs[lk + 1][lr] = xv.y; xs[lk + 2][lr] = xv.z; xs[lk + 3][lr] = xv.w;
+    ys[lk][lr] = yv.x; ys[lk + 1][lr] = yv.y; ys[lk + 2][lr] = yv.z; ys[lk + 3][lr] = yv.w;
+    __syncthreads();
+#pragma unroll
+    for (int kk = 0; kk < AG_KC; ++kk) {
+      const float4 xa = *reinterpret_cast<const float4*>(&xs[kk][4 * ty]);
+      const float4 yb = *reinterpret_cast<const float4*>(&ys[kk][4 * tx]);
+      const float xr[4] = {xa.x, xa.y, xa.z, xa.w}, yr[4] = {yb.x, yb.y, yb.z, yb.w};
+#pragma unroll
+      for (int u = 0; u < 4; ++u)
+#pragma unroll
+        for (int v = 0; v < 4; ++v) acc[u][v] = fmaf(xr[u], yr[v], acc[u][v]);
+    }
+  }
+  const float* nv = a.node + (size_t)b * 4 * n;
+  const float* colA = nv + 2 * n;
+  const float totA = a.tot[2 * b], f4 = a.fus[4];
+  const int j = j0 + 4 * tx;
+  if (j >= n) return;
+#pragma unroll
+  for (int u = 0; u < 4; ++u) {
+    const int i = i0 + 4 * ty + u;
+    if (i >= n) break;
+    const float ri = nv[i] + totA, dq = f4 * a.q[(size_t)b * n + i];
+    float* gr = g + ((size_t)b * ldn + i) * ldn;
+    const float4 s = make_float4(acc[u][0], acc[u][1], acc[u][2], acc[u][3]);
+    if (j + 4 <= n) {
+      const float4 t = adj_epilogue(s, i, j, ri, dq, colA);
+      float4 o = *reinterpret_cast<float4*>(gr + j);
+      o.x += t.x; o.y += t.y; o.z += t.z; o.w += t.w;
+      *reinterpret_cast<float4*>(gr + j) = o;
+    } else {
+      const float sv[4] = {s.x, s.y, s.z, s.w};
+      for (int v = 0; v < n - j; ++v) gr[j + v] += sv[v] + ri + colA[j + v] + (i == j + v ? dq : 0.f);
+    }
+  }
+}
+
 // lanes per row of k_sparse_adj_grad: as k_sparse_contract, at most 8
 inline int sparse_adj_glog(int d) {
   int g = 0;

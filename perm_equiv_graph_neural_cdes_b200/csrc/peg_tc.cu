@@ -2089,4 +2089,192 @@ int tc_weight_grad(cudaStream_t st, const PegDims& dm, const float* Mbar, const 
   return PEG_OK;
 }
 
+// ==========================================================================================
+// Gradient of a static adjacency through one layer on tcgen05 (3xTF32):  G[b] += X Y^T + rank-one / diagonal terms, with
+// X = [Obar | M] and Y = [(1 + p1) M | p2 Obar] ([n, 2d] each, K-major rows in global memory: no transpose).  Each CTA owns a
+// 128 x 128 output tile of one graph and the whole K = 2d, looped in chunks of 32 through a ring of swizzled hi / lo tiles that
+// the 8 loader warps fill (each thread: 4 float4 of X and 4 of Y per chunk, split and stored like k_tc_weight_grad's operands).
+// The MMA warp accumulates 128 x 128 fp32 in TMEM; the same 8 warps then read one row each (32 lanes x 64 columns per warp) and
+// read-modify-write G with 128-bit accesses, adding rowA_i + totA, colA_j and p3 q_i on the diagonal.  One owner per element,
+// no atomics: the result is reproducible bit for bit.
+// grid (ceil(n/128) row tiles, ceil(n/128) column tiles, B), block 288
+// ==========================================================================================
+constexpr int AGT_THREADS = 288;
+
+struct AgtParams {
+  const float* G;      // Obar [B, n, d]
+  const float* M;      // [B, n, d]
+  const float* fus;    // the layer's fusion scalars
+  const float* node;   // [B][4][n]
+  const float* q;      // [B][n]
+  const float* tot;    // [B][2]
+  float* out;          // [B, ldn, ldn]
+  int n, d, ldn, stages, nsplit;
+};
+
+__global__ void __launch_bounds__(AGT_THREADS, 1) k_tc_adj_grad(const AgtParams p) {
+  extern __shared__ __align__(1024) uint8_t smem_raw[];
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int S = p.stages, n = p.n, d = p.d, K = 2 * d;
+  const bool split = p.nsplit == 3;
+  const int b = blockIdx.z, i0 = blockIdx.x * 128, j0 = blockIdx.y * 128;
+  const int nchunks = (K + TC_BK - 1) / TC_BK;
+
+  const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
+  const int a_bytes = (split ? 2 : 1) * TC_ATILE;
+  const int stage_bytes = 2 * a_bytes;
+  const uint32_t bar_base = smem_base + S * stage_bytes;
+  auto full = [&](int s) { return bar_base + 8u * s; };
+  auto empty = [&](int s) { return bar_base + 8u * (S + s); };
+  const uint32_t accum_bar = bar_base + 8u * (2 * S);
+  const uint32_t tmem_slot = accum_bar + 8u;
+  uint8_t* smem_gen = smem_raw + (smem_base - smem_u32(smem_raw));
+
+  if (tid == 0) {
+    for (int s = 0; s < S; ++s) { mbar_init(full(s), 256); mbar_init(empty(s), 1); }
+    mbar_init(accum_bar, 1);
+    fence_barrier_init();
+  }
+  if (warp == 8) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(128));
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(smem_gen + (tmem_slot - smem_base));
+  const float* Gb = p.G + (size_t)b * n * d;
+  const float* Mb = p.M + (size_t)b * n * d;
+
+  if (warp < 8) {
+    const float alpha = 1.f + __ldg(p.fus), gamma = __ldg(p.fus + 2);
+    // 128 rows x 8 chunks of 16 bytes per operand tile: item f = tid + 256 u -> row f >> 3, 16-byte chunk f & 7
+    for (int j = 0; j < nchunks; ++j) {
+      float4 xv[4], yv[4];
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        const int f = tid + 256 * u, row = f >> 3, k = j * TC_BK + 4 * (f & 7);
+        const bool kin = k < K, first = k < d;
+        const int kc = first ? k : k - d;
+        const int i = i0 + row, jr = j0 + row;
+        xv[u] = (kin && i < n) ? __ldg(reinterpret_cast<const float4*>((first ? Gb : Mb) + (size_t)i * d + kc)) : make_float4(0.f, 0.f, 0.f, 0.f);
+        yv[u] = (kin && jr < n) ? __ldg(reinterpret_cast<const float4*>((first ? Mb : Gb) + (size_t)jr * d + kc)) : make_float4(0.f, 0.f, 0.f, 0.f);
+        const float s = first ? alpha : gamma;
+        yv[u].x *= s; yv[u].y *= s; yv[u].z *= s; yv[u].w *= s;
+      }
+      const int st = j % S;
+      mbar_wait(empty(st), ((uint32_t)(j / S) & 1u) ^ 1u);
+      const uint32_t x_base = smem_base + st * stage_bytes, y_base = x_base + a_bytes;
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        const int f = tid + 256 * u, row = f >> 3, c = f & 7;
+        const uint32_t off = (uint32_t)(row >> 3) * 1024u + (uint32_t)(row & 7) * 128u + (uint32_t)((c ^ (row & 7)) << 4);
+        const float4 src[2] = {xv[u], yv[u]};
+        const uint32_t base[2] = {x_base, y_base};
+#pragma unroll
+        for (int o = 0; o < 2; ++o) {
+          const float4 v = src[o];
+          const float h0 = tf32_rna(v.x), h1 = tf32_rna(v.y), h2 = tf32_rna(v.z), h3 = tf32_rna(v.w);
+          asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(base[o] + off), "f"(h0), "f"(h1), "f"(h2), "f"(h3) : "memory");
+          if (split)
+            asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(base[o] + TC_ATILE + off), "f"(v.x - h0), "f"(v.y - h1),
+                         "f"(v.z - h2), "f"(v.w - h3) : "memory");
+        }
+      }
+      fence_proxy_async();
+      mbar_arrive(full(st));
+    }
+  } else {
+    if (lane == 0) {
+      const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(128 >> 3) << 17) | ((uint32_t)(TC_BM >> 4) << 24);
+      for (int j = 0; j < nchunks; ++j) {
+        const int st = j % S;
+        mbar_wait(full(st), (uint32_t)(j / S) & 1u);
+        tc_fence_after();
+        const uint32_t xhi = smem_base + st * stage_bytes, xlo = xhi + TC_ATILE;
+        const uint32_t yhi = xhi + a_bytes, ylo = yhi + TC_ATILE;
+#pragma unroll
+        for (int k8 = 0; k8 < TC_BK / 8; ++k8) {
+          const uint64_t dxh = make_desc_sw128(xhi + k8 * 32), dyh = make_desc_sw128(yhi + k8 * 32);
+          umma_tf32(tmem_base, dxh, dyh, idesc, (j > 0 || k8 > 0) ? 1u : 0u);
+          if (split) {
+            umma_tf32(tmem_base, make_desc_sw128(xlo + k8 * 32), dyh, idesc, 1u);
+            umma_tf32(tmem_base, dxh, make_desc_sw128(ylo + k8 * 32), idesc, 1u);
+          }
+        }
+        umma_commit(empty(st));
+      }
+      umma_commit(accum_bar);
+    }
+  }
+
+  if (warp < 8) {
+    mbar_wait(accum_bar, 0u);
+    tc_fence_after();
+    const int qd = warp & 3, half = warp >> 2;
+    const int i = i0 + qd * 32 + lane;
+    const float* nv = p.node + (size_t)b * 4 * n;
+    const float* colA = nv + 2 * n;
+    const bool row_ok = i < n;
+    const float ri = row_ok ? nv[i] + p.tot[2 * b] : 0.f;
+    const float dq = row_ok ? __ldg(p.fus + 4) * p.q[(size_t)b * n + i] : 0.f;
+    float* gr = p.out + ((size_t)b * p.ldn + (row_ok ? i : 0)) * p.ldn;
+    for (int cc = 0; cc < 64; cc += 16) {
+      const int col = half * 64 + cc;
+      uint32_t r[16];
+      tmem_ld16(tmem_base + ((uint32_t)(qd * 32) << 16) + (uint32_t)col, r);
+      tmem_wait_ld();
+      if (!row_ok) continue;
+#pragma unroll
+      for (int v4 = 0; v4 < 4; ++v4) {
+        const int jc = j0 + col + 4 * v4;
+        const float s[4] = {__uint_as_float(r[4 * v4]), __uint_as_float(r[4 * v4 + 1]), __uint_as_float(r[4 * v4 + 2]),
+                            __uint_as_float(r[4 * v4 + 3])};
+        if (jc + 4 <= n) {
+          float4 o = *reinterpret_cast<float4*>(gr + jc);
+          o.x += s[0] + ri + colA[jc] + (i == jc ? dq : 0.f);
+          o.y += s[1] + ri + colA[jc + 1] + (i == jc + 1 ? dq : 0.f);
+          o.z += s[2] + ri + colA[jc + 2] + (i == jc + 2 ? dq : 0.f);
+          o.w += s[3] + ri + colA[jc + 3] + (i == jc + 3 ? dq : 0.f);
+          *reinterpret_cast<float4*>(gr + jc) = o;
+        } else {
+          for (int v = 0; v < 4 && jc + v < n; ++v) gr[jc + v] += s[v] + ri + colA[jc + v] + (i == jc + v ? dq : 0.f);
+        }
+      }
+    }
+    tc_fence_before();
+  }
+  __syncthreads();
+  if (warp == 8) {
+    __syncwarp();
+    tc_fence_after();
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(128));
+  }
+}
+
+int tc_adj_grad(cudaStream_t st, const PegDims& dm, const float* Obar, const float* M, int dcols, const float* fus, const float* node,
+                const float* q, const float* tot, float* g) {
+  if (dm.n < 128 || (dcols % 4) != 0) return PEG_ERR_UNSUPPORTED;
+  AgtParams p;
+  memset(&p, 0, sizeof(p));
+  p.G = Obar; p.M = M; p.fus = fus; p.node = node; p.q = q; p.tot = tot; p.out = g;
+  p.n = dm.n; p.d = dcols; p.ldn = dm.ldn;
+  p.nsplit = (dm.flags & PEG_FLAG_TF32_FAST) ? 1 : 3;
+  const int stage_bytes = 2 * (p.nsplit == 3 ? 2 : 1) * TC_ATILE;
+  int stages = (200 * 1024) / stage_bytes;
+  p.stages = stages > 4 ? 4 : stages;
+  const size_t smem = (size_t)p.stages * stage_bytes + 1024 + 8 * (2 * p.stages + 2) + 64;
+  static std::atomic<unsigned> done{0u};
+  PEG_TRY(optin_smem(k_tc_adj_grad, done));
+  const unsigned tiles = (unsigned)((dm.n + 127) / 128);
+  k_tc_adj_grad<<<dim3(tiles, tiles, dm.B), AGT_THREADS, smem, st>>>(p);
+  if (cudaPeekAtLastError() != cudaSuccess) {
+    const cudaError_t e = cudaGetLastError();
+    fprintf(stderr, "pegncde: k_tc_adj_grad launch failed (%s): grid %u x %u x %d, smem %zu\n", cudaGetErrorString(e), tiles, tiles, dm.B, smem);
+    set_last_cuda((int)e);
+    return PEG_ERR_CUDA;
+  }
+  return PEG_OK;
+}
+
 }  // namespace peg

@@ -61,6 +61,11 @@ int tc_weight_grad(cudaStream_t st, const PegDims& d, const float* Mbar, const f
                    float* gb);
 int tc_norm_linear(cudaStream_t st, const PegDims& d, const TcLinear& w, int layer, const float* Z, int din, int dout, float* M,
                    const ProducerOut& po);
+// gradient of a static adjacency through one layer (k_tc_adj_grad, 3xTF32): g [B, ldn, ldn] += X Y^T + the rank-one / diagonal
+// terms, X = [Obar | M], Y = [(1 + fus[0]) M | fus[2] Obar]; node = [B][4][n] (rowA, rowD, colA, colD), q = [B][n], tot = [B][2]
+// as k_sparse_adj_node / k_sparse_adj_tot write them.  fus is a device pointer.  Takes n >= 128.
+int tc_adj_grad(cudaStream_t st, const PegDims& d, const float* Obar, const float* M, int dcols, const float* fus, const float* node,
+                const float* q, const float* tot, float* g);
 bool tc_supported(const PegDims& d, int dcols);
 int tc_fmt(const PegDims& d, bool have_absmax);   // operand format of the contraction (PEG_FMT_*)
 int tc_convert_v(cudaStream_t st, const PegDims& d, const TcWs& w, const ContractArgs& a);

@@ -173,7 +173,8 @@ struct Ctx {
   unsigned int* xticket;   // arrival counter of k_shard_push (in the tickets area)
   int small_C;             // > 0: the cluster-per-graph kernels of peg_small.cuh evaluate f and its VJP (CTAs per graph)
   size_t small_smem;
-  float* g_adj;            // sparse controls (nullable): the VJP also accumulates the cotangent of PegSparse.coef here
+  float* g_adj;            // (nullable) the VJP also accumulates the cotangent of PegSparse.coef (sparse controls) or of the
+                           // static adjacency [B, ldn, ldn] (static controls) here
 };
 
 // ------------------------------------------------------------------------------------------
@@ -502,8 +503,11 @@ static int feval_fwd(Ctx& c, float t, const float* yin, float* dy, float* const*
   return PEG_OK;
 }
 
-// cotangent of the sparse coefficients through layer l (peg_sparse.cuh).  The node tables live in Za / Zb, which the VJP does not
-// use otherwise: [B][4][n] fits in Za and [B][n] + [B][2] in Zb, since h >= 4.
+// cotangent of the sparse coefficients, or of the static adjacency, through layer l (peg_sparse.cuh, peg_tc.cu).  The node tables
+// live in Za / Zb, which the VJP does not use otherwise: [B][4][n] fits in Za and [B][n] + [B][2] in Zb, since h >= 4.
+// The static n x n product runs on k_tc_adj_grad with PEG_FLAG_TENSOR_CORES and n >= 128, on the fp32 k_adj_grad otherwise.
+static bool adj_grad_on_tc(const Ctx& c) { return c.use_tc && c.d.n >= 128; }
+
 static int adj_grad(Ctx& c, int l, const float* M, const float* colM) {
   const PegDims& d = c.d;
   const LayerDesc& ld = c.m.layer[l];
@@ -520,6 +524,17 @@ static int adj_grad(Ctx& c, int l, const float* M, const float* colM) {
   PEG_LAUNCH_CHECK();
   k_sparse_adj_tot<<<d.B, 1024, 0, c.st>>>(a);
   PEG_LAUNCH_CHECK();
+  if (c.ctl.adj_static) {
+    if (adj_grad_on_tc(c)) {
+      PEG_TRY(tc_adj_grad(c.st, d, a.G, a.M, ld.dout, a.fus, a.node, a.q, a.tot, c.g_adj));
+      g_launches.fetch_add(1);
+    } else {
+      const unsigned tiles = (unsigned)((d.n + AG_TILE - 1) / AG_TILE);
+      k_adj_grad<<<dim3(tiles, tiles, d.B), 256, 0, c.st>>>(a, c.g_adj, d.ldn);
+      PEG_LAUNCH_CHECK();
+    }
+    return PEG_OK;
+  }
   const int glog = sparse_adj_glog(ld.dout), G = 1 << glog;
   k_sparse_adj_grad<<<dim3((unsigned)((d.n + 8 * (32 / G) - 1) / (8 * (32 / G))), d.B), 256, 0, c.st>>>(a, *c.ctl.sparse, glog);
   PEG_LAUNCH_CHECK();
@@ -1089,11 +1104,23 @@ static int set_adj_grad(Ctx& c, const PegControl* ctl, float* g_adj) {
   return PEG_OK;
 }
 
+// g_static (nullable): the cotangent of a static control's adjacency, [B, ldn, ldn] row-major, accumulated.  The small-graph cluster
+// kernels compute no adjacency gradient: a call that asks for one runs the per-operator path, as with PEG_FLAG_NO_FUSED_SMALL.
+static int set_adj_grad_static(Ctx& c, const PegControl* ctl, float* g_static) {
+  if (!g_static) return PEG_OK;
+  if (!ctl->adj_static) return PEG_ERR_UNSUPPORTED;
+  if (((uintptr_t)g_static & 15) != 0) return PEG_ERR_ALIGNMENT;
+  c.g_adj = g_static;
+  c.small_C = 0;
+  return PEG_OK;
+}
+
 static int vf_vjp(peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params, float t, const float* y,
-                  const float* g_dy, float* g_y, float* g_params, float* g_xdot, float* g_adj, void* workspace, size_t workspace_bytes) {
+                  const float* g_dy, float* g_y, float* g_params, float* g_xdot, float* g_adj, bool adj_static, void* workspace,
+                  size_t workspace_bytes) {
   Ctx c;
   PEG_TRY(make_ctx(c, stream, dims, ctl, params));
-  PEG_TRY(set_adj_grad(c, ctl, g_adj));
+  PEG_TRY(adj_static ? set_adj_grad_static(c, ctl, g_adj) : set_adj_grad(c, ctl, g_adj));
   if (!y || !g_dy || !g_y || !g_params || !workspace) return PEG_ERR_NULL_POINTER;
   if (workspace_bytes < plan(*dims, PEG_WS_VF_VJP, 0, nullptr, nullptr, nullptr)) return PEG_ERR_WORKSPACE;
   SolveWs s;
@@ -1111,13 +1138,19 @@ static int vf_vjp(peg_stream_t stream, const PegDims* dims, const PegControl* ct
 int pegncde_vf_vjp(peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params, float t,
                    const float* y, const float* g_dy, float* g_y, float* g_params, float* g_xdot, void* workspace,
                    size_t workspace_bytes) {
-  return vf_vjp(stream, dims, ctl, params, t, y, g_dy, g_y, g_params, g_xdot, nullptr, workspace, workspace_bytes);
+  return vf_vjp(stream, dims, ctl, params, t, y, g_dy, g_y, g_params, g_xdot, nullptr, false, workspace, workspace_bytes);
 }
 
 int pegncde_vf_vjp_adj(peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params, float t,
                        const float* y, const float* g_dy, float* g_y, float* g_params, float* g_xdot, float* g_adj_coef,
                        void* workspace, size_t workspace_bytes) {
-  return vf_vjp(stream, dims, ctl, params, t, y, g_dy, g_y, g_params, g_xdot, g_adj_coef, workspace, workspace_bytes);
+  return vf_vjp(stream, dims, ctl, params, t, y, g_dy, g_y, g_params, g_xdot, g_adj_coef, false, workspace, workspace_bytes);
+}
+
+int pegncde_vf_vjp_adj_static(peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params, float t,
+                              const float* y, const float* g_dy, float* g_y, float* g_params, float* g_xdot, float* g_adj_static,
+                              void* workspace, size_t workspace_bytes) {
+  return vf_vjp(stream, dims, ctl, params, t, y, g_dy, g_y, g_params, g_xdot, g_adj_static, true, workspace, workspace_bytes);
 }
 
 int pegncde_step_fwd(peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params, float t,
@@ -1325,11 +1358,13 @@ int pegncde_solve_fwd(peg_stream_t stream, const PegDims* dims, const PegControl
 
 static int solve_bwd(peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params, const float* step_ts,
                      int32_t steps, const float* y_ckpt, const float* stage_store, const float* g_yT, const float* g_ckpt,
-                     const float* g_stage, float* g_y0, float* g_params, float* g_xcoef, float* g_adj, void* workspace,
-                     size_t workspace_bytes) {
+                     const float* g_stage, float* g_y0, float* g_params, float* g_xcoef, float* g_adj, bool adj_static,
+                     void* workspace, size_t workspace_bytes) {
   Ctx c;
   PEG_TRY(make_ctx(c, stream, dims, ctl, params));
-  PEG_TRY(set_adj_grad(c, ctl, g_adj));
+  // a forward on the small-graph kernels keeps no M_l in the stage store: an adjoint moved off them must recompute M_l
+  const bool store_has_m = c.small_C == 0;
+  PEG_TRY(adj_static ? set_adj_grad_static(c, ctl, g_adj) : set_adj_grad(c, ctl, g_adj));
   if (!step_ts || !y_ckpt || (!g_yT && !g_ckpt) || !g_y0 || !g_params || !workspace) return PEG_ERR_NULL_POINTER;
   if (steps < 1) return PEG_ERR_BAD_DIMS;
   if (g_xcoef && dims->e == 0) return PEG_ERR_BAD_DIMS;
@@ -1410,7 +1445,7 @@ static int solve_bwd(peg_stream_t stream, const PegDims* dims, const PegControl*
       if (stage_store) {
         StoreSlots kept = store_slots(*dims, const_cast<float*>(stage_store), sidx, i);
         if (i == 0) kept.z[0] = const_cast<float*>(y);
-        PEG_TRY(stage_vjp(tis[i], kept.z, s.kbar, s.Ybar[i], kept.m, kept.cm));
+        PEG_TRY(stage_vjp(tis[i], kept.z, s.kbar, s.Ybar[i], store_has_m ? kept.m : nullptr, store_has_m ? kept.cm : nullptr));
       } else {
         float* save[PEG_MAX_LAYERS];
         save[0] = (i == 0) ? const_cast<float*>(y) : s.save[i][0];
@@ -1439,7 +1474,7 @@ int pegncde_solve_bwd(peg_stream_t stream, const PegDims* dims, const PegControl
                       const float* g_yT, const float* g_ckpt, const float* g_stage, float* g_y0, float* g_params,
                       float* g_xcoef, void* workspace, size_t workspace_bytes) {
   return solve_bwd(stream, dims, ctl, params, step_ts, steps, y_ckpt, stage_store, g_yT, g_ckpt, g_stage, g_y0, g_params, g_xcoef,
-                   nullptr, workspace, workspace_bytes);
+                   nullptr, false, workspace, workspace_bytes);
 }
 
 int pegncde_solve_bwd_adj(peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params,
@@ -1447,7 +1482,15 @@ int pegncde_solve_bwd_adj(peg_stream_t stream, const PegDims* dims, const PegCon
                           const float* g_yT, const float* g_ckpt, const float* g_stage, float* g_y0, float* g_params,
                           float* g_xcoef, float* g_adj_coef, void* workspace, size_t workspace_bytes) {
   return solve_bwd(stream, dims, ctl, params, step_ts, steps, y_ckpt, stage_store, g_yT, g_ckpt, g_stage, g_y0, g_params, g_xcoef,
-                   g_adj_coef, workspace, workspace_bytes);
+                   g_adj_coef, false, workspace, workspace_bytes);
+}
+
+int pegncde_solve_bwd_adj_static(peg_stream_t stream, const PegDims* dims, const PegControl* ctl, const float* params,
+                                 const float* step_ts, int32_t steps, const float* y_ckpt, const float* stage_store,
+                                 const float* g_yT, const float* g_ckpt, const float* g_stage, float* g_y0, float* g_params,
+                                 float* g_xcoef, float* g_adj_static, void* workspace, size_t workspace_bytes) {
+  return solve_bwd(stream, dims, ctl, params, step_ts, steps, y_ckpt, stage_store, g_yT, g_ckpt, g_stage, g_y0, g_params, g_xcoef,
+                   g_adj_static, true, workspace, workspace_bytes);
 }
 
 const char* pegncde_strerror(int code) {

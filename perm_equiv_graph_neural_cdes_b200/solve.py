@@ -32,8 +32,9 @@ import numpy as np
 import torch
 
 from ._lib import PEG_WS_SOLVE_BWD, PEG_WS_SOLVE_FWD, PEG_WS_STEP, PEG_WS_VF_FWD, check, lib
-from .control import _stream_ptr
-from .vector_field import CDEWrapperVectorField, PermEquivGraphVectorField, adj_grad_buffer, resolve_control, workspace
+from .control import StaticControl, _stream_ptr
+from .vector_field import (CDEWrapperVectorField, PermEquivGraphVectorField, adj_grad_buffer, adj_grad_out, resolve_control,
+                           workspace)
 
 
 STREAM_MIN_PIECE_BYTES = 128 << 20   # host coefficient arrays are streamed piece by piece above this size per cubic piece
@@ -130,11 +131,13 @@ def constant_step_table(t0: float, t1: float, dt0: float, rule: str = "state", m
     return np.asarray(out, dtype=np.float32)
 
 
-def _solve_bwd(l, g_adj, *args) -> None:
-    """pegncde_solve_bwd, or pegncde_solve_bwd_adj when the cotangent of the sparse coefficients is asked for (``args`` = the
-    arguments up to g_xcoef, then the workspace pointer and size)."""
+def _solve_bwd(l, pc, g_adj, *args) -> None:
+    """pegncde_solve_bwd, or pegncde_solve_bwd_adj / pegncde_solve_bwd_adj_static when the cotangent of the sparse coefficients / the
+    static adjacency is asked for (``args`` = the arguments up to g_xcoef, then the workspace pointer and size)."""
     if g_adj is None:
         check(l.pegncde_solve_bwd(*args), "pegncde_solve_bwd")
+    elif isinstance(pc, StaticControl):
+        check(l.pegncde_solve_bwd_adj_static(*args[:-2], g_adj.data_ptr(), *args[-2:]), "pegncde_solve_bwd_adj_static")
     else:
         check(l.pegncde_solve_bwd_adj(*args[:-2], g_adj.data_ptr(), *args[-2:]), "pegncde_solve_bwd_adj")
 
@@ -204,12 +207,12 @@ class _SolveFunction(torch.autograd.Function):
         g_adj = adj_grad_buffer(pc, ctx.needs_input_grad[3])
         ctl = pc.struct()
         store = ctx.store
-        _solve_bwd(l, g_adj, _stream_ptr(dev), dims, ctl, flat.data_ptr(),
+        _solve_bwd(l, pc, g_adj, _stream_ptr(dev), dims, ctl, flat.data_ptr(),
                    ctx.host_ts.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), S, y_ckpt.data_ptr(),
                    store.data_ptr() if store is not None else None, g_yT.data_ptr(), g_ckpt.data_ptr() if g_ckpt is not None else None, None, g_y0.data_ptr(),
                    g_flat.data_ptr(), g_x.data_ptr() if g_x is not None else None, ws.data_ptr(), ws.numel())
         ctx.store = None
-        return g_y0, g_flat, g_x, g_adj, None, None, None, None, None
+        return g_y0, g_flat, g_x, adj_grad_out(pc, g_adj), None, None, None, None, None
 
 
 def dense_samples_of_table(step_ts: np.ndarray, save_ts: np.ndarray):
@@ -290,10 +293,10 @@ class _FixedDenseFunction(torch.autograd.Function):
         g_flat = torch.zeros_like(flat)
         g_x = torch.zeros_like(pc.x_coef) if ctx.needs_input_grad[2] else None
         g_adj = adj_grad_buffer(pc, ctx.needs_input_grad[3])
-        _solve_bwd(l, g_adj, _stream_ptr(dev), dims, pc.struct(), flat.data_ptr(), host_ts.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), S,
+        _solve_bwd(l, pc, g_adj, _stream_ptr(dev), dims, pc.struct(), flat.data_ptr(), host_ts.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), S,
                    y_ckpt.data_ptr(), None, None, g_ckpt.data_ptr(), g_stage.data_ptr(), g_y0.data_ptr(), g_flat.data_ptr(),
                    g_x.data_ptr() if g_x is not None else None, ws.data_ptr(), ws.numel())
-        return g_y0, g_flat, g_x, g_adj, None, None, None, None
+        return g_y0, g_flat, g_x, adj_grad_out(pc, g_adj), None, None, None, None
 
 
 def _stream_pieces(pc, step_ts, run_steps) -> None:
@@ -545,7 +548,7 @@ class _AdaptiveSolveFunction(torch.autograd.Function):
             pc1 = pc.select(b)
             rec["dims"], rec["pc1"] = vf.dims_for(pc1, with_wrapper=wrapped), pc1
             stats_out.append(rec["stats"])
-        ctx.recs, ctx.has_ts = recs, save_ts is not None
+        ctx.recs, ctx.has_ts, ctx.pc = recs, save_ts is not None, pc
         ctx.save_for_backward(flat)
         return out   # [M or 1, B, n, h]
 
@@ -556,7 +559,8 @@ class _AdaptiveSolveFunction(torch.autograd.Function):
         dev = flat.device
         g_out = g_out.contiguous().to(torch.float32)
         g_flat = torch.zeros_like(flat)
-        g_adj = adj_grad_buffer(ctx.recs[0]["pc1"], ctx.needs_input_grad[2])   # shared by the per-graph views: entries are absolute
+        # shared by the per-graph views: sparse entries are absolute, a static view writes its graph's slice
+        g_adj = adj_grad_buffer(ctx.pc, ctx.needs_input_grad[2])
         g_y0s = []
         for b, rec in enumerate(ctx.recs):
             dims, pc1, y_ckpt, step_ts = rec["dims"], rec["pc1"], rec["y_ckpt"], rec["step_ts"]
@@ -576,12 +580,13 @@ class _AdaptiveSolveFunction(torch.autograd.Function):
                             g_stage[s, i].add_(gm, alpha=float(w[i]))
             else:
                 g_ckpt[S] = g_out[0, b:b + 1]
-            _solve_bwd(l, g_adj, _stream_ptr(dev), dims, pc1.struct(), flat.data_ptr(),
+            g_adj1 = g_adj[b:b + 1] if g_adj is not None and isinstance(pc1, StaticControl) else g_adj
+            _solve_bwd(l, pc1, g_adj1, _stream_ptr(dev), dims, pc1.struct(), flat.data_ptr(),
                        step_ts.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), S, y_ckpt.data_ptr(), None, None,
                        g_ckpt.data_ptr(), g_stage.data_ptr() if g_stage is not None else None, g_y0.data_ptr(),
                        g_flat.data_ptr(), None, ws.data_ptr(), ws.numel())
             g_y0s.append(g_y0)
-        return (torch.cat(g_y0s, dim=0), g_flat, g_adj) + (None,) * 10
+        return (torch.cat(g_y0s, dim=0), g_flat, adj_grad_out(ctx.pc, g_adj)) + (None,) * 10
 
 
 def _diffeqsolve_adaptive(vf, wrapped, pc, t0, t1, dt0, yb, unb, ctrl, saveat, max_steps) -> Solution:

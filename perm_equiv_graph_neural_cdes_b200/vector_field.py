@@ -15,7 +15,7 @@ import torch
 from torch import nn
 
 from ._lib import PEG_FLAG_DIRECTED, PEG_FLAG_TENSOR_CORES, PEG_WS_VF_VJP, PegDims, check, lib
-from .control import CubicInterpolation, PackedControl, _stream_ptr, pack_control
+from .control import CubicInterpolation, PackedControl, StaticControl, _stream_ptr, pack_control
 
 _WS_CACHE = {}
 
@@ -265,8 +265,20 @@ def resolve_control(control_adj, control_data, device) -> PackedControl:
 
 
 def adj_grad_buffer(pc, needed: bool):
-    """Zeroed cotangent of a sparse control's coefficients (``pegncde_*_adj``), or None when it is not asked for."""
-    return torch.zeros_like(pc.coef) if needed else None
+    """Zeroed cotangent of a sparse control's coefficients (``pegncde_*_adj``) or of a static control's adjacency, ``[B, ldn, ldn]``
+    (``pegncde_*_adj_static``), or None when it is not asked for."""
+    if not needed:
+        return None
+    if isinstance(pc, StaticControl):
+        return torch.zeros((pc.B, pc.ldn, pc.ldn), dtype=torch.float32, device=pc.adj_static.device)
+    return torch.zeros_like(pc.coef)
+
+
+def adj_grad_out(pc, g):
+    """The cotangent of ``pc.adj_packed`` from an :func:`adj_grad_buffer` buffer: a static control's ``[B, n, n]`` corner."""
+    if g is None or not isinstance(pc, StaticControl):
+        return g
+    return g[:, :pc.n, :pc.n]
 
 
 class _VFFunction(torch.autograd.Function):
@@ -300,9 +312,11 @@ class _VFFunction(torch.autograd.Function):
                 g_flat.data_ptr(), None)
         if g_adj is None:
             check(l.pegncde_vf_vjp(*args, ws.data_ptr(), ws.numel()), "pegncde_vf_vjp")
+        elif isinstance(pc, StaticControl):
+            check(l.pegncde_vf_vjp_adj_static(*args, g_adj.data_ptr(), ws.data_ptr(), ws.numel()), "pegncde_vf_vjp_adj_static")
         else:
             check(l.pegncde_vf_vjp_adj(*args, g_adj.data_ptr(), ws.data_ptr(), ws.numel()), "pegncde_vf_vjp_adj")
-        return g_y, g_flat, g_adj, None, None, None, None
+        return g_y, g_flat, adj_grad_out(pc, g_adj), None, None, None, None
 
 
 def fused_vector_field(vf: PermEquivGraphVectorField, t, y: torch.Tensor, control_adj, control_data) -> torch.Tensor:
